@@ -2,24 +2,33 @@
 """bench.py -- env-steps/s of the batched environment engine (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload uav_pos|uav_att|cartpole] [--impl reference]
+                    [--dump-outputs DIR]
 
 Default workload = config #4 of BASELINE.json: UavFntsmcParam position tracking (quadrotor RK4 + FNTSMC outer and
 inner loops), 1,048,576 instances per GPU, fp64, 8 fresh gains per instance per step, auto-reset on.  One "step" is
 one launch of the fused step kernel over all instances of this rank.  Instances shard independently over ranks (weak
 scaling, no data-path collective); the timed region is bracketed by barrier + synchronize and the reported time is
-the max over ranks.
+the max over ranks.  Exactly K steps are timed, in up to 5 blocks.
+
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step returned to its caller (current_state,
+next_state, policy_state, reward, is_terminal, terminal_flag, time) as DIR/<name>.npy, instances first, float64 or
+float32; at most 64 MB in all, so larger batches are cut to a fixed sample of instances (their indices in
+DIR/instance_index.npy).  Actions and initial states are seeded: the same arguments give the same inputs on every run,
+so the files of two builds can be compared one to one.
 
 The JSON line carries, besides the contract keys: `roofline` (the binding resource of the step kernel -- the FP64 pipe
 for the UAV / cart-pole kernels -- with the HBM view beside it; DRAM traffic and executed-instruction counts are parsed at
-run time from the committed ncu summaries under profiles/), `repeats` (the timed block of K steps run 5 times: median
-and spread), `cpu_baseline` (the UNMODIFIED Python reference on every host core, one process per core, from the
-byte-compiled staging oracle/_ref, and the C port beside it), `e2e` (same metric through the public VecEnv API with host
-buffers: pinned H2D of the actions and D2H of next_state / reward / done every step, plus a raw cudaMemcpyAsync probe of
-the same bytes), `clocks`, `gpu_launches`, and `also` (the other configs of BASELINE.json; under torchrun every rank
+run time from the committed ncu summaries under profiles/), `repeats` (the blocks the K timed steps ran in: median and
+spread of their time per step), `cpu_baseline` (the UNMODIFIED Python reference on every host core, one process per
+core, from the byte-compiled staging oracle/_ref, and the C port beside it), `e2e` (same metric through the public
+VecEnv API with host buffers: pinned H2D of the actions and D2H of next_state / reward / done every step, plus a raw
+cudaMemcpyAsync probe of the same bytes), `clocks`, `gpu_launches`, and `also` (the other configs of BASELINE.json; under torchrun every rank
 takes part in the sharded ones -- config #3's rollout + GAE + statistics all-reduce, config #5's DPPO2 iteration).
 
-`--impl reference` times the reference's own Python loop (oracle/_ref, or /root/reference where it exists) on all host
+`--impl reference` times the reference's own Python loop (oracle/_ref, or the tree RLP_REFERENCE names) on all host
 cores and never imports the product package.
+
+Nothing is written into the source tree: no bytecode caches either, so the tree may be read-only.
 """
 from __future__ import annotations
 
@@ -35,6 +44,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True
 
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
@@ -219,6 +229,27 @@ def timed_steps(env, pool, steps, warmup, dist_on, sampler=None, dis_pool=None):
     return ms
 
 
+DUMP_LIMIT = 63_000_000   # bytes of array data written by --dump-outputs: with the .npy headers, under 64 MB
+
+
+def dump_outputs(env, out_dir, seed=0):
+    """What the caller of the last step_soa receives, as out_dir/<name>.npy ([instances, ...], float64 or float32).  When
+    the whole batch would exceed DUMP_LIMIT, a fixed sample of instances (drawn from `seed`, sorted) is written instead,
+    with its indices in instance_index.npy."""
+    outs = {"current_state": env.current_state, "next_state": env.next_state, "policy_state": env.policy_state,
+            "reward": env.reward, "is_terminal": env.is_terminal, "terminal_flag": env.terminal_flag, "time": env.time}
+    outs = {k: (v if v.dtype in (torch.float64, torch.float32) else v.to(torch.float32)) for k, v in outs.items()}
+    n = env.n_envs
+    per_instance = 8 + sum(v[0].numel() * v.element_size() for v in outs.values())   # + the index column
+    k = min(n, DUMP_LIMIT // per_instance)
+    idx = np.arange(n) if k == n else np.sort(np.random.default_rng(seed).choice(n, size=k, replace=False))
+    sel = torch.as_tensor(idx, device=env.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "instance_index.npy"), idx.astype(np.float64))
+    for name, v in outs.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), v.index_select(0, sel).cpu().numpy())
+
+
 # Shards of the host-buffer path (timed_e2e): shard c's copies overlap shard c+1's kernel.  Measured on one B200 at 1 M
 # instances (tools/e2e_sweep.py): 1 shard 0.76e9, 2 shards 1.30e9, 3 shards 1.29e9, 4 shards 1.21e9, 8 shards 1.07e9
 # env-steps/s against 1.46e9 for the bare copies -- two shards already keep both directions of the link busy, more only add
@@ -303,9 +334,9 @@ def cpu_port(workload, n, steps, threads, seed=2024):
 
 
 def reference_tree():
-    """Where the UNMODIFIED Python reference can be imported from: the live tree in the build container, else the
-    byte-compiled staging made by oracle/stage_reference.py (travels to the GPU box as a built artefact)."""
-    for d in (os.environ.get("RLP_REFERENCE"), "/root/reference", os.path.join(ROOT, "oracle", "_ref")):
+    """Where the UNMODIFIED Python reference can be imported from: the tree RLP_REFERENCE names, else the byte-compiled
+    staging made by oracle/stage_reference.py."""
+    for d in (os.environ.get("RLP_REFERENCE"), os.path.join(ROOT, "oracle", "_ref")):
         if d and os.path.isdir(os.path.join(d, "environment")):
             return d
     return None
@@ -320,7 +351,7 @@ def reference_python(workload, seconds, procs):
     if tree is None:
         return None
     env = dict(os.environ, OMP_NUM_THREADS="1", MKL_NUM_THREADS="1", OPENBLAS_NUM_THREADS="1", RLP_REFERENCE=tree,
-               CUDA_VISIBLE_DEVICES="")
+               CUDA_VISIBLE_DEVICES="", PYTHONDONTWRITEBYTECODE="1")
     cmd = [sys.executable, os.path.join(ROOT, "oracle", "bench_reference_python.py"), "--worker", workload,
            "--seconds", str(seconds)]
     ps = [subprocess.Popen(cmd + ["--seed", str(k + 1)], stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, env=env, text=True)
@@ -713,14 +744,19 @@ def rollout_pipeline(workload, n, T, dev, dist_on, seed=5, offset=0):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=1000, help="timed steps of the headline workload, split into up to 5 blocks")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--workload", default="uav_pos", choices=sorted(WORKLOADS))
     ap.add_argument("--envs", type=int, default=0, help="instances per GPU (default: the config's)")
     ap.add_argument("--dtype", default="f64", choices=["f64", "f32"])
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-extras", action="store_true", help="skip cpu_baseline / e2e / also (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         return run_reference_arm(args)
@@ -754,14 +790,18 @@ def main():
     pool = action_pool(env, n, 4, dev, dtype, seed=rank + 1)
     sampler = ClockSampler(local)
     sampler.start()
-    # the timed block (exactly K steps between barrier + synchronize, CUDA events, max over ranks), five times: `value`
-    # comes from the median block, the spread is reported
-    REPEATS = 5
-    blocks = [timed_steps(env, pool, args.steps, args.warmup if r == 0 else 1, dist_on, sampler) for r in range(REPEATS)]
+    # the K timed steps, in up to five blocks (each between barrier + synchronize, CUDA events, max over ranks): `value`
+    # comes from the median block's time per step, the spread is reported
+    REPEATS = min(5, args.steps)
+    sizes = [args.steps // REPEATS + (r < args.steps % REPEATS) for r in range(REPEATS)]
+    blocks = [timed_steps(env, pool, k, args.warmup if r == 0 else 1, dist_on, sampler) for r, k in enumerate(sizes)]
     clocks = sampler.result()
-    ms = float(np.median(blocks))
-    value = world * n * args.steps / (ms * 1e-3)
-    per_launch_s = ms * 1e-3 / args.steps
+    per_step = [b_ / k for b_, k in zip(blocks, sizes)]
+    ms_step = float(np.median(per_step))
+    value = world * n / (ms_step * 1e-3)
+    per_launch_s = ms_step * 1e-3
+    if args.dump_outputs and rank == 0:
+        dump_outputs(env, args.dump_outputs)
     el = 8 if dtype == torch.float64 else 4
     algo_bytes = ALGO_BYTES[args.workload] * el / 8.0 * n
     peaks = {}
@@ -800,17 +840,16 @@ def main():
                      "traffic_source": facts["src"] if (facts and same_size) else None, "kernel": kernel})
     line = {
         "metric": "env-steps/sec", "value": value, "unit": "env-steps/s", "n_gpus": world, "steps": args.steps,
-        "warmup": args.warmup, "ms_per_step": ms / args.steps, "higher_is_better": True, "scaling": "weak",
+        "warmup": args.warmup, "ms_per_step": ms_step, "higher_is_better": True, "scaling": "weak",
         "vs_baseline": None, "dtype": args.dtype, "data": "synthetic",
         "config": {"workload": args.workload, "envs_per_gpu": n, "desc": WORKLOADS[args.workload]["desc"],
                    "auto_reset": True, "parallelism": f"env-shard x{world}",
                    "l2": "per-step working set (state + action + outputs) exceeds the 126 MB L2; 4 rotating action buffers"
                    if n >= (1 << 19) else "working set fits L2 (config size); launch-bound"},
-        "repeats": {"blocks": REPEATS, "steps_per_block": args.steps, "ms_per_step": [b_ / args.steps for b_ in blocks],
-                    "median_ms_per_step": ms / args.steps,
-                    "spread": (max(blocks) - min(blocks)) / ms},
+        "repeats": {"blocks": REPEATS, "steps_per_block": sizes, "ms_per_step": per_step, "median_ms_per_step": ms_step,
+                    "spread": (max(per_step) - min(per_step)) / ms_step},
         "roofline": roofline,
-        "clocks": clocks, "gpu_launches": args.steps * REPEATS,
+        "clocks": clocks, "gpu_launches": args.steps,
     }
     if not args.no_extras:
         A_dim, S_dim = env.action_dim, env.state_dim

@@ -20,7 +20,8 @@ pytestmark = pytest.mark.gpu
 def _load():
     from oracle import ref_shim as R
     if not R.available():
-        pytest.skip("reference tree not staged (oracle/_ref)")
+        pytest.skip("runs the original project's own PPO2 learner code, which is not part of the repository: "
+                    "no reference tree (RLP_REFERENCE, or oracle/_ref staged by build())")
     R.install()
     with R.quiet():
         envmod = R.load_file("demonstration/PPO2/PPO2-4-CartPoleAngleOnly/cartpole_angleonly.py", "ref_learner_env")
