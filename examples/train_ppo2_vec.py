@@ -39,6 +39,9 @@ def main(argv=None):
     ap.add_argument("--iters", type=int, default=30)
     ap.add_argument("--epochs", type=int, default=8)
     ap.add_argument("--seed", type=int, default=3407)   # the reference script's seed (train.py:36)
+    ap.add_argument("--eval-envs", type=int, default=0,
+                    help="after the last iteration, run the deterministic policy for one episode on this many instances "
+                         "in total (sharded over ranks)")
     args = ap.parse_args(argv)
     rank, world, local = D.init_from_env()
     dev = torch.device("cuda", local)
@@ -51,7 +54,7 @@ def main(argv=None):
     actor, critic = reference_nets(env.state_dim, env.action_dim, dev, init_std=net_kw["std"], mean_act=net_kw["mean_act"])
     agent = VecPPO2(env, actor, critic, {"buffer_size": args.steps, "K_epochs": args.epochs,
                                           "mini_batch_size": 16384}, std=net_kw["std"],
-                    seed=args.seed)
+                    seed=args.seed, track_episodes=True)
     env.reset(True)
     log = []
     for it in range(args.iters):
@@ -59,6 +62,8 @@ def main(argv=None):
         mean_r = agent.collect()
         torch.cuda.synchronize()
         t1 = time.perf_counter()
+        episodes = agent.episodes.summary()          # the episodes that ended in this rollout, raw rewards
+        agent.episodes.reset_stats()
         losses = agent.learn()
         torch.cuda.synchronize()
         t2 = time.perf_counter()
@@ -66,10 +71,21 @@ def main(argv=None):
         timeout_share = float(((agent.buffer.flag == env.TIMEOUT_FLAG) & (agent.buffer.done != 0)).float().sum() /
                               max(1.0, float(agent.buffer.done.sum())))
         row = {"iter": it, "mean_reward": mean_r, "done_rate": done_rate, "timeout_share": timeout_share,
-               "collect_env_steps_per_s": args.steps * n_local * world / (t1 - t0), "learn_s": t2 - t1, **losses}
+               "collect_env_steps_per_s": args.steps * n_local * world / (t1 - t0), "learn_s": t2 - t1, **losses,
+               "episodes": episodes["episodes"], "mean_episode_return": episodes["mean_return"],
+               "mean_episode_length": episodes["mean_length"], "flag_counts": episodes["flag_counts"]}
         log.append(row)
         if rank == 0:
             print(json.dumps(row))
+    if args.eval_envs > 0:
+        n_eval, off_eval = D.shard(args.eval_envs, rank, world)
+        eval_env = make(n_envs=n_eval, device=dev, dtype=torch.float64, io_dtype=torch.float32, auto_reset=True,
+                        seed=args.seed + 1, env_index_offset=off_eval)
+        ev = agent.evaluate_episodes(eval_env, max_steps=100000)
+        ev = {k: v for k, v in ev.items() if not torch.is_tensor(v)}
+        log.append({"eval": ev})
+        if rank == 0:
+            print(json.dumps({"eval": ev}))
     if world > 1:
         torch.distributed.destroy_process_group()
     return log

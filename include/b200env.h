@@ -429,6 +429,32 @@ B200_API int b200_adv_normalize(int64_t count, float *adv, const double *stats, 
 B200_API int b200_mc_returns(int r_dtype, int64_t T, int64_t N, const void *r, const uint8_t *done, double gamma,
                              float *returns, void *cuda_stream);
 
+/* K-EPISODE: episode returns, lengths and end reasons of an auto-reset rollout -- the per-episode reward sums of the
+ * reference's train loops and their deterministic test episodes, for N instance columns at once.  r is [T][N] in r_dtype
+ * (B200ENV_F32 / B200ENV_F64), done [T][N] u8 and flag [T][N] i32: the rollout columns the step kernels write (with T = 1
+ * an env's own reward / is_terminal / terminal_flag buffers).  Every done row ends an episode, so the rollout must come
+ * from an env stepped with B200ENV_AUTO_RESET.
+ * Per instance n, for t = 0 .. T-1:  acc_return[n] = acc_return[n] + (double)r[t][n] (one rounded float64 add);
+ *   acc_length[n] += 1;  if done[t][n]: emit (acc_return[n], acc_length[n], flag[t][n]) and zero the carry.
+ * acc_return (f64 [N]) and acc_length (i32 [N]) are the caller-owned carry of the episode in progress; zero them when
+ * the env is reset.  ep_return (f64), ep_length, ep_flag (i32), each [N] and each may be NULL: the last episode emitted
+ * by instance n (left untouched if it emitted none).  first_only = 1: an instance whose ep_flag is not -1 emits nothing
+ * (each instance contributes its first episode only; needs ep_flag, initialised to -1 by the caller).
+ * stats (device double[B200_EPISODE_STATS], may be NULL) is INCREMENTED over the emitted episodes:
+ *   [0] count  [1] sum return  [2] sum return^2  [3] sum length  [4] sum length^2
+ *   [5 + f] episodes that ended with flag f, f = 0 .. 15  [21] episodes with any other flag
+ * so it can be summed over calls and all-reduced over ranks.  It needs scratch (device, 8-byte aligned,
+ * b200_episode_scratch_bytes(N) bytes): per-block partials added in a fixed order, the same bits on every run.
+ * Errors, all returned before any CUDA call: B200ENV_ESIZE (T <= 0, N <= 0 or N >= 2^31), B200ENV_EDTYPE (r_dtype),
+ * B200ENV_ENULL (r, done, flag or the carry NULL; ep_flag NULL with first_only; scratch NULL with stats),
+ * B200ENV_EPARAMS (scratch too small or misaligned). */
+#define B200_EPISODE_STATS 22
+B200_API size_t b200_episode_scratch_bytes(int64_t N);
+B200_API int b200_episode_scan(int r_dtype, int64_t T, int64_t N, const void *r, const uint8_t *done,
+                               const int32_t *flag, double *acc_return, int32_t *acc_length, double *ep_return,
+                               int32_t *ep_length, int32_t *ep_flag, int first_only, double *stats, void *scratch,
+                               size_t scratch_bytes, void *cuda_stream);
+
 /* ------------------------------------------------------------- running normalisation */
 
 /* Replaces RunningMeanStd.update + Normalization.__call__ (utils/classes.py:626-656) as used on rewards

@@ -1,7 +1,8 @@
 """B200-native batched environment engine for the environment-step hot path of
 HKPolyU-UAV/ReinforcementLearningPlatform (see DESIGN.md, include/b200env.h)."""
 from . import _lib  # noqa: F401
-from . import compat, dist, gae, normalization, policy, rollout  # noqa: F401
+from . import compat, dist, episodes, gae, normalization, policy, rollout  # noqa: F401
+from .episodes import EpisodeTracker  # noqa: F401
 from .policy import GaussianPolicy  # noqa: F401
 from . import ppo2  # noqa: F401
 from .ppo2 import VecPPO2  # noqa: F401
@@ -15,7 +16,7 @@ from .envs.simple import (BallBalancer1D, Flight_Attitude_Simulator, FlightAttit
 from .envs.uavrobust import uav_hover, uav_hover_outer_loop, uav_inner_loop, uav_tracking_outer_loop  # noqa: F401
 from .envs.uav import UavAttCtrlRL, UavPosCtrlRL, uav_param, fntsmc_param  # noqa: F401
 
-__all__ = ["VecEnvBase", "RolloutBuffer", "Normalization", "GaussianPolicy", "VecPPO2", "SingleEnv", "single", "CartPole", "CartPoleAngleOnly", "UavAttCtrlRL", "UavPosCtrlRL", "uav_param", "fntsmc_param",
+__all__ = ["VecEnvBase", "RolloutBuffer", "EpisodeTracker", "Normalization", "GaussianPolicy", "VecPPO2", "SingleEnv", "single", "CartPole", "CartPoleAngleOnly", "UavAttCtrlRL", "UavPosCtrlRL", "uav_param", "fntsmc_param",
            "Flight_Attitude_Simulator", "FlightAttitudeSimulatorDiscrete", "SecondOrderIntegration", "BallBalancer1D", "TwoLinkManipulator", "UGVForward",
            "UGVBidirectional", "UGVForwardObstacleAvoidance", "uav_hover", "uav_hover_outer_loop",
            "uav_inner_loop", "uav_tracking_outer_loop"]

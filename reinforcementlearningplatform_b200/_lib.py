@@ -177,6 +177,10 @@ def load() -> C.CDLL:
     lib.b200_adv_normalize.argtypes = [i64, vp, vp, f64, vp]
     lib.b200_mc_returns.restype = i32
     lib.b200_mc_returns.argtypes = [i32, i64, i64, vp, vp, f64, vp, vp]
+    lib.b200_episode_scratch_bytes.restype = sz
+    lib.b200_episode_scratch_bytes.argtypes = [i64]
+    lib.b200_episode_scan.restype = i32
+    lib.b200_episode_scan.argtypes = [i32, i64, i64, vp, vp, vp, vp, vp, vp, vp, vp, i32, vp, vp, sz, vp]
     lib.b200_norm_scratch_bytes.restype = sz
     lib.b200_norm_scratch_bytes.argtypes = [i32]
     lib.b200_norm_seq.restype = i32

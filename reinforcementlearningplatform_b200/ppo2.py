@@ -27,6 +27,7 @@ import torch
 import torch.nn.functional as F
 
 from . import dist as _dist
+from .episodes import EpisodeTracker
 from .learn import FusedPPO2Update, fused_supported
 from .normalization import Normalization
 from .policy import GaussianPolicy, linear_layers
@@ -42,7 +43,7 @@ DEFAULT_PPO_MSG = {  # demonstration/PPO2/PPO2-4-CartPoleAngleOnly/train.py:141-
 class VecPPO2:
     def __init__(self, env, actor: torch.nn.Module, critic: torch.nn.Module, ppo_msg: Optional[dict] = None,
                  std=None, reward_norm: bool = True, seed: int = 0, group=None, actor_out_act: Optional[str] = None,
-                 learner: str = "auto"):
+                 learner: str = "auto", track_episodes: bool = False):
         """``env``: a vector env built with ``io_dtype=torch.float32, auto_reset=True``; ``actor`` / ``critic``: tanh
         MLPs on ``env.device`` (the reference's PPOActor_Gaussian / PPOCritic shapes, utils/classes.py:529-615);
         ``buffer_size`` of ``ppo_msg`` is the number of time steps T per rollout (T x N transitions per learn()).
@@ -50,7 +51,9 @@ class VecPPO2:
         ``out_act`` attribute, else "relu" (PPOActor_Gaussian.forward, utils/classes.py:563-569).  The behaviour policy
         (K-POLICY in ``collect``) and the learner's ``actor(s)`` must use the same head, or the ratios are wrong.
         ``std``: a float or one value per action dimension.
-        ``learner``: "fused" (K-LEARN, nets <= 64 wide), "torch" (autograd on the modules) or "auto" (fused if it fits)."""
+        ``learner``: "fused" (K-LEARN, nets <= 64 wide), "torch" (autograd on the modules) or "auto" (fused if it fits).
+        ``track_episodes``: keep per-episode statistics of the raw rewards of every rollout in ``self.episodes``
+        (an :class:`EpisodeTracker`; ``self.episodes.summary()`` reads them)."""
         self.env, self.actor, self.critic, self.group = env, actor, critic, group
         m = dict(DEFAULT_PPO_MSG)
         m.update(ppo_msg or {})
@@ -81,6 +84,7 @@ class VecPPO2:
             self.reduce_critic = _dist.FlatGradAllReducer(critic.parameters(), group)
         self._epoch_key = (int(seed) * 0x9E3779B97F4A7C15 + 0x5851F42D4C957F2D) & (2 ** 64 - 1)
         self.reward_norm = Normalization(1, device=env.device, group=group) if reward_norm else None
+        self.episodes = EpisodeTracker(env.n_envs, env.device, group=group) if track_episodes else None
         self.total_steps = 0
         self._gen = torch.Generator(device=env.device)
         self._gen.manual_seed(seed + 1)
@@ -91,6 +95,8 @@ class VecPPO2:
         env, buf = self.env, self.buffer
         if not env._policy_obs_valid:
             env.reset(True)
+            if self.episodes is not None:
+                self.episodes.reset_carry()
         # Row t of buf.s is the observation the policy acts on at step t: s[0] is copied once, every step then writes its
         # policy-facing observation straight into the next row (rollout.RolloutBuffer.step, chain_policy_obs).
         buf.s[0].copy_(env._reset_obs)
@@ -100,6 +106,8 @@ class VecPPO2:
         for t in range(buf.batch_size):
             self.policy(buf.s[t], action=buf.a[t], log_prob=buf.a_lp[t])            # choose_action, PPO2.py:69-76
             buf.step(env, t, buf.a[t], chain_policy_obs=True)                       # step_update + buffer.append
+        if self.episodes is not None:
+            self.episodes.update(buf.r, buf.done, buf.flag)                         # raw rewards: before K-NORM
         if self.reward_norm is not None:
             # r = reward_norm(env.reward) (:210) for the whole column at once: row t enters the statistics after rows < t
             # and is normalised with the statistics after row t, as the per-step calls did (three launches per rollout)
@@ -211,6 +219,36 @@ class VecPPO2:
         """actor mean for ``[state_dim, N]`` observations (``agent.evaluate``, PPO2.py:62-66)."""
         zero = torch.zeros(self.policy.action_dim, obs_soa.shape[1], dtype=torch.float32, device=obs_soa.device)
         return self.policy(obs_soa, noise=zero)["action"]
+
+    def evaluate_episodes(self, env, max_steps: int) -> dict:
+        """The deterministic policy (``evaluate``: the clamped actor mean) on every instance of ``env`` for one whole
+        episode each -- the test episodes of the reference's train loops, vectorised.  ``env``: a separate instance of the
+        training env's class built with ``io_dtype=torch.float32, auto_reset=True``; it is reset here and stepped until
+        every instance has finished an episode (checked every 64 steps, one host read each) or ``max_steps`` steps have
+        run.  Each instance contributes its FIRST episode, so short episodes are not over-represented.  Nothing of the
+        agent changes: not the training env, the policy's noise counter, the reward normaliser or the parameters.
+        Returns ``ep_return`` (float64, NaN = unfinished), ``ep_length`` and ``ep_flag`` (int32, -1 = unfinished), all
+        ``[N]`` device tensors, and the keys of :meth:`EpisodeTracker.summary`."""
+        if env is self.env or type(env) is not type(self.env):
+            raise ValueError("evaluate_episodes: env must be a separate instance of the training env's class")
+        if not env.auto_reset or env.io_dtype != torch.float32:
+            raise ValueError("evaluate_episodes: env must be built with auto_reset=True and io_dtype=torch.float32")
+        if (env.state_dim, env.action_dim) != (self.policy.state_dim, self.policy.action_dim):
+            raise ValueError("evaluate_episodes: env dimensions differ from the policy's")
+        tracker = EpisodeTracker(env.n_envs, env.device, first_only=True, group=self.group)
+        zero = torch.zeros(env.action_dim, env.n_envs, dtype=torch.float32, device=env.device)
+        action = torch.empty_like(zero)
+        log_prob = torch.empty_like(zero)
+        env.reset(True)
+        for t in range(int(max_steps)):
+            # env._reset_obs is the policy-facing observation; step_soa may swap it with _obs, so it is read every step
+            self.policy(env._reset_obs, noise=zero, action=action, log_prob=log_prob)
+            env.step_soa(action)
+            tracker.update(env._reward, env._done, env._flag)
+            if (t + 1) % 64 == 0 and bool(tracker.finished().all()):
+                break
+        return {"ep_return": tracker.ep_return, "ep_length": tracker.ep_length, "ep_flag": tracker.ep_flag,
+                **tracker.summary()}
 
 
 def reference_nets(state_dim: int, action_dim: int, device, init_std: float = 0.5, mean_act: str = "relu"):
