@@ -510,12 +510,11 @@ typedef struct b200_mlp {
  * value are not written); log_prob, mean may be NULL.  a_min, a_max: device float32 [A].  All nets must fit in shared
  * memory together with the tile's activations (the reference's 64-64-32 / 64-32 nets use ~110 KB) and no layer may be
  * wider than 64, else B200ENV_ESIZE. */
-/* precision: B200_POLICY_FP32 = float32 FMA pipe, sums in k order (<= 2e-6 absolute from torch's float32 GEMM);
- * B200_POLICY_TF32X3 = legacy warp-level tensor-core MMA with every operand split into two TF32 halves (3 MMAs per
- * product, fp32 accumulation; <= 5e-6 absolute).  Both keep every net in shared memory and reject layers wider than 64
- * (B200ENV_ESIZE); the tcgen05 path below has neither limit and is the one the Python mirror uses. */
+/* precision: must be B200_POLICY_FP32 = float32 FMA pipe, sums in k order (<= 2e-6 absolute from torch's float32 GEMM);
+ * any other value returns B200ENV_EPARAMS before any CUDA call.  This kernel keeps every net in shared memory and
+ * rejects layers wider than 64 (B200ENV_ESIZE); the tcgen05 path below has neither limit and is the one the Python
+ * mirror uses by default. */
 #define B200_POLICY_FP32   0
-#define B200_POLICY_TF32X3 1
 B200_API int b200_policy_forward(int64_t n, const b200_mlp *actor, const b200_mlp *critic, const float *obs,
                                  const float *a_min, const float *a_max, float std, const float *noise, uint64_t seed,
                                  uint64_t step, int64_t env_index_offset, int precision, float *action,

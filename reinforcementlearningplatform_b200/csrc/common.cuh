@@ -49,11 +49,7 @@ template <> struct Mth<double> {
     static __device__ __forceinline__ double div(double x, double y) { return fm64::div(x, y); }
     static __device__ __forceinline__ double tanh(double x) { return fm64::tanh(x); }
     static __device__ __forceinline__ double log(double x) { return fm64::log(x); }
-#ifdef B200_SMC_FULL_LOG
-    static __device__ __forceinline__ double log_nonneg(double x) { return fm64::log(x); }
-#else
     static __device__ __forceinline__ double log_nonneg(double x) { return fm64::log_nonneg(x); }
-#endif
     static __device__ __forceinline__ double exp(double x) { return fm64::exp(x); }
     static __device__ __forceinline__ double asin(double x) { return fm64::asin(x); }
 #endif

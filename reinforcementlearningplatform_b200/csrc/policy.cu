@@ -223,7 +223,6 @@ extern "C" B200_API int b200_policy_forward(int64_t n, const b200_mlp *actor, co
     io.seed = seed; io.step = step; io.off = env_index_offset;
     io.action = action; io.log_prob = log_prob; io.mean = mean; io.value = value;
     if (precision == B200_POLICY_FP32) return policy_launch_fp32(n, actor, critic, io, (cudaStream_t)cuda_stream);
-    if (precision == B200_POLICY_TF32X3) return policy_launch_tc(n, actor, critic, io, (cudaStream_t)cuda_stream);
     return B200ENV_EPARAMS;
 }
 

@@ -1,4 +1,5 @@
-// policy_common.cuh -- pieces shared by the two K-POLICY kernels (policy.cu: FP32 FMA pipe; policy_tc.cu: tensor cores).
+// policy_common.cuh -- pieces shared by the K-POLICY kernels (policy.cu: FP32 FMA pipe; policy_umma.cu and
+// policy_umma16.cu: tcgen05 tensor cores).
 #pragma once
 #include "common.cuh"
 
@@ -16,7 +17,6 @@ struct PolicyIO {
 };
 
 int policy_launch_fp32(int64_t n, const b200_mlp *actor, const b200_mlp *critic, const PolicyIO &io, cudaStream_t s);
-int policy_launch_tc(int64_t n, const b200_mlp *actor, const b200_mlp *critic, const PolicyIO &io, cudaStream_t s);
 // policy_umma.cu (tcgen05 / TMEM): weights pre-packed into a caller-owned workspace
 size_t policy_umma_workspace_bytes(const b200_mlp *actor, const b200_mlp *critic);
 int policy_umma_pack(const b200_mlp *actor, const b200_mlp *critic, void *workspace, size_t bytes, cudaStream_t s);
@@ -24,8 +24,7 @@ int policy_launch_umma(int64_t n, const b200_mlp *actor, const b200_mlp *critic,
                        const PolicyIO &io, cudaStream_t s);
 int policy_umma_probe(const float *A, const float *W, float *D, int N, int K, int three_pass, cudaStream_t s);
 // policy_umma16.cu (tcgen05 / TMEM, fp16-split operands, four tiles in flight): the nets it holds (layers <= 64 wide,
-// <= 32 observation fields) are routed to it by the three policy_umma_* entry points above; B200_POLICY_UMMA16=0 in the
-// environment keeps them on policy_umma.cu (A/B runs)
+// <= 32 observation fields) are routed to it by the three policy_umma_* entry points above
 bool policy_umma16_fits(const b200_mlp *actor, const b200_mlp *critic);
 size_t policy_umma16_workspace_bytes(const b200_mlp *actor, const b200_mlp *critic);
 int policy_umma16_pack(const b200_mlp *actor, const b200_mlp *critic, void *workspace, size_t bytes, cudaStream_t s);

@@ -1,6 +1,6 @@
 // policy_umma.cu -- K-POLICY on the 5th-generation tensor cores: tcgen05.mma (UMMA) with TMEM accumulators.
 //
-// Same contract as policy.cu / policy_tc.cu (Proximal_Policy_Optimization2.choose_action, algorithm/policy_base/
+// Same contract as policy.cu (Proximal_Policy_Optimization2.choose_action, algorithm/policy_base/
 // Proximal_Policy_Optimization2.py:69-76, and the critic forward of learn() :88-90; nets of utils/classes.py:529-615 and
 // the 256-wide copies of demonstration/DPPO2/DPPO2-4-UGVForwardObstacleAvoidance/train.py:26-107), rebuilt around the
 // Blackwell execution model after round 1's profile showed the legacy HMMA version at 0.50 ms per 1 M instances -- 63 %
@@ -40,7 +40,6 @@
 // of a core matrix 16 B apart, core matrices 128 B apart along M/N (SBO) and one "slab" (rows x 16 B) apart along K
 // (LBO): element (row, k) of an operand with R rows lives at (k / 4) * R * 16 + row * 16 + (k % 4) * 4.  With thread =
 // row the epilogue's 16-byte stores of a warp are 512 contiguous bytes: conflict-free without swizzling.
-#include <stdlib.h>
 #include <cuda_fp16.h>
 #include "policy_common.cuh"
 #include "umma_ptx.cuh"
@@ -641,16 +640,6 @@ int add_net(const b200_mlp *m, bool is_actor, UPlan *P, int *k_real, const float
     return B200ENV_OK;
 }
 
-// B200_POLICY_F16_WIDE=0 in the environment keeps the streamed mode on 3xTF32 (A/B runs)
-bool use_f16_streamed() {
-    static int enabled = -1;
-    if (enabled < 0) {
-        const char *e = getenv("B200_POLICY_F16_WIDE");
-        enabled = !(e && e[0] == '0');
-    }
-    return enabled != 0;
-}
-
 int build_plan(const b200_mlp *actor, const b200_mlp *critic, UPlan *P, int *k_real, const float **w, const float **b) {
     *P = UPlan{};
     int rc;
@@ -682,7 +671,7 @@ int build_plan(const b200_mlp *actor, const b200_mlp *critic, UPlan *P, int *k_r
         int cols = slots * slot_cols, pow2 = 32;
         while (pow2 < cols) pow2 *= 2;
         if (total > SMEM_LIMIT || pow2 > 512) continue;
-        if (streamed && use_f16_streamed()) {
+        if (streamed) {
             // streamed mode: every layer after a net's first multiplies fp16 pairs -- half the image bytes pulled through the
             // ring per tile and half the MMAs (kind::f16 covers K = 16); the image offsets are laid out again
             uint32_t off = 0;
@@ -707,24 +696,15 @@ int build_plan(const b200_mlp *actor, const b200_mlp *critic, UPlan *P, int *k_r
 
 } // namespace
 
-static bool use_umma16(const b200_mlp *actor, const b200_mlp *critic) {
-    static int enabled = -1;
-    if (enabled < 0) {
-        const char *e = getenv("B200_POLICY_UMMA16");
-        enabled = !(e && e[0] == '0');
-    }
-    return enabled && policy_umma16_fits(actor, critic);
-}
-
 size_t policy_umma_workspace_bytes(const b200_mlp *actor, const b200_mlp *critic) {
-    if (use_umma16(actor, critic)) return policy_umma16_workspace_bytes(actor, critic);
+    if (policy_umma16_fits(actor, critic)) return policy_umma16_workspace_bytes(actor, critic);
     UPlan P;
     if (build_plan(actor, critic, &P, nullptr, nullptr, nullptr)) return 0;
     return (size_t)(P.img_bytes + 127) / 128 * 128 + (size_t)P.bias_floats * 4;
 }
 
 int policy_umma_pack(const b200_mlp *actor, const b200_mlp *critic, void *workspace, size_t bytes, cudaStream_t stream) {
-    if (use_umma16(actor, critic)) return policy_umma16_pack(actor, critic, workspace, bytes, stream);
+    if (policy_umma16_fits(actor, critic)) return policy_umma16_pack(actor, critic, workspace, bytes, stream);
     PackArgs pa = {};
     UPlan P;
     int rc = build_plan(actor, critic, &P, pa.k_real, pa.w, pa.b);
@@ -745,7 +725,7 @@ int policy_umma_pack(const b200_mlp *actor, const b200_mlp *critic, void *worksp
 
 int policy_launch_umma(int64_t n, const b200_mlp *actor, const b200_mlp *critic, const void *workspace, size_t bytes,
                        const PolicyIO &io, cudaStream_t stream) {
-    if (use_umma16(actor, critic)) return policy_launch_umma16(n, actor, critic, workspace, bytes, io, stream);
+    if (policy_umma16_fits(actor, critic)) return policy_launch_umma16(n, actor, critic, workspace, bytes, io, stream);
     UArgs a = {};
     int rc = build_plan(actor, critic, &a.p, nullptr, nullptr, nullptr);
     if (rc) return rc;

@@ -86,9 +86,9 @@ __device__ __forceinline__ void epi16_compute(const uint32_t (&v)[16], const flo
     // tanh(x) = 1 - 2 / (2^t + 1), t = 2 log2(e) x; zs = 2 log2(e) / (the layer's weight scale)
 #pragma unroll
     for (int j = 0; j < 16; ++j) t[j] = fmaf(__uint_as_float(v[j]), zs, t[j]);
-#ifndef H_SEPARATE_RCP   // shared reciprocal: 0.2218 vs 0.2255 ms per 1 M instances (A/B on one box, twice)
     // one reciprocal for two activations: 1 / a = b / (a b), 1 / b = a / (a b); the exponent is clamped so that a b stays
-    // finite (2^60 + 1: tanh is 1 to the last bit long before).  1.5 instead of 2 MUFU per activation, +2 issue slots.
+    // finite (2^60 + 1: tanh is 1 to the last bit long before).  1.5 instead of 2 MUFU per activation, +2 issue slots:
+    // 0.2218 vs 0.2255 ms per 1 M instances for one reciprocal each (A/B on one box, twice).
 #pragma unroll
     for (int j = 0; j < 16; ++j) t[j] = fminf(t[j], 60.0f);
 #pragma unroll
@@ -101,12 +101,6 @@ __device__ __forceinline__ void epi16_compute(const uint32_t (&v)[16], const flo
         t[j] = r * b;
         t[j + 1] = r * a;
     }
-#else
-#pragma unroll
-    for (int j = 0; j < 16; ++j) asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(t[j]) : "f"(t[j]));
-#pragma unroll
-    for (int j = 0; j < 16; ++j) asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(t[j]) : "f"(t[j] + 1.0f));
-#endif
 #pragma unroll
     for (int j = 0; j < 16; ++j) t[j] = fmaf(-2.0f, t[j], 1.0f);
     uint32_t hi[8], lo[8];
@@ -126,14 +120,6 @@ __device__ __forceinline__ void epi16_compute(const uint32_t (&v)[16], const flo
 template <int NCH>
 __device__ __forceinline__ void epi_hidden(uint32_t slot_t, const float *bias_scaled, float zs) {
     uint32_t v[2][16];
-#ifdef H_NO_LDPIPE
-#pragma unroll
-    for (int c = 0; c < NCH; ++c) {
-        tmem_ld<16>(slot_t + 16 * c, v[0]);
-        tmem_wait_ld();
-        epi16_compute(v[0], bias_scaled + 16 * c, zs, slot_t + H_A_COL + 8 * c, slot_t + H_A_COL + H_A_LO + 8 * c);
-    }
-#else
     tmem_ld<16>(slot_t, v[0]);
 #pragma unroll
     for (int c = 0; c < NCH; ++c) {
@@ -141,7 +127,6 @@ __device__ __forceinline__ void epi_hidden(uint32_t slot_t, const float *bias_sc
         if (c + 1 < NCH) tmem_ld<16>(slot_t + 16 * (c + 1), v[(c + 1) & 1]);
         epi16_compute(v[c & 1], bias_scaled + 16 * c, zs, slot_t + H_A_COL + 8 * c, slot_t + H_A_COL + H_A_LO + 8 * c);
     }
-#endif
 }
 
 __global__ void __launch_bounds__(H_THREADS, 1)
@@ -180,6 +165,9 @@ policy_umma16_kernel(const __grid_constant__ HArgs a, int64_t n) {
         float *scr = scr_all + s * (16 * H_TILE) + r;                  // the row's means: scr[j * H_TILE]
         const uint32_t af = sbase + HBar::a_full + s * 8, dr = sbase + HBar::d_ready + s * 8;
         uint32_t layers_done = 0;
+        // xn: the first tile's observation fields.  These loads are dead (x8 is reloaded for every tile below and the
+        // compiler drops them), but they steer ptxas: without them the kernel has the same instructions in another order
+        // and measured 0.9 % slower (0.2208 vs 0.2189 ms per 1 M instances, five alternated runs each, B200 at 1000 W).
         float xn[8];
         {
             const int64_t t0 = (int64_t)blockIdx.x * H_SLOTS + s, i0 = t0 * H_TILE + r;
@@ -193,22 +181,12 @@ policy_umma16_kernel(const __grid_constant__ HArgs a, int64_t n) {
             const int64_t i = tile * H_TILE + r;
             const bool live = i < n;
             int pending_A = 0;
-            // the row's first 8 observation fields: fetched once per tile (both nets start from them) -- and for the
-            // NEXT tile one tile ahead, so that the DRAM latency is off the layer chain
+            // the row's first 8 observation fields: fetched once per tile (both nets start from them)
             float x8[8];
 #pragma unroll
             for (int e = 0; e < 8; ++e) x8[e] = xn[e];
-#ifndef H_PREFETCH  // fetching the next tile's observations one tile ahead measured 4 % SLOWER (0.233 vs 0.224 ms): not adopted
 #pragma unroll
             for (int e = 0; e < 8; ++e) x8[e] = (live && e < P.S) ? __ldg(a.io.obs + (int64_t)e * n + i) : 0.0f;
-#else
-            {
-                const int64_t tn = (grp + gridDim.x) * H_SLOTS + s, in = tn * H_TILE + r;
-                const bool ln = tn < tiles && in < n;
-#pragma unroll
-                for (int e = 0; e < 8; ++e) xn[e] = (ln && e < P.S) ? __ldg(a.io.obs + (int64_t)e * n + in) : 0.0f;
-            }
-#endif
             for (int li = 0; li < P.n_layers; ++li) {
                 const HLayer &L = P.L[li];
                 if (L.first) {

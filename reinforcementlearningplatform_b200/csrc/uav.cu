@@ -23,14 +23,6 @@
 #endif
 #include "uav_common.cuh"
 
-// -DUAV_RESET_NOINLINE: the auto-reset body (Philox draws, trajectory parameters) as an out-of-line call -- A/B switch for
-// the instruction-cache footprint of the step kernels' hot path
-#ifdef UAV_RESET_NOINLINE
-#define UAV_RESET_INLINE __noinline__
-#else
-#define UAV_RESET_INLINE __forceinline__
-#endif
-
 namespace {
 using namespace uavk;
 
@@ -54,8 +46,8 @@ __device__ __forceinline__ int terminal_flag(const P &p, const T *x, double time
 enum { A_S1 = 6, A_K1 = 9, A_K2 = 12, A_GAM = 15, A_LMD = 18, A_AMP = 21, A_PER = 24, A_PHS = 27, A_REF = 30, A_DREF = 33 };
 
 template <typename T, typename I>
-__device__ UAV_RESET_INLINE void att_reset_state(const P &p, const b200env_io &io, I n, I i, uint64_t seed,
-                                                int64_t off, T *x /* out: 12 states */) {
+__device__ __forceinline__ void att_reset_state(const P &p, const b200env_io &io, I n, I i, uint64_t seed,
+                                               int64_t off, T *x /* out: 12 states */) {
     const uint32_t ep = io.episode[i];
 #pragma unroll
     for (int k = 0; k < 6; ++k) { x[k] = (T)0; x[6 + k] = (T)p.init_state[6 + k]; UAV_STS(io.state, n, k, i, x[6 + k]); }
@@ -247,8 +239,8 @@ enum { P_SIG = 12, P_S1 = 15, P_AREF = 18, P_K1 = 21, P_K2 = 24, P_GAM = 27, P_L
        P_PHS = 41, P_PREF = 45, P_DPREF = 48, P_NEXT_PQR0 = 51 /* layout variant 1 only */ };
 
 template <typename T, typename I>
-__device__ UAV_RESET_INLINE void pos_reset_state(const P &p, const b200env_io &io, I n, I i, uint64_t seed,
-                                                int64_t off, T *x) {
+__device__ __forceinline__ void pos_reset_state(const P &p, const b200env_io &io, I n, I i, uint64_t seed,
+                                               int64_t off, T *x) {
     const uint32_t ep = io.episode[i];
 #pragma unroll
     for (int k = 0; k < 12; ++k) { x[k] = (T)p.init_state[k]; UAV_STS(io.state, n, k, i, x[k]); }
@@ -446,39 +438,10 @@ __device__ __forceinline__ void uav_pos_step_one(const P &p, const Consts<T> &c,
     }
 }
 
-#ifdef UAV_PREFETCH_AHEAD
-// Experiment (tools/build_variant.sh): L2 bulk prefetch of the SoA rows that the block UAV_PREFETCH_AHEAD positions
-// later in the grid will load.  Measured on B200: no gain (3.76e9 -> 3.4e9 with a persistent loop, whose blocks stay in
-// lock-step and all load at once; see DESIGN.md), so it is off by default.
-__device__ __forceinline__ void prefetch_row_l2(const void *base, size_t elsize, int64_t n, int row, int64_t start, int count) {
-    const char *ptr = static_cast<const char *>(base) + ((int64_t)row * n + start) * (int64_t)elsize;
-    const unsigned bytes = (unsigned)((size_t)count * elsize) & ~15u;
-    if (bytes && (reinterpret_cast<uintptr_t>(ptr) & 15) == 0)
-        asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(ptr), "r"(bytes));
-}
-#endif
-
 template <typename T, typename I, bool IO32>
 __global__ void __launch_bounds__(B200_BLOCK, UAV_POS_MINBLOCKS)
 uav_pos_step_kernel(const __grid_constant__ P p, const __grid_constant__ UavDerived dv,
                     const __grid_constant__ b200env_io io, int64_t n_, uint32_t flags, uint64_t seed, int64_t off) {
-#ifdef UAV_PREFETCH_AHEAD
-    {
-        const int64_t start = ((int64_t)blockIdx.x + UAV_PREFETCH_AHEAD) * B200_BLOCK;
-        if (start < n_) {
-            const int count = (int)((n_ - start) < (int64_t)B200_BLOCK ? (n_ - start) : (int64_t)B200_BLOCK);
-            const int w = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0); // warp-uniform for the compiler
-            const size_t es = sizeof(T), eio = IO32 ? sizeof(float) : sizeof(T);
-            if ((threadIdx.x & 31) == 0) {
-                for (int r = w; r < P_PREF + 9; r += B200_BLOCK / 32) {
-                    if (r < P_PREF) prefetch_row_l2(io.state, es, n_, r, start, count);
-                    else if (r < P_PREF + 8) prefetch_row_l2(io.action, eio, n_, r - P_PREF, start, count);
-                    else prefetch_row_l2(io.time, sizeof(double), n_, 0, start, count);
-                }
-            }
-        }
-    }
-#endif
     const int64_t gi = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (gi >= n_) return;
     const Consts<T> c(p.m, p.g, p.J, p.kr, p.kt, p.dt, dv);

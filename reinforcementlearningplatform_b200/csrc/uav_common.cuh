@@ -34,9 +34,8 @@
 // A thread's accesses to all fields are then ONE base register plus an immediate (f * 1024 B); with the field-major
 // layout of the other buffers ([f][n], n a run-time value) every access needed its own IMAD.WIDE and a live 64-bit register
 // pair: 144 -> 61 IMAD.WIDE in the position kernel, 0.220 -> 0.198 ms per 1 M instances (A/B on one box).  Coalescing is
-// unchanged (128 consecutive doubles per field and block).  -DB200_UAV_FIELD_MAJOR restores [f][n] (A/B only: the host
-// side follows b200env_state_layout).
-#ifndef B200_UAV_FIELD_MAJOR
+// unchanged (128 consecutive doubles per field and block).  The `n` argument of the macros is unused; it keeps their
+// call sites in the form of ld() / st() (common.cuh).
 template <typename T, typename I>
 __device__ __forceinline__ const char *uav_blk_base(const void *base, I i) {
     return static_cast<const char *>(base) +
@@ -45,10 +44,6 @@ __device__ __forceinline__ const char *uav_blk_base(const void *base, I i) {
 }
 #define UAV_LDS(base, n, field, i) (*reinterpret_cast<const T *>(uav_blk_base<T>(base, i) + (field) * (int)(128 * sizeof(T))))
 #define UAV_STS(base, n, field, i, v) (*reinterpret_cast<T *>(const_cast<char *>(uav_blk_base<T>(base, i)) + (field) * (int)(128 * sizeof(T))) = (v))
-#else
-#define UAV_LDS(base, n, field, i) ld<T>(base, n, field, i)
-#define UAV_STS(base, n, field, i, v) st<T>(base, n, field, i, v)
-#endif
 
 namespace uavk {
 
@@ -153,13 +148,8 @@ __device__ __forceinline__ void uav_rk44(const Consts<T> &c, T *x, Trig<T> t, T 
 }
 
 // FNTSMC sliding surface pieces shared by both loops (FNTSMC.py:61-66 / 128-134), one axis.
-#ifdef B200_SMC_NOINLINE
-#define SMC_INLINE __noinline__
-#else
-#define SMC_INLINE __forceinline__
-#endif
 template <typename T>
-__device__ SMC_INLINE void smc_axis(T e, T de, T k1, T gamma, T alpha, T beta, T lmd, T dt, T &integ,
+__device__ __forceinline__ void smc_axis(T e, T de, T k1, T gamma, T alpha, T beta, T lmd, T dt, T &integ,
                                          T &s_out, T &dot_s1, T &pa1_de) {
     // |e|^(alpha-1) = exp((alpha-1) log|e|) and |e|^alpha = |e|^(alpha-1) * |e|: one log, one exp and one product for the
     // two powers of FNTSMC.py:61-63 (numpy evaluates two pow()).  e = 0: 0^alpha = 0 (alpha > 0) while 0^(alpha-1) = inf.
@@ -175,12 +165,8 @@ __device__ SMC_INLINE void smc_axis(T e, T de, T k1, T gamma, T alpha, T beta, T
 #endif
     const T L = Mth<T>::log_nonneg(ae);
     const T pa1 = pow_from_log<T>(L, alpha - (T)1);
-#ifdef B200_SMC_TWO_EXP
-    const T pa = pow_from_log<T>(L, alpha);
-#else
     const T pa_ = pa1 * ae;
     const T pa = alpha == (T)0 ? (T)1 : ((ae == (T)0 && alpha > (T)0) ? (T)0 : pa_);
-#endif
     const T s = de + k1 * e + gamma * pa * Mth<T>::tanh((T)5 * e);
     dot_s1 = pow_from_log<T>(Mth<T>::log_nonneg(Mth<T>::abs(s)), beta) * Mth<T>::tanh((T)5 * s);
     integ += dot_s1 * dt;
@@ -281,34 +267,20 @@ __device__ __forceinline__ T cos_of_asin(T u, T phi_d) {
     return cs;
 }
 
-// ref_cmd.py:4-43, one channel
-template <typename T>
-__device__ __forceinline__ void ref_channel(T time, T A, T period, T bias, T phase, T &r, T &dr, T &ddr) {
-    const T w = Mth<T>::div((T)(2 * M_PI), period); // <= 1 ulp from the IEEE quotient (fastmath64.cuh), ~half the instructions
-    T s, co;
-    Mth<T>::sincos(w * time + phase, &s, &co);
-    r = A * s + bias;
-    dr = A * w * co;
-    ddr = -A * (w * w) * s;
-}
-
-// NCH channels of ref_uav / ref_inner at once.  The training scripts draw ONE period for all channels of a trajectory and
-// use the phases (pi/2, 0, 0, 0) (uav_pos_ctrl.py:404-408, train.py:61-66), so channels 1..3 have the same angular frequency
-// and the same sincos argument as their predecessor: a channel whose (period, phase) equal the previous channel's reuses
-// its w, sin and cos -- the same inputs through the same code give the same bits, so this is not an approximation -- and
-// only distinct channels pay for the quotient and the sincos (two instead of four per step in the bench configuration).
-// The test is per thread; lanes with distinct channels simply take the full path.
+// NCH channels of ref_uav / ref_inner at once (ref_cmd.py:4-43).  The training scripts draw ONE period for all channels
+// of a trajectory and use the phases (pi/2, 0, 0, 0) (uav_pos_ctrl.py:404-408, train.py:61-66), so channels 1..3 have
+// the same angular frequency and the same sincos argument as their predecessor: a channel whose (period, phase) equal
+// the previous channel's reuses its w, sin and cos -- the same inputs through the same code give the same bits, so this
+// is not an approximation -- and only distinct channels pay for the quotient and the sincos (two instead of four per
+// step in the bench configuration).  The test is per thread; lanes with distinct channels simply take the full path.
 template <typename T, int NCH>
 __device__ __forceinline__ void ref_channels(T time, const T *A, const T *period, const T *bias, const T *phase, T *r,
                                              T *dr, T *ddr) {
-#ifdef B200_UAV_REF_NO_SHARE
-#pragma unroll
-    for (int k = 0; k < NCH; ++k) ref_channel<T>(time, A[k], period[k], bias[k], phase[k], r[k], dr[k], ddr[k]);
-#else
     T w = (T)0, s = (T)0, co = (T)1;
 #pragma unroll
     for (int k = 0; k < NCH; ++k) {
         if (k == 0 || period[k] != period[k - 1] || phase[k] != phase[k - 1]) {
+            // <= 1 ulp from the IEEE quotient (fastmath64.cuh), ~half the instructions
             if (k == 0 || period[k] != period[k - 1]) w = Mth<T>::div((T)(2 * M_PI), period[k]);
             Mth<T>::sincos(w * time + phase[k], &s, &co);
         }
@@ -316,7 +288,6 @@ __device__ __forceinline__ void ref_channels(T time, const T *A, const T *period
         dr[k] = A[k] * w * co;
         ddr[k] = -A[k] * (w * w) * s;
     }
-#endif
 }
 
 

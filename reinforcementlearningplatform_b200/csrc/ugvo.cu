@@ -278,18 +278,6 @@ __device__ __forceinline__ void reset_map(const P &p, uint64_t seed, uint64_t gi
             for (int j = 0; j < NC; ++j)
                 legal[j] = !within(sx - cx[j], sy - cy[j], r[j] + p.safety_dis_st) &&
                            !within(tx - cx[j], ty - cy[j], r[j] + p.safety_dis_st);
-#ifdef UGVO_SHFL_PLACED
-            for (int q = 0; q < nobs; ++q) { // placed obstacles: broadcast from lane q
-                bool any = false;
-#pragma unroll
-                for (int j = 0; j < NC; ++j) any = any || legal[j];
-                if (!__any_sync(FULL, any)) break; // all candidates of this round are already rejected
-                const double qx = __shfl_sync(FULL, ocx, q), qy = __shfl_sync(FULL, ocy, q), qr = __shfl_sync(FULL, orr, q);
-#pragma unroll
-                for (int j = 0; j < NC; ++j)
-                    if (within(qx - cx[j], qy - cy[j], qr + r[j] + p.safety_dis_obs)) legal[j] = false;
-            }
-#else
             for (int q0 = 0; q0 < nobs; q0 += UGVO_PLACED_GROUP) { // placed obstacles, a group per vote
                 bool any = false;
 #pragma unroll
@@ -306,7 +294,6 @@ __device__ __forceinline__ void reset_map(const P &p, uint64_t seed, uint64_t gi
                     }
                 }
             }
-#endif
 #pragma unroll
             for (int j = 0; j < NC; ++j) {
                 const unsigned m = __ballot_sync(FULL, legal[j]);
@@ -651,18 +638,12 @@ ugvo_autoreset_kernel(const __grid_constant__ P p, const __grid_constant__ b200e
         // equal shares left most warps idle behind the unlucky ones (warps active 12 % of peak under ncu); every warp now
         // takes the next entry when it is free -- work[0] is the ticket counter, counted down (it ends below zero; the
         // launcher clears it before every step kernel).
-#ifdef UGVO_STATIC_DEAL
-        const int count = io.work[0];
-        for (int64_t k = gw; k < count; k += nw) {
-            const int64_t ir = io.work[1 + k];
-#else
         for (;;) {
             int tk = 0;
             if (lane == 0) tk = atomicSub(io.work, 1);
             tk = __shfl_sync(FULL, tk, 0);
             if (tk <= 0) break;
             const int64_t ir = io.work[tk];
-#endif
             WarpInst<T> e;
             warp_reset<T>(p, io, n, ir, seed, off, lane, s_pl[w], e);
             if (io.reset_obs) warp_observe<T, IO32>(p, n, ir, lane, e, io.reset_obs, s_o[w][0], s_o[w][1], s_o[w][2], s_o[w][3]);

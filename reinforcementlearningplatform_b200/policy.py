@@ -1,4 +1,4 @@
-"""Batched Gaussian actor / critic forward on device (kernel K-POLICY, csrc/policy_umma.cu; policy.cu / policy_tc.cu).
+"""Batched Gaussian actor / critic forward on device (kernel K-POLICY, csrc/policy_umma.cu; policy.cu).
 
 ``GaussianPolicy`` runs ``Proximal_Policy_Optimization2.choose_action`` (algorithm/policy_base/
 Proximal_Policy_Optimization2.py:69-76) for all N instances at once on the engine's own buffers: the policy-state
@@ -39,9 +39,11 @@ class GaussianPolicy:
         or one value per action dimension (the DPPO2 demos' ``init_std`` vector; "umma" only).
         ``actor_out_act``: "relu" (PPOActor_Gaussian.forward, utils/classes.py:563-569), "identity", or "tanh_range"
         (``tanh(mean_layer) * gain + off`` of the DPPO2 demo nets).
-        ``precision``: "umma" (tcgen05 tensor cores + TMEM, 3xTF32 split, layers up to 256 wide; default), "tf32x3"
-        (round 1's warp-level MMA kernel, layers <= 64) or "fp32" (FMA pipe, sums in k order, layers <= 64)."""
-        self.precision = {"fp32": 0, "tf32x3": 1, "umma": 2}[precision]
+        ``precision``: "umma" (tcgen05 tensor cores + TMEM, 3xTF32 split, layers up to 256 wide; default) or "fp32"
+        (FMA pipe, sums in k order, layers <= 64: the reference the tests compare "umma" with)."""
+        if precision not in ("umma", "fp32"):
+            raise ValueError(f"precision must be 'umma' or 'fp32', not {precision!r}")
+        self.precision = precision
         self._lib = _lib.load()
         self.device = torch.device(device)
         if self.device.type != "cuda":
@@ -54,7 +56,7 @@ class GaussianPolicy:
         std_arr = np.asarray(std, dtype=np.float32).reshape(-1)
         self.std_vec = None
         if std_arr.size > 1:
-            if self.precision != 2:
+            if self.precision != "umma":
                 raise ValueError("a per-dimension std needs precision='umma'")
             self.std_vec = torch.as_tensor(std_arr, device=self.device).contiguous()
             self.std = 1.0
@@ -107,7 +109,7 @@ class GaussianPolicy:
             cm = self._mlp(self.critic, 0)
             out["value"] = value if value is not None else torch.empty(n, dtype=torch.float32, device=dev)
         p = lambda t: None if t is None else C.c_void_p(t.data_ptr())
-        if self.precision == 2:
+        if self.precision == "umma":
             self._forward_umma(n, am, cm, obs_soa, noise, out)
             if noise is None:
                 self.step += 1
@@ -116,7 +118,7 @@ class GaussianPolicy:
             stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
             _lib.check(self._lib.b200_policy_forward(
                 n, None if am is None else C.byref(am), None if cm is None else C.byref(cm), p(obs_soa), p(self.a_min),
-                p(self.a_max), self.std, p(noise), self.seed, self.step, self.env_index_offset, self.precision,
+                p(self.a_max), self.std, p(noise), self.seed, self.step, self.env_index_offset, 0,  # B200_POLICY_FP32
                 p(out.get("action")),
                 p(out.get("log_prob")), p(out.get("mean")), p(out.get("value")), stream), "b200_policy_forward")
         if noise is None:

@@ -54,7 +54,7 @@ def _build(c, torch):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("precision,tol", [("fp32", 2e-6), ("tf32x3", 5e-6), ("umma", 5e-6)])
+@pytest.mark.parametrize("precision,tol", [("fp32", 2e-6), ("umma", 5e-6)])
 def test_engine_policy_matches_reference_nets(precision, tol):
     import torch
     import reinforcementlearningplatform_b200 as rlp
@@ -171,37 +171,42 @@ def test_engine_policy_matches_the_256_wide_dppo2_demo_nets():
         np.testing.assert_allclose(f(out[name]), np.tile(c[name], (reps, 1)), atol=t, err_msg=name)
     np.testing.assert_allclose(out["value"].cpu().numpy(), np.tile(c["value"], reps), atol=tol)
     with pytest.raises(ValueError):
-        rlp.GaussianPolicy(actor, critic, c["a_min"], c["a_max"], c["std"], precision="tf32x3")  # vector std: umma only
+        rlp.GaussianPolicy(actor, critic, c["a_min"], c["a_max"], c["std"], precision="fp32")  # vector std: umma only
 
 
 @pytest.mark.gpu
 def test_umma_policy_sees_optimizer_steps_and_ragged_sizes():
-    """the packed weight copy follows in-place parameter updates; n need not be a multiple of the 128-instance tile"""
+    """the packed weight copy follows in-place parameter updates; n need not be a multiple of the 128-instance tile.
+    Rows: the reference nets (policy_umma16.cu) and nets with 41 observation fields, more than policy_umma16.cu holds
+    (the resident modes of policy_umma.cu)."""
     import torch
     import reinforcementlearningplatform_b200 as rlp
     c = cases()[0]
-    actor, critic = _build(c, torch)
-    pol = rlp.GaussianPolicy(actor, critic, c["a_min"], c["a_max"], float(c["std"]))
-    ref = rlp.GaussianPolicy(actor, critic, c["a_min"], c["a_max"], float(c["std"]), precision="fp32")
-    for n in (1, 127, 129, 1000, 128 * 148 * 2 + 77):
-        obs = torch.randn(6, n, device="cuda")
-        eps = torch.randn(8, n, device="cuda")
+    torch.manual_seed(0)
+    lins = lambda dims: [torch.nn.Linear(i, o).cuda() for i, o in zip(dims[:-1], dims[1:])]
+    for actor, critic in (_build(c, torch), (lins((41, 64, 64, 32, 8)), lins((41, 64, 32, 1)))):
+        S = actor[0].in_features
+        pol = rlp.GaussianPolicy(actor, critic, c["a_min"], c["a_max"], float(c["std"]))
+        ref = rlp.GaussianPolicy(actor, critic, c["a_min"], c["a_max"], float(c["std"]), precision="fp32")
+        for n in (1, 127, 129, 1000, 128 * 148 * 2 + 77):
+            obs = torch.randn(S, n, device="cuda")
+            eps = torch.randn(8, n, device="cuda")
+            a, b = pol(obs, noise=eps, want_mean=True), ref(obs, noise=eps, want_mean=True)
+            for k in ("mean", "action", "value"):
+                assert float((a[k] - b[k]).abs().max()) <= 7e-6, (S, n, k)
+        with torch.no_grad():
+            for l in actor + critic:
+                l.weight.mul_(0.5)
+                l.bias.add_(0.1)
+        obs = torch.randn(S, 777, device="cuda")
+        eps = torch.randn(8, 777, device="cuda")
         a, b = pol(obs, noise=eps, want_mean=True), ref(obs, noise=eps, want_mean=True)
-        for k in ("mean", "action", "value"):
-            assert float((a[k] - b[k]).abs().max()) <= 7e-6, (n, k)
-    with torch.no_grad():
-        for l in actor + critic:
-            l.weight.mul_(0.5)
-            l.bias.add_(0.1)
-    obs = torch.randn(6, 777, device="cuda")
-    eps = torch.randn(8, 777, device="cuda")
-    a, b = pol(obs, noise=eps, want_mean=True), ref(obs, noise=eps, want_mean=True)
-    assert float((a["mean"] - b["mean"]).abs().max()) <= 7e-6 and float((a["value"] - b["value"]).abs().max()) <= 7e-6
+        assert float((a["mean"] - b["mean"]).abs().max()) <= 7e-6 and float((a["value"] - b["value"]).abs().max()) <= 7e-6
 
 
-def test_wide_nets_are_rejected_by_the_round1_kernels_not_silently_slow():
-    """nets that do not fit the shared-memory design of policy.cu / policy_tc.cu return B200ENV_ESIZE there (the tcgen05
-    kernel streams them; no fallback path exists)"""
+def test_wide_nets_are_rejected_by_the_fp32_kernel_not_silently_slow():
+    """nets that do not fit the shared-memory design of policy.cu return B200ENV_ESIZE there (the tcgen05 kernel streams
+    them; no fallback path exists); any precision other than B200_POLICY_FP32 (0) returns B200ENV_EPARAMS"""
     import ctypes as C
     from reinforcementlearningplatform_b200 import _lib
     lib = _lib.load()
@@ -213,7 +218,10 @@ def test_wide_nets_are_rejected_by_the_round1_kernels_not_silently_slow():
         m.w[l] = 1 << 20
         m.b[l] = 1 << 20
     m.out_act = 1
-    for precision in (0, 1):
+    for precision, want in ((0, -6), (1, -3)):
         rc = lib.b200_policy_forward(16, C.byref(m), None, C.c_void_p(1 << 20), C.c_void_p(1 << 20), C.c_void_p(1 << 20),
                                      C.c_float(0.5), None, 0, 0, 0, precision, C.c_void_p(1 << 20), None, None, None, None)
-        assert rc == -6
+        assert rc == want, precision
+    import reinforcementlearningplatform_b200 as rlp
+    with pytest.raises(ValueError):
+        rlp.GaussianPolicy(None, None, [0.0], [1.0], 1.0, precision="fp16")

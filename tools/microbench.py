@@ -56,7 +56,7 @@ def run(kind, reps=10, T=2048, N=131072, dev="cuda"):
         fn = lambda: pol(obs, action=outs["action"], log_prob=outs["log_prob"], value=outs["value"])
         flops = 2.0 * (2 * (S * 256 + 256 * 256) + 256 * A + 256)
         nbytes, units = (S + 2 * A + 1) * 4.0, n
-    elif kind in ("policy", "policy_fp32", "policy_tf32x3"):
+    elif kind in ("policy", "policy_fp32"):
         # the reference's PPOActor_Gaussian / PPOCritic shapes for UavFntsmcParamPos (state 6, 8 gains), 1 M instances
         S, A, n = 6, 8, 1 << 20
         torch.manual_seed(0)
@@ -64,7 +64,7 @@ def run(kind, reps=10, T=2048, N=131072, dev="cuda"):
         actor = [mk_l(S, 64), mk_l(64, 64), mk_l(64, 32), mk_l(32, A)]
         critic = [mk_l(S, 64), mk_l(64, 32), mk_l(32, 1)]
         pol = rlp.GaussianPolicy(actor, critic, [0.0] * A, [5.0] * A, 0.45, device=dev,
-                                 precision={"policy": "umma", "policy_fp32": "fp32", "policy_tf32x3": "tf32x3"}[kind])
+                                 precision={"policy": "umma", "policy_fp32": "fp32"}[kind])
         obs = torch.randn((S, n), generator=g, device=dev, dtype=torch.float32)
         outs = pol(obs)
         fn = lambda: pol(obs, action=outs["action"], log_prob=outs["log_prob"], value=outs["value"])

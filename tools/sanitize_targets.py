@@ -1,5 +1,5 @@
 """Small invocations of the kernels that share data across threads (shared memory / warp votes / TMEM), for
-compute-sanitizer:  compute-sanitizer --tool racecheck|memcheck python tools/sanitize_targets.py [ugvo norm policy_tc policy_umma]"""
+compute-sanitizer:  compute-sanitizer --tool racecheck|memcheck python tools/sanitize_targets.py [ugvo norm policy_umma]"""
 import os
 import sys
 
@@ -9,7 +9,7 @@ import numpy as np  # noqa: E402
 import torch  # noqa: E402
 import reinforcementlearningplatform_b200 as rlp  # noqa: E402
 
-which = sys.argv[1:] or ["ugvo", "norm", "policy_tc", "policy_umma"]
+which = sys.argv[1:] or ["ugvo", "norm", "policy_umma"]
 dev = "cuda"
 if "ugvo" in which:  # block-cooperative ray casting + warp-vote rejection sampler (auto-reset list)
     env = rlp.UGVForwardObstacleAvoidance(variant="dppo2", n_envs=777, device=dev, auto_reset=True, seed=3)
@@ -29,18 +29,15 @@ if "norm" in which:  # last-block reduction
     torch.cuda.synchronize()
     print("norm ok", float(y.std()))
 mk = lambda i, o: torch.nn.Linear(i, o).to(dev)
-if "policy_tc" in which or "policy_umma" in which:
+if "policy_umma" in which:
     actor = [mk(6, 64), mk(64, 64), mk(64, 32), mk(32, 8)]
     critic = [mk(6, 64), mk(64, 32), mk(32, 1)]
-    obs = torch.randn(6, 3000, device=dev)
-    for prec in [p for p in ("tf32x3", "umma") if ("policy_tc" in which and p == "tf32x3") or ("policy_umma" in which and p == "umma")]:
-        pol = rlp.GaussianPolicy(actor, critic, [0.0] * 8, [5.0] * 8, 0.45, precision=prec)
-        out = pol(obs)
-        torch.cuda.synchronize()
-        print("policy", prec, "ok", float(out["value"].mean()))
-    if "policy_umma" in which:
-        a2, c2 = [mk(41, 256), mk(256, 256), mk(256, 2)], [mk(41, 256), mk(256, 256), mk(256, 1)]
-        pol = rlp.GaussianPolicy(a2, c2, [-3.0, -6.28], [3.0, 6.28], [1.0, 2.09], actor_out_act="tanh_range")
-        out = pol(torch.randn(41, 700, device=dev))
-        torch.cuda.synchronize()
-        print("policy umma wide ok", float(out["value"].mean()))
+    pol = rlp.GaussianPolicy(actor, critic, [0.0] * 8, [5.0] * 8, 0.45)
+    out = pol(torch.randn(6, 3000, device=dev))
+    torch.cuda.synchronize()
+    print("policy umma ok", float(out["value"].mean()))
+    a2, c2 = [mk(41, 256), mk(256, 256), mk(256, 2)], [mk(41, 256), mk(256, 256), mk(256, 1)]
+    pol = rlp.GaussianPolicy(a2, c2, [-3.0, -6.28], [3.0, 6.28], [1.0, 2.09], actor_out_act="tanh_range")
+    out = pol(torch.randn(41, 700, device=dev))
+    torch.cuda.synchronize()
+    print("policy umma wide ok", float(out["value"].mean()))
