@@ -2,9 +2,12 @@
 """PPO2 on a vector env, entirely on the device: the vector form of
 demonstration/PPO2/PPO2-4-CartPoleAngleOnly/train.py (collection loop :186-216, learn :219-222) and of
 PPO2-4-UavFntsmcParamPos/train.py.  Under torchrun every rank owns a shard of the instances and gradients are
-all-reduced (DPPO2 as synchronous data parallelism).
+all-reduced (DPPO2 as synchronous data parallelism).  ``--algo ppo`` trains with the PPO v1 learner instead (VecPPO:
+normalised Monte-Carlo returns, full-batch epochs of the joint loss), the learner of the PPO v1 demos such as
+PPO-4-UavHoverOuterLoop (``--env uav_hover``).
 
     python examples/train_ppo2_vec.py --env cartpole_angleonly --envs 4096 --iters 30
+    python examples/train_ppo2_vec.py --algo ppo --env uav_hover --envs 65536 --steps 32 --iters 20
     python -m torch.distributed.run --nproc-per-node 2 --master-addr 127.0.0.1 examples/train_ppo2_vec.py --env soi
 """
 import argparse
@@ -18,6 +21,7 @@ import torch  # noqa: E402
 
 import reinforcementlearningplatform_b200 as rlp  # noqa: E402
 from reinforcementlearningplatform_b200 import dist as D  # noqa: E402
+from reinforcementlearningplatform_b200.ppo import VecPPO  # noqa: E402
 from reinforcementlearningplatform_b200.ppo2 import VecPPO2, reference_nets  # noqa: E402
 
 ENVS = {
@@ -28,12 +32,16 @@ ENVS = {
     # BASELINE config #5: the DPPO2 copy of UGVForwardObstacleAvoidance (41-dim observation with the 37-ray laser);
     # under torchrun this is DPPO2 as synchronous data parallelism (flat gradient all-reduce per mini-batch)
     "ugvo": (lambda **kw: rlp.UGVForwardObstacleAvoidance(variant="dppo2", **kw), dict(std=0.8, mean_act="identity")),
+    # K-UAVR's UavHover (12 observations, 3 accelerations + 3 torques), the env of the PPO v1 UavRobust demos
+    "uav_hover": (lambda **kw: rlp.uav_hover(**kw), dict(std=0.5, mean_act="identity")),
 }
 
 
 def main(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument("--env", default="cartpole_angleonly", choices=sorted(ENVS))
+    ap.add_argument("--algo", default="ppo2", choices=("ppo2", "ppo"),
+                    help="ppo2: VecPPO2 (GAE, mini-batches, gradient clip); ppo: VecPPO (the v1 learner)")
     ap.add_argument("--envs", type=int, default=4096, help="instances in total (sharded over ranks)")
     ap.add_argument("--steps", type=int, default=64, help="time steps per rollout (buffer_size)")
     ap.add_argument("--iters", type=int, default=30)
@@ -52,9 +60,9 @@ def main(argv=None):
     env = make(n_envs=n_local, device=dev, dtype=torch.float64, io_dtype=torch.float32, auto_reset=True, seed=args.seed,
                env_index_offset=off)
     actor, critic = reference_nets(env.state_dim, env.action_dim, dev, init_std=net_kw["std"], mean_act=net_kw["mean_act"])
-    agent = VecPPO2(env, actor, critic, {"buffer_size": args.steps, "K_epochs": args.epochs,
-                                          "mini_batch_size": 16384}, std=net_kw["std"],
-                    seed=args.seed, track_episodes=True)
+    agent = (VecPPO2 if args.algo == "ppo2" else VecPPO)(
+        env, actor, critic, {"buffer_size": args.steps, "K_epochs": args.epochs, "mini_batch_size": 16384},
+        std=net_kw["std"], seed=args.seed, track_episodes=True)
     env.reset(True)
     log = []
     for it in range(args.iters):

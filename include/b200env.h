@@ -429,6 +429,16 @@ B200_API int b200_adv_normalize(int64_t count, float *adv, const double *stats, 
 B200_API int b200_mc_returns(int r_dtype, int64_t T, int64_t N, const void *r, const uint8_t *done, double gamma,
                              float *returns, void *cuda_stream);
 
+/* The same scan (returns bit-identical to b200_mc_returns) that also INCREMENTS stats (device double[3]) by
+ * (sum R, sum R^2, T * N) over the stored float32 returns, summed in float64: the statistics b200_adv_normalize reads,
+ * for the v1 return normalisation R_hat = (R - mean) / (std + eps); all-reduce them over ranks first for a global one.
+ * The sums are reduced in a fixed order through scratch (device, 8-byte aligned, b200_gae_scratch_bytes(N) bytes): the
+ * same bits on every run.  Errors, all returned before any CUDA call: B200ENV_ESIZE (T <= 0, N <= 0 or N >= 2^31),
+ * B200ENV_EDTYPE (r_dtype), B200ENV_ENULL (r, done, returns, stats or scratch NULL), B200ENV_EPARAMS (scratch too small
+ * or misaligned). */
+B200_API int b200_mc_returns_stats(int r_dtype, int64_t T, int64_t N, const void *r, const uint8_t *done, double gamma,
+                                   float *returns, double *stats, void *scratch, size_t scratch_bytes, void *cuda_stream);
+
 /* K-EPISODE: episode returns, lengths and end reasons of an auto-reset rollout -- the per-episode reward sums of the
  * reference's train loops and their deterministic test episodes, for N instance columns at once.  r is [T][N] in r_dtype
  * (B200ENV_F32 / B200ENV_F64), done [T][N] u8 and flag [T][N] i32: the rollout columns the step kernels write (with T = 1
@@ -578,6 +588,22 @@ B200_API int b200_ppo2_grad(const b200_ppo2_batch *batch, const b200_mlp *actor,
                             const float *std_vec, const float *a_min, const float *a_max, float eps_clip,
                             float entropy_coef, float *grad_actor, float *grad_critic, float *loss_out, void *workspace,
                             size_t workspace_bytes, void *cuda_stream);
+
+/* The gradient of one PPO v1 update (the v1 demos' joint loss, restated):
+ *   V = critic(s);  adv = R_hat - V (no gradient through adv);  ratio and the clipped surrogate as b200_ppo2_grad;
+ *   loss = mean(-min(ratio adv, clamp(ratio, 1 - eps_clip, 1 + eps_clip) adv)) + value_coef mse(V, R_hat) - entropy_coef H
+ * batch->v_target holds R_hat (the normalised returns) and batch->adv is a caller-owned [T][N] buffer that this call
+ * WRITES at the batch's samples (one float32 subtraction R_hat - V); value (device [T][N], may be NULL) receives V there.
+ * Three launches: the critic forward over the batch (V bit-identical to the V of b200_ppo2_grad's critic), the
+ * b200_ppo2_grad kernel, and its reduction with the critic's gradient and loss multiplied by value_coef: grad_critic is
+ * value_coef times b200_ppo2_grad's critic gradient for v_target = R_hat, bit for bit, and loss_out[1] = value_coef mse.
+ * Both nets are required.  Errors, all returned before any CUDA call: B200ENV_ENULL (batch, actor, critic or a pointer
+ * b200_ppo2_grad needs), B200ENV_EPARAMS (value_coef < 0 or NaN; adv or value overlapping each other or an input:
+ * v_target, s, a, a_lp, index; and b200_ppo2_grad's), B200ENV_ESIZE (as b200_ppo2_grad).  workspace: b200_ppo2_workspace_bytes(actor, critic) bytes. */
+B200_API int b200_ppo1_grad(const b200_ppo2_batch *batch, const b200_mlp *actor, const b200_mlp *critic, float std,
+                            const float *std_vec, const float *a_min, const float *a_max, float eps_clip,
+                            float entropy_coef, float value_coef, float *value, float *grad_actor, float *grad_critic,
+                            float *loss_out, void *workspace, size_t workspace_bytes, void *cuda_stream);
 
 /* torch.nn.utils.clip_grad_norm_(params, max_norm) followed by torch.optim.Adam.step() (PPO2.py:118-121,126-129; Adam
  * eps 1e-5, :50-55) as ONE kernel over flat buffers: for each of the n_seg segments (one per net) the global gradient

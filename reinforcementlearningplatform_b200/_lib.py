@@ -177,6 +177,8 @@ def load() -> C.CDLL:
     lib.b200_adv_normalize.argtypes = [i64, vp, vp, f64, vp]
     lib.b200_mc_returns.restype = i32
     lib.b200_mc_returns.argtypes = [i32, i64, i64, vp, vp, f64, vp, vp]
+    lib.b200_mc_returns_stats.restype = i32
+    lib.b200_mc_returns_stats.argtypes = [i32, i64, i64, vp, vp, f64, vp, vp, vp, sz, vp]
     lib.b200_episode_scratch_bytes.restype = sz
     lib.b200_episode_scratch_bytes.argtypes = [i64]
     lib.b200_episode_scan.restype = i32
@@ -205,6 +207,8 @@ def load() -> C.CDLL:
     lib.b200_ppo2_workspace_bytes.argtypes = [vp, vp]
     lib.b200_ppo2_grad.restype = i32
     lib.b200_ppo2_grad.argtypes = [vp, vp, vp, f32, vp, vp, vp, f32, f32, vp, vp, vp, vp, sz, vp]
+    lib.b200_ppo1_grad.restype = i32
+    lib.b200_ppo1_grad.argtypes = [vp, vp, vp, f32, vp, vp, vp, f32, f32, f32, vp, vp, vp, vp, vp, sz, vp]
     lib.b200_adam_step.restype = i32
     lib.b200_adam_step.argtypes = [i32, C.POINTER(i64), C.POINTER(i64), C.POINTER(f32), vp, vp, vp, vp, i64, f32, f32, f32,
                                    f32, f32, vp, vp]

@@ -30,6 +30,32 @@ __device__ __forceinline__ double warp_sum(double v) {
     return v;
 }
 
+// per-block part of the (sum, sum of squares, count) statistics: warp sums, then the block's warps in order; thread 0
+// writes the block's two partials to scratch (partial[2 b], partial[2 b + 1], added up by gae_stats_reduce_kernel) or,
+// without scratch, adds them atomically
+template <int WARPS>
+__device__ __forceinline__ void block_stats(double s1, double s2, int64_t T, int64_t N, double *stats, double *partial) {
+    __shared__ double sh1[WARPS], sh2[WARPS];
+    s1 = warp_sum(s1);
+    s2 = warp_sum(s2);
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    if (lane == 0) { sh1[w] = s1; sh2[w] = s2; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double a = 0, b = 0;
+#pragma unroll
+        for (int k = 0; k < WARPS; ++k) { a += sh1[k]; b += sh2[k]; }
+        if (partial) {                      // deterministic path: block b owns partial[2 b], partial[2 b + 1]
+            partial[2 * (int64_t)blockIdx.x] = a;
+            partial[2 * (int64_t)blockIdx.x + 1] = b;
+        } else {
+            atomicAdd(stats + 0, a);
+            atomicAdd(stats + 1, b);
+            if (blockIdx.x == 0) atomicAdd(stats + 2, (double)T * (double)N);
+        }
+    }
+}
+
 // how the two masks of the scan are stored: FloatMasks = the reference's float32 `done` / `success` columns
 // (RolloutBuffer.to_tensor, utils/classes.py:292-301); FlagMasks = what the step kernels write into a device-resident
 // rollout (rollout.py): `done` as u8 and the terminal flag as i32, with success = done && flag != timeout_flag -- the
@@ -110,27 +136,7 @@ gae_kernel(int64_t T, int64_t N, const float *__restrict__ r, const float *__res
             s2 += (double)a * (double)a;
         }
     }
-    if (stats) {
-        __shared__ double sh1[GAE_BLOCK / 32], sh2[GAE_BLOCK / 32];
-        s1 = warp_sum(s1);
-        s2 = warp_sum(s2);
-        const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-        if (lane == 0) { sh1[w] = s1; sh2[w] = s2; }
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            double a = 0, b = 0;
-#pragma unroll
-            for (int k = 0; k < GAE_BLOCK / 32; ++k) { a += sh1[k]; b += sh2[k]; }
-            if (partial) {                      // deterministic path: block b owns partial[2 b], partial[2 b + 1]
-                partial[2 * (int64_t)blockIdx.x] = a;
-                partial[2 * (int64_t)blockIdx.x + 1] = b;
-            } else {
-                atomicAdd(stats + 0, a);
-                atomicAdd(stats + 1, b);
-                if (blockIdx.x == 0) atomicAdd(stats + 2, (double)T * (double)N);
-            }
-        }
-    }
+    if (stats) block_stats<GAE_BLOCK / 32>(s1, s2, T, N, stats, partial);
 }
 
 // acc_mode 2: the same recurrence as a warp-level scan ALONG TIME, for rollouts with few columns (the reference's own
@@ -248,37 +254,54 @@ adv_normalize_kernel(int64_t count, float *__restrict__ adv, const double *__res
 //     rewards = torch.tensor(np.array(rewards), dtype=torch.float32)
 // buffer.r is a float64 numpy array, so the recurrence runs in float64 (separately rounded multiply and add) and only
 // the stored return is rounded to float32.  One thread per instance column, like K-GAE.
-template <typename TR>
+// STATS: the scan also sums the stored float32 returns and their squares in float64 and hands them to K-GAE's fixed-order
+// reduction (block_stats into scratch, then gae_stats_reduce_kernel): the statistics of the v1 return normalisation.
+// STATS = false is b200_mc_returns, instruction for instruction the kernel it was before the statistics existed.
+template <typename TR, bool STATS>
 __global__ void __launch_bounds__(GAE_BLOCK)
 mc_returns_kernel(int64_t T, int64_t N, const TR *__restrict__ r, const uint8_t *__restrict__ done, double gamma,
-                  float *__restrict__ ret) {
+                  float *__restrict__ ret, double *partial) {
     const int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (n >= N) return;
-    double acc = 0.0;
-    int64_t t = T - 1;
-    constexpr int RET_UNROLL = 8;
-    for (; t >= RET_UNROLL - 1; t -= RET_UNROLL) {
-        double rr[RET_UNROLL];
-        uint8_t dd[RET_UNROLL];
+    if (!STATS && n >= N) return;
+    double s1 = 0.0, s2 = 0.0;
+    if (n < N) {
+        double acc = 0.0;
+        int64_t t = T - 1;
+        constexpr int RET_UNROLL = 8;
+        for (; t >= RET_UNROLL - 1; t -= RET_UNROLL) {
+            double rr[RET_UNROLL];
+            uint8_t dd[RET_UNROLL];
 #pragma unroll
-        for (int u = 0; u < RET_UNROLL; ++u) {
-            const int64_t idx = (t - u) * N + n;
-            rr[u] = (double)__ldcs(r + idx);
-            dd[u] = __ldcs(done + idx);
+            for (int u = 0; u < RET_UNROLL; ++u) {
+                const int64_t idx = (t - u) * N + n;
+                rr[u] = (double)__ldcs(r + idx);
+                dd[u] = __ldcs(done + idx);
+            }
+#pragma unroll
+            for (int u = 0; u < RET_UNROLL; ++u) {
+                if (dd[u]) acc = 0.0;
+                acc = __dadd_rn(rr[u], __dmul_rn(gamma, acc));
+                const float rf = (float)acc;
+                __stcs(ret + (t - u) * N + n, rf);
+                if (STATS) {
+                    s1 += (double)rf;
+                    s2 += (double)rf * (double)rf;
+                }
+            }
         }
-#pragma unroll
-        for (int u = 0; u < RET_UNROLL; ++u) {
-            if (dd[u]) acc = 0.0;
-            acc = __dadd_rn(rr[u], __dmul_rn(gamma, acc));
-            __stcs(ret + (t - u) * N + n, (float)acc);
+        for (; t >= 0; --t) {
+            const int64_t idx = t * N + n;
+            if (done[idx]) acc = 0.0;
+            acc = __dadd_rn((double)r[idx], __dmul_rn(gamma, acc));
+            const float rf = (float)acc;
+            ret[idx] = rf;
+            if (STATS) {
+                s1 += (double)rf;
+                s2 += (double)rf * (double)rf;
+            }
         }
     }
-    for (; t >= 0; --t) {
-        const int64_t idx = t * N + n;
-        if (done[idx]) acc = 0.0;
-        acc = __dadd_rn((double)r[idx], __dmul_rn(gamma, acc));
-        ret[idx] = (float)acc;
-    }
+    if (STATS) block_stats<GAE_BLOCK / 32>(s1, s2, T, N, nullptr, partial);
 }
 
 } // namespace
@@ -344,14 +367,37 @@ extern "C" B200_API int b200_adv_normalize(int64_t count, float *adv, const doub
     return b200_check_launch();
 }
 
+namespace {
+int mc_returns_launch(int r_dtype, int64_t T, int64_t N, const void *r, const uint8_t *done, double gamma, float *returns,
+                      double *stats, double *partial, cudaStream_t s) {
+    const unsigned grid = (unsigned)((N + GAE_BLOCK - 1) / GAE_BLOCK);
+    if (!stats) {
+        if (r_dtype == B200ENV_F64) mc_returns_kernel<double, false><<<grid, GAE_BLOCK, 0, s>>>(T, N, (const double *)r, done, gamma, returns, nullptr);
+        else mc_returns_kernel<float, false><<<grid, GAE_BLOCK, 0, s>>>(T, N, (const float *)r, done, gamma, returns, nullptr);
+        return b200_check_launch();
+    }
+    if (r_dtype == B200ENV_F64) mc_returns_kernel<double, true><<<grid, GAE_BLOCK, 0, s>>>(T, N, (const double *)r, done, gamma, returns, partial);
+    else mc_returns_kernel<float, true><<<grid, GAE_BLOCK, 0, s>>>(T, N, (const float *)r, done, gamma, returns, partial);
+    gae_stats_reduce_kernel<<<1, 256, 0, s>>>((int64_t)grid, partial, (double)T * (double)N, stats);
+    return b200_check_launch();
+}
+} // namespace
+
 extern "C" B200_API int b200_mc_returns(int r_dtype, int64_t T, int64_t N, const void *r, const uint8_t *done,
                                         double gamma, float *returns, void *cuda_stream) {
     if (T <= 0 || N <= 0) return B200ENV_ESIZE;
     if (r_dtype != B200ENV_F64 && r_dtype != B200ENV_F32) return B200ENV_EDTYPE;
     if (!r || !done || !returns) return B200ENV_ENULL;
-    cudaStream_t s = (cudaStream_t)cuda_stream;
-    const unsigned grid = (unsigned)((N + GAE_BLOCK - 1) / GAE_BLOCK);
-    if (r_dtype == B200ENV_F64) mc_returns_kernel<double><<<grid, GAE_BLOCK, 0, s>>>(T, N, (const double *)r, done, gamma, returns);
-    else mc_returns_kernel<float><<<grid, GAE_BLOCK, 0, s>>>(T, N, (const float *)r, done, gamma, returns);
-    return b200_check_launch();
+    return mc_returns_launch(r_dtype, T, N, r, done, gamma, returns, nullptr, nullptr, (cudaStream_t)cuda_stream);
+}
+
+extern "C" B200_API int b200_mc_returns_stats(int r_dtype, int64_t T, int64_t N, const void *r, const uint8_t *done,
+                                              double gamma, float *returns, double *stats, void *scratch,
+                                              size_t scratch_bytes, void *cuda_stream) {
+    if (T <= 0 || N <= 0 || N >= ((int64_t)1 << 31)) return B200ENV_ESIZE;
+    if (r_dtype != B200ENV_F64 && r_dtype != B200ENV_F32) return B200ENV_EDTYPE;
+    if (!r || !done || !returns || !stats || !scratch) return B200ENV_ENULL;
+    if (scratch_bytes < b200_gae_scratch_bytes(N) || ((uintptr_t)scratch & 7)) return B200ENV_EPARAMS;
+    return mc_returns_launch(r_dtype, T, N, r, done, gamma, returns, stats, static_cast<double *>(scratch),
+                             (cudaStream_t)cuda_stream);
 }

@@ -536,6 +536,11 @@ struct ReduceArgs {
     int ent_slot, A;
     float ent_coef, std_;
     const float *std_vec;
+    // factor of slot 1's gradient and loss, i.e. of the critic of a two-net launch: value_coef for the v1 critic (c_v mse
+    // of the joint loss), 1 for PPO2.  Selected by slot (j == 1) rather than indexed: an indexed per-slot factor moved the
+    // kernel's block and address arithmetic off the uniform datapath, and b200_ppo2_grad measured 3.7 % (4096 samples)
+    // and 4.1 % (16,384) slower than the parent on a B200 at 1000 W (profiles/ppo1/README.md)
+    float scale1;
 };
 __global__ void __launch_bounds__(256) ppo2_reduce_kernel(const __grid_constant__ ReduceArgs a) {
     const int j = (a.nets > 1 && (int)blockIdx.x >= a.first_block[1]) ? 1 : 0;
@@ -555,17 +560,103 @@ __global__ void __launch_bounds__(256) ppo2_reduce_kernel(const __grid_constant_
         for (int q = 0; q < 8; ++q) t += v[q];
     }
     for (; b < nblk; ++b) t += __ldcg(base + (size_t)b * stride);
+    const float scale = j == 1 ? a.scale1 : 1.0f;
     if (p < P) {
-        a.grad[j][p] = t;
+        a.grad[j][p] = t * scale;
         return;
     }
-    float loss = t * a.inv_count;
+    float loss = t * a.inv_count * scale;
     if (j == a.ent_slot) {
         float h = 0.0f;
         for (int d = 0; d < a.A; ++d) h += 0.5f + 0.9189385332046727f + logf(a.std_vec ? a.std_vec[d] : a.std_);
         loss -= a.ent_coef * h;
     }
     a.loss_out[j] = loss;
+}
+
+// PPO v1 advantage (the joint loss of b200_ppo1_grad): adv = R_hat - V(s) with the CURRENT critic at the batch's samples,
+// before ppo2_grad_kernel reads adv.  Same sample selection, tile, shared-memory layout and fwd_layer calls as the critic
+// blocks of ppo2_grad_kernel, so V is bit-identical to the V those blocks compute from the same weights.  A separate
+// launch rather than the critic forward inside the actor's blocks: that would put both nets' weights into those blocks
+// and change the shipped gradient kernel; this costs one more read of the observations.
+struct AdvArgs {
+    LNet net;                    // the critic
+    int S;
+    int64_t T, N, first, count;
+    const float *s, *ret_hat;
+    const int64_t *index;
+    uint64_t perm_key;
+    int perm_half_bits;
+    float *adv, *value;          // value may be NULL
+};
+__global__ void __launch_bounds__(LT, BLOCKS_PER_SM) ppo1_advantage_kernel(const __grid_constant__ AdvArgs A) {
+    extern __shared__ __align__(16) float sm[];
+    __shared__ int s_t[TM], s_i[TM];
+    const LNet &net = A.net;
+    const int L = net.n_layers;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int sg = (lane & 3) + 4 * warp, ng = lane >> 2;
+    for (int l = 0; l < L; ++l) {
+        const LLayer &Ly = net.L[l];
+        const int pw = Ly.K + 4;
+        for (int e = tid; e < Ly.N * pw; e += LT) {
+            const int n = e / pw, k = e - n * pw;
+            sm[Ly.w_off + e] = (n < Ly.n_real && k < Ly.k_real) ? __ldg(Ly.w + n * Ly.k_real + k) : 0.0f;
+        }
+        for (int n = tid; n < Ly.N; n += LT) sm[Ly.b_off + n] = n < Ly.n_real ? __ldg(Ly.b + n) : 0.0f;
+    }
+    const int64_t tiles = (A.count + TM - 1) / TM;
+    const LLayer &L0 = net.L[0];
+    float *gout = sm + net.gout_off;
+    const int pgo = net.L[L - 1].N + 4;
+    for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
+        __syncthreads();   // the previous tile's last reads of H and s_t / s_i are done
+        if (tid < TM) {
+            const int64_t j = tile * TM + tid;
+            int t = -1, i = 0;
+            if (j < A.count) {
+                const int64_t b = A.index ? A.index[A.first + j] : perm_index(A.perm_key, A.first + j, A.T * A.N, A.perm_half_bits);
+                t = (int)(b / A.N);
+                i = (int)(b - (int64_t)t * A.N);
+            }
+            s_t[tid] = t;
+            s_i[tid] = i;
+        }
+        __syncthreads();
+        {   // H_0 = the gathered observations, zero-padded to K_0 (thread = sample s, fields q, q + 4, ...)
+            float *H0 = sm + L0.h_off;
+            const int p0 = L0.K + 4;
+            const int s = tid & (TM - 1), q = tid >> TM_LOG2;
+            const int t = s_t[s];
+            const int64_t i = s_i[s], tt = t < 0 ? 0 : t;
+            for (int k = q; k < L0.K; k += LT / TM)
+                H0[s * p0 + k] = (t >= 0 && k < A.S) ? __ldg(A.s + (tt * A.S + k) * A.N + i) : 0.0f;
+        }
+        __syncthreads();
+#pragma unroll
+        for (int l = 0; l < LMAX; ++l) {
+            if (l < L) {
+                const LLayer &Ly = net.L[l];
+                const bool last = l == L - 1;
+                float *out = last ? gout : sm + net.L[l + 1 < LMAX ? l + 1 : l].h_off;
+                const float *H = sm + Ly.h_off, *W = sm + Ly.w_off, *bs = sm + Ly.b_off;
+                const int ph = Ly.K + 4, po = Ly.N + 4;
+                switch (Ly.N >> 3) {
+                case 1: fwd_layer<1>(H, ph, W, ph, bs, Ly.K, out, po, !last, sg, ng); break;
+                case 2: fwd_layer<2>(H, ph, W, ph, bs, Ly.K, out, po, !last, sg, ng); break;
+                case 4: fwd_layer<4>(H, ph, W, ph, bs, Ly.K, out, po, !last, sg, ng); break;
+                default: fwd_layer<8>(H, ph, W, ph, bs, Ly.K, out, po, !last, sg, ng); break;
+                }
+                __syncthreads();
+            }
+        }
+        if (tid < TM && s_t[tid] >= 0) {
+            const int64_t b = (int64_t)s_t[tid] * A.N + s_i[tid];
+            const float v = gout[tid * pgo];
+            A.adv[b] = __fsub_rn(__ldg(A.ret_hat + b), v);
+            if (A.value) A.value[b] = v;
+        }
+    }
 }
 
 // ------------------------------------------------------------------------------------------------ clip + Adam
@@ -743,7 +834,7 @@ int make_plan(const b200_ppo2_batch *bt, const b200_mlp *actor, const b200_mlp *
     return B200ENV_OK;
 }
 
-int launch_grad(Plan &pl, cudaStream_t stream) {
+int launch_grad(Plan &pl, cudaStream_t stream, float critic_scale = 1.0f) {
     static size_t configured[64] = {0};
     int dev = 0;
     cudaGetDevice(&dev);
@@ -789,6 +880,7 @@ int launch_grad(Plan &pl, cudaStream_t stream) {
     r.nets = pl.nets;
     r.nblk[0] = pl.a.nblk[0]; r.nblk[1] = pl.a.nblk[1];
     r.inv_count = pl.a.inv_count;
+    r.scale1 = critic_scale;   // slot 1 exists only in two-net launches, and is the critic there
     r.ent_slot = (pl.a.net_of_y[0] == 0 && pl.a.entropy_coef != 0.0f) ? 0 : -1;
     r.A = pl.a.A; r.ent_coef = pl.a.entropy_coef; r.std_ = pl.a.std_; r.std_vec = pl.a.std_vec;
     ppo2_reduce_kernel<<<blocks, 256, 0, stream>>>(r);
@@ -850,6 +942,66 @@ extern "C" B200_API int b200_ppo2_grad(const b200_ppo2_batch *batch, const b200_
                        loss_out, workspace, workspace_bytes, &pl);
     if (rc) return rc;
     return launch_grad(pl, (cudaStream_t)cuda_stream);
+}
+
+namespace {
+bool overlaps(const void *a, size_t a_bytes, const void *b, size_t b_bytes) {
+    const uintptr_t x = (uintptr_t)a, y = (uintptr_t)b;
+    return x < y + b_bytes && y < x + a_bytes;
+}
+} // namespace
+
+extern "C" B200_API int b200_ppo1_grad(const b200_ppo2_batch *batch, const b200_mlp *actor, const b200_mlp *critic,
+                                       float std_, const float *std_vec, const float *a_min, const float *a_max,
+                                       float eps_clip, float entropy_coef, float value_coef, float *value,
+                                       float *grad_actor, float *grad_critic, float *loss_out, void *workspace,
+                                       size_t workspace_bytes, void *cuda_stream) {
+    if (!batch || !actor || !critic) return B200ENV_ENULL;
+    if (!(value_coef >= 0.0f)) return B200ENV_EPARAMS;
+    Plan pl;
+    int rc = make_plan(batch, actor, critic, std_, std_vec, a_min, a_max, eps_clip, entropy_coef, grad_actor, grad_critic,
+                       loss_out, workspace, workspace_bytes, &pl);
+    if (rc) return rc;
+    {   // adv and value are written by the advantage launch while R_hat, s, a, a_lp and the index are read by both launches:
+        // an output that overlaps an input (e.g. adv == v_target for an in-place call) would be read back as that input
+        const size_t tn = (size_t)pl.a.T * (size_t)pl.a.N * sizeof(float);
+        const size_t tan_ = tn * (size_t)pl.a.A, tsn = tn * (size_t)pl.a.S;
+        const void *in[5] = {batch->v_target, batch->s, batch->a, batch->a_lp, batch->index};
+        const size_t in_bytes[5] = {tn, tsn, tan_, tan_, (size_t)(pl.a.first + pl.a.count) * sizeof(int64_t)};
+        const void *out[2] = {batch->adv, value};
+        for (int o = 0; o < 2; ++o) {
+            if (!out[o]) continue;
+            for (int k = 0; k < 5; ++k)
+                if (in[k] && overlaps(out[o], tn, in[k], in_bytes[k])) return B200ENV_EPARAMS;
+        }
+        if (value && overlaps(value, tn, batch->adv, tn)) return B200ENV_EPARAMS;
+    }
+    AdvArgs v = {};
+    v.net = pl.a.net[1];
+    v.S = pl.a.S;
+    v.T = pl.a.T; v.N = pl.a.N; v.first = pl.a.first; v.count = pl.a.count;
+    v.s = batch->s; v.ret_hat = batch->v_target;
+    v.index = batch->index;
+    v.perm_key = pl.a.perm_key;
+    v.perm_half_bits = pl.a.perm_half_bits;
+    v.adv = const_cast<float *>(batch->adv);   // the caller-owned [T][N] buffer this call fills
+    v.value = value;
+    const size_t smem = (size_t)v.net.smem_floats * sizeof(float);
+    cudaStream_t stream = (cudaStream_t)cuda_stream;
+    static size_t configured[64] = {0};
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (dev < 0 || dev >= 64) dev = 0;
+    if (smem > 48 * 1024 && smem > configured[dev]) {
+        if (cudaFuncSetAttribute(ppo1_advantage_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+            return b200_check_launch();
+        configured[dev] = smem;
+    }
+    const int64_t tiles = (v.count + TM - 1) / TM;
+    const int cap = grid_cap();
+    ppo1_advantage_kernel<<<(unsigned)(tiles < cap ? tiles : cap), LT, smem, stream>>>(v);
+    if ((rc = b200_check_launch())) return rc;
+    return launch_grad(pl, stream, value_coef);
 }
 
 extern "C" B200_API int b200_adam_step(int n_seg, const int64_t *seg_off, const int64_t *seg_len, const float *lr,

@@ -82,17 +82,28 @@ def normalize_advantage(adv: torch.Tensor, stats: torch.Tensor, eps: float = 1e-
     return adv
 
 
-def mc_returns(r: torch.Tensor, done_u8: torch.Tensor, gamma: float) -> torch.Tensor:
+def mc_returns(r: torch.Tensor, done_u8: torch.Tensor, gamma: float, stats: torch.Tensor = None) -> torch.Tensor:
     """Monte-Carlo returns of PPO / DPPO v1 (Proximal_Policy_Optimization.py:113-119) over a time-major ``[T, N]``
-    rollout: ``r`` float64 (like ``RolloutBuffer.r``) or float32, ``done_u8`` uint8; float64 recurrence, float32 out."""
+    rollout: ``r`` float64 (like ``RolloutBuffer.r``) or float32, ``done_u8`` uint8; float64 recurrence, float32 out.
+    ``stats``: a CUDA float64 ``[3]`` tensor that is INCREMENTED by (sum R, sum R^2, T * N), summed in a fixed order --
+    what :func:`normalize_advantage` reads to normalise the returns."""
     if not (r.is_cuda and r.dim() == 2 and r.is_contiguous() and r.dtype in (torch.float32, torch.float64)):
         raise ValueError("mc_returns: r must be a contiguous CUDA [T, N] float32/float64 tensor")
     if not (done_u8.dtype == torch.uint8 and done_u8.shape == r.shape and done_u8.is_contiguous()):
         raise ValueError("mc_returns: done must be a contiguous uint8 [T, N] tensor")
+    if stats is not None and not (stats.is_cuda and stats.dtype == torch.float64 and stats.numel() == 3
+                                  and stats.is_contiguous()):
+        raise ValueError("mc_returns: stats must be a contiguous CUDA float64 tensor of 3 elements")
     T, N = r.shape
     out = torch.empty(T, N, dtype=torch.float32, device=r.device)
+    dt = _lib.F64 if r.dtype == torch.float64 else _lib.F32
     with torch.cuda.device(r.device):
         stream = C.c_void_p(torch.cuda.current_stream(r.device).cuda_stream)
-        _lib.check(_lib.load().b200_mc_returns(_lib.F64 if r.dtype == torch.float64 else _lib.F32, T, N, _p(r),
-                                               _p(done_u8), float(gamma), _p(out), stream), "b200_mc_returns")
+        if stats is None:
+            _lib.check(_lib.load().b200_mc_returns(dt, T, N, _p(r), _p(done_u8), float(gamma), _p(out), stream),
+                       "b200_mc_returns")
+        else:
+            scr = _scratch(N, r.device)
+            _lib.check(_lib.load().b200_mc_returns_stats(dt, T, N, _p(r), _p(done_u8), float(gamma), _p(out), _p(stats),
+                                                         _p(scr), scr.numel() * 8, stream), "b200_mc_returns_stats")
     return out

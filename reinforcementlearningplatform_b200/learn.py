@@ -131,6 +131,25 @@ class FusedPPO2Update:
                 self.eps_clip, self.entropy_coef, p(self.grad), C.c_void_p(self.grad.data_ptr() + 4 * o), p(self.loss),
                 p(self.workspace), self.workspace.numel(), self._stream()), "b200_ppo2_grad")
 
+    def ppo1_grad_step(self, s, a, a_lp, ret_hat, adv_out, value_coef: float, first: int, count: int, perm_key: int = 0,
+                       index: Optional[torch.Tensor] = None, value: Optional[torch.Tensor] = None) -> None:
+        """Gradient of the PPO v1 joint loss for one batch (``b200_ppo1_grad``) -> ``self.grad``; ``self.loss`` =
+        (actor loss with the entropy term, ``value_coef`` x mse).  ``ret_hat [T, N]``: the normalised returns;
+        ``adv_out [T, N]`` receives ``ret_hat - critic(s)`` at the batch's samples, ``value`` (optional) ``critic(s)``."""
+        b = self._batch(s, a, a_lp, adv_out, ret_hat, first, count, perm_key, index)
+        if value is not None and not (value.is_cuda and value.dtype == torch.float32 and value.is_contiguous()
+                                      and tuple(value.shape) == tuple(ret_hat.shape)):
+            raise ValueError("K-LEARN: value must be a contiguous CUDA float32 [T, N] tensor")
+        am, cm = self.params.mlp(0, self.out_act), self.params.mlp(1, 0)
+        p = lambda t: None if t is None else C.c_void_p(t.data_ptr())
+        o = self.params.net_off[1]
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.b200_ppo1_grad(
+                C.byref(b), C.byref(am), C.byref(cm), self.std, p(self.std_vec), p(self.a_min), p(self.a_max),
+                self.eps_clip, self.entropy_coef, float(value_coef), p(value), p(self.grad),
+                C.c_void_p(self.grad.data_ptr() + 4 * o), p(self.loss), p(self.workspace), self.workspace.numel(),
+                self._stream()), "b200_ppo1_grad")
+
     def adam_step(self, grad_scale: float = 1.0) -> None:
         """clip_grad_norm_ + Adam over both parameter segments (one launch)."""
         self.step_count += 1

@@ -120,6 +120,26 @@ class VecPPO2:
         n1, m1 = float(ms.n), float(np.asarray(ms.mean).reshape(-1)[0])
         return (n1 * m1 - n0 * m0) / max(n1 - n0, 1.0)
 
+    def set_action_std(self, std) -> None:
+        """Change the exploration std between iterations: ``self.std``, the sampling policy of ``collect()`` and the
+        learner's log-probabilities change together.  ``std`` keeps the form the agent was built with: a scalar for a
+        scalar std, a vector of the same length for a per-dimension one; anything else raises ``ValueError``."""
+        new = np.asarray(std.detach().cpu() if torch.is_tensor(std) else std, dtype=np.float32)
+        if new.ndim > 1 or new.size != self.std.numel():
+            raise ValueError(f"set_action_std: expected {'a scalar' if self.std.numel() == 1 else f'{self.std.numel()} values'}, "
+                             f"got shape {new.shape}")
+        if not (np.isfinite(new).all() and (new > 0).all()):
+            raise ValueError("set_action_std: std must be finite and positive")
+        new = new.reshape(-1)
+        self.std.copy_(torch.as_tensor(new, device=self.std.device))
+        for holder in (self.policy, self.fused):
+            if holder is None:
+                continue
+            if holder.std_vec is not None:
+                holder.std_vec.copy_(self.std)
+            else:
+                holder.std = float(new[0])
+
     # ------------------------------------------------------------------ update (PPO2.py:78-170)
     def _log_prob_entropy(self, s, a):
         mean = self.actor(s)
