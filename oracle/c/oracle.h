@@ -43,7 +43,7 @@ int oracle_reset(int env_id, int64_t n, const void *params, const oracle_io *io,
                  uint64_t seed, int64_t env_index_offset);
 int oracle_observe(int env_id, int64_t n, const void *params, const oracle_io *io);
 
-/* Philox4x32-10 block (Random123 known-answer tests are in tests/test_philox.py) */
+/* Philox4x32-10 block (Random123 known-answer tests are in tests/test_policy_routes_gpu.py) */
 void oracle_philox4x32_10(const uint32_t ctr[4], const uint32_t key[2], uint32_t out[4]);
 
 /* GAE reverse scan, float32 sequential exactly like the Python loop under numpy >= 2

@@ -89,7 +89,7 @@ __device__ __forceinline__ void dense(const float *__restrict__ wt, const float 
     for (int c = 0; c < CH; ++c) {
         float v = acc[c];
         if (act == 2) v = tanhf(v);
-        else if (act == 1) v = fmaxf(v, 0.0f);
+        else if (act == 1) v = policy_fmax_nan(v, 0.0f);
         buf[c * PB + t] = v;
     }
 }

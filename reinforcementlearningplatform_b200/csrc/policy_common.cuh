@@ -52,6 +52,21 @@ __device__ __forceinline__ void policy_dims_fill(const PolicyIO &a, int A, float
     }
 }
 
+// min / max that return NaN when either input is NaN (PTX min.NaN / max.NaN, sm_80+), one instruction like fminf / fmaxf,
+// which would return the other input.  torch's choose_action turns a NaN observation into NaN outputs; with these the
+// hidden-layer clamp, the relu head and the action clamp do too, instead of handing a diverged instance a plausible
+// finite action.
+__device__ __forceinline__ float policy_fmin_nan(float a, float b) {
+    float d;
+    asm("min.NaN.f32 %0, %1, %2;" : "=f"(d) : "f"(a), "f"(b));
+    return d;
+}
+__device__ __forceinline__ float policy_fmax_nan(float a, float b) {
+    float d;
+    asm("max.NaN.f32 %0, %1, %2;" : "=f"(d) : "f"(a), "f"(b));
+    return d;
+}
+
 // tanh on the SFU (ex2.approx + rcp.approx), absolute error <= 4e-7: the range-mapped actor head
 __device__ __forceinline__ float policy_tanh_sfu(float x) {
     float e, r;
@@ -123,7 +138,7 @@ __device__ __forceinline__ void policy_sample_store_fn(const PolicyIO &a, int64_
                     m = policy_tanh_sfu(m) * (amax - off) + off;
                 }
                 float act = fmaf(sd, e[q], m);                                   // dist.sample()
-                act = fmaxf(fminf(act, amax), amin);
+                act = policy_fmax_nan(policy_fmin_nan(act, amax), amin);
                 const float d = act - m;                                         // Normal.log_prob
                 const float lp = -(d * d) * iv - lstd;
                 __stcs(p_act + (int64_t)q * n, act);

@@ -434,7 +434,7 @@ __device__ __forceinline__ void epilogue_loop(const UArgs &a, int64_t n, unsigne
 #pragma unroll
                     for (int j = 0; j < 16; ++j) {
                         float m = fmaf(__uint_as_float(v[j]), zs, bias_s[L.b_off + j]);
-                        if (L.out_act == 1) m = fmaxf(m, 0.0f);
+                        if (L.out_act == 1) m = policy_fmax_nan(m, 0.0f);
                         scr[j * TILE_M] = m;
                     }
                     pending_A = L.n_real;

@@ -88,9 +88,10 @@ __device__ __forceinline__ void epi16_compute(const uint32_t (&v)[16], const flo
     for (int j = 0; j < 16; ++j) t[j] = fmaf(__uint_as_float(v[j]), zs, t[j]);
     // one reciprocal for two activations: 1 / a = b / (a b), 1 / b = a / (a b); the exponent is clamped so that a b stays
     // finite (2^60 + 1: tanh is 1 to the last bit long before).  1.5 instead of 2 MUFU per activation, +2 issue slots:
-    // 0.2218 vs 0.2255 ms per 1 M instances for one reciprocal each (A/B on one box, twice).
+    // 0.2218 vs 0.2255 ms per 1 M instances for one reciprocal each (A/B on one box, twice).  The clamp keeps a NaN
+    // (fminf would turn it into 60, i.e. tanh = 1).
 #pragma unroll
-    for (int j = 0; j < 16; ++j) t[j] = fminf(t[j], 60.0f);
+    for (int j = 0; j < 16; ++j) t[j] = policy_fmin_nan(t[j], 60.0f);
 #pragma unroll
     for (int j = 0; j < 16; ++j) asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(t[j]) : "f"(t[j]));
 #pragma unroll
@@ -233,7 +234,7 @@ policy_umma16_kernel(const __grid_constant__ HArgs a, int64_t n) {
 #pragma unroll
                     for (int j = 0; j < 16; ++j) {
                         float m = fmaf(__uint_as_float(v[j]), zs, bias_s[L.b_off + j]);
-                        if (L.out_act == 1) m = fmaxf(m, 0.0f);
+                        if (L.out_act == 1) m = policy_fmax_nan(m, 0.0f);
                         scr[j * H_TILE] = m;
                     }
                     pending_A = L.n_real;
