@@ -635,6 +635,58 @@ B200_API int b200_ppo2_learn(const b200_ppo2_batch *batch, const b200_mlp *actor
                              float *grad, float *exp_avg, float *exp_avg_sq, float *loss_out, void *workspace,
                              size_t workspace_bytes, void *cuda_stream);
 
+/* ------------------------------------------------------------- DQN / Double DQN (K-DQN) */
+
+/* Epsilon-greedy action of n instances from a Q-net (tanh hidden layers, identity head: q->out_act must be 0;
+ * A = q->dims[q->n_layers] <= 64 actions): obs [S][n] float32 field-major (a row of the replay ring or an env's policy
+ * observation).  greedy = argmax_a Q(obs)[a] (lowest index on ties, a NaN output wins as in torch.argmax); with
+ * probability epsilon the instance takes a uniform index in [0, A) instead, drawn from ONE Philox4x32-10 block keyed by
+ * (seed, offset + i, step) in the key domain 0x44514E41 (csrc/learn.cu states the counter layout and the mapping bit for
+ * bit).  Writes action_index [n] int32, action_value [n] = table[action_index] (table: device float32 [A], the float32
+ * image of the env's action_space, so that action_value is the env's action buffer [1][n]) and, if q_out is given,
+ * q_out [A][n].  Errors, all returned before any CUDA call: B200ENV_ENULL (q, obs, table, action_index, action_value or a
+ * weight / bias pointer NULL), B200ENV_ESIZE (n <= 0 or >= 2^31; > 4 layers, a layer or state_dim > 64, > 64 actions),
+ * B200ENV_EPARAMS (epsilon outside [0, 1] or NaN, q->out_act != 0, an output overlapping an input or another output). */
+B200_API int b200_dqn_act(int64_t n, const b200_mlp *q, const float *obs, const float *table, float epsilon,
+                          uint64_t seed, uint64_t step, int64_t offset, int32_t *action_index, float *action_value,
+                          float *q_out, void *cuda_stream);
+
+/* The replay ring: R rows of s [R][S][N], r [R][N], s_ [R][S][N] float32, a [R][N] int32 and done [R][N] uint8 (the
+ * rollout's is_terminal: terminal states AND time-outs end the bootstrap).  A mini-batch is `count` samples drawn
+ * uniformly WITH replacement over the valid_rows newest rows: sample b in [0, valid_rows N) is row
+ * (newest_row - b / N) mod R, instance b % N, b from a keyed 64-bit hash of (sample_key, j) and a multiply-high; `index`
+ * (device int64 [count] of ring positions row * N + i) overrides the draw.  1 <= valid_rows <= R - 1. */
+typedef struct b200_dqn_batch {
+    int64_t R, N;
+    const float *s, *r, *s_;
+    const int32_t *a;
+    const uint8_t *done;
+    int64_t newest_row, valid_rows, count;
+    const int64_t *index;
+    uint64_t sample_key;
+} b200_dqn_batch;
+
+/* Device bytes of the workspace of b200_dqn_grad for this net and mini-batch size (0 for a net it cannot hold). */
+B200_API size_t b200_dqn_workspace_bytes(const b200_mlp *q, int64_t count);
+
+/* One DQN / Double DQN gradient:  y = r + gamma (1 - done) Q_next  (done: y = r exactly), with
+ *   DQN         Q_next = max_a Q_target(s', a)
+ *   Double DQN  Q_next = Q_target(s', argmax_a Q(s', a))          (double_q != 0)
+ * loss = mean_j (Q(s_j)[a_j] - y_j)^2;  grad (device float32 [P], torch parameter order of q) = d loss / d theta;
+ * loss_out (device float32 [1]).  Three launches: target, gradient (per-block partials, no atomics), the fixed-order
+ * reduction: the bits do not depend on scheduling.  The caller then runs b200_adam_step with n_seg = 1.  q and q_target
+ * have the same shapes.  Errors, all returned before any CUDA call: B200ENV_ENULL (a pointer NULL; index may be),
+ * B200ENV_ESIZE (R < 2, N <= 0, R or N >= 2^31, count <= 0, net limits as b200_dqn_act, workspace too small),
+ * B200ENV_EPARAMS (gamma NaN, valid_rows < 1 or > R - 1, newest_row outside [0, R), shapes differ, out_act != 0, grad /
+ * loss_out / workspace overlapping an input, a weight or each other). */
+B200_API int b200_dqn_grad(const b200_dqn_batch *batch, const b200_mlp *q, const b200_mlp *q_target, float gamma,
+                           int double_q, float *grad, float *loss_out, void *workspace, size_t workspace_bytes,
+                           void *cuda_stream);
+
+/* The mini-batch sampler of b200_dqn_grad on the HOST: out_host[j] = ring position (row * N + i) of sample first + j. */
+B200_API int b200_dqn_sample_indices(uint64_t sample_key, int64_t newest_row, int64_t valid_rows, int64_t R, int64_t N,
+                                     int64_t first, int64_t count, int64_t *out_host);
+
 /* ------------------------------------------------------------- diagnostics */
 
 /* Measures the FP64 (dtype = B200ENV_F64) or FP32 vector FMA peak of the current device in TFLOP/s (2 flops per

@@ -8,6 +8,8 @@ from . import ppo2  # noqa: F401
 from .ppo2 import VecPPO2  # noqa: F401
 from . import ppo  # noqa: F401
 from .ppo import VecPPO  # noqa: F401
+from . import dqn  # noqa: F401
+from .dqn import VecDQN  # noqa: F401
 from .compat import SingleEnv, single  # noqa: F401
 from .normalization import Normalization  # noqa: F401
 from .rollout import RolloutBuffer  # noqa: F401
@@ -18,7 +20,7 @@ from .envs.simple import (BallBalancer1D, Flight_Attitude_Simulator, FlightAttit
 from .envs.uavrobust import uav_hover, uav_hover_outer_loop, uav_inner_loop, uav_tracking_outer_loop  # noqa: F401
 from .envs.uav import UavAttCtrlRL, UavPosCtrlRL, uav_param, fntsmc_param  # noqa: F401
 
-__all__ = ["VecEnvBase", "RolloutBuffer", "EpisodeTracker", "Normalization", "GaussianPolicy", "VecPPO2", "VecPPO", "SingleEnv", "single", "CartPole", "CartPoleAngleOnly", "UavAttCtrlRL", "UavPosCtrlRL", "uav_param", "fntsmc_param",
+__all__ = ["VecEnvBase", "RolloutBuffer", "EpisodeTracker", "Normalization", "GaussianPolicy", "VecPPO2", "VecPPO", "VecDQN", "SingleEnv", "single", "CartPole", "CartPoleAngleOnly", "UavAttCtrlRL", "UavPosCtrlRL", "uav_param", "fntsmc_param",
            "Flight_Attitude_Simulator", "FlightAttitudeSimulatorDiscrete", "SecondOrderIntegration", "BallBalancer1D", "TwoLinkManipulator", "UGVForward",
            "UGVBidirectional", "UGVForwardObstacleAvoidance", "uav_hover", "uav_hover_outer_loop",
            "uav_inner_loop", "uav_tracking_outer_loop"]

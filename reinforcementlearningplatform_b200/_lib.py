@@ -58,6 +58,13 @@ class PPO2Batch(C.Structure):
         ("first", C.c_int64), ("count", C.c_int64), ("perm_key", C.c_uint64)]
 
 
+class DQNBatch(C.Structure):
+    """struct b200_dqn_batch"""
+    _fields_ = [("R", C.c_int64), ("N", C.c_int64)] + [(k, C.c_void_p) for k in ("s", "r", "s_", "a", "done")] + [
+        ("newest_row", C.c_int64), ("valid_rows", C.c_int64), ("count", C.c_int64), ("index", C.c_void_p),
+        ("sample_key", C.c_uint64)]
+
+
 class CartPoleParams(C.Structure):
     """struct b200_cartpole_params"""
     _fields_ = [(k, C.c_double) for k in (
@@ -217,6 +224,14 @@ def load() -> C.CDLL:
     lib.b200_ppo2_learn.restype = i32
     lib.b200_ppo2_learn.argtypes = [vp, vp, vp, f32, vp, vp, vp, f32, f32, i32, i64, f32, f32, f32, f32, f32, f32, i64, vp,
                                     vp, vp, vp, vp, vp, sz, vp]
+    lib.b200_dqn_act.restype = i32
+    lib.b200_dqn_act.argtypes = [i64, vp, vp, vp, f32, u64, u64, i64, vp, vp, vp, vp]
+    lib.b200_dqn_workspace_bytes.restype = sz
+    lib.b200_dqn_workspace_bytes.argtypes = [vp, i64]
+    lib.b200_dqn_grad.restype = i32
+    lib.b200_dqn_grad.argtypes = [vp, vp, vp, f32, i32, vp, vp, vp, sz, vp]
+    lib.b200_dqn_sample_indices.restype = i32
+    lib.b200_dqn_sample_indices.argtypes = [u64, i64, i64, i64, i64, i64, i64, C.POINTER(i64)]
     lib.b200_umma_probe.restype = i32
     lib.b200_umma_probe.argtypes = [vp, vp, vp, i32, i32, i32, vp]
     lib.b200_fastmath_eval.restype = i32

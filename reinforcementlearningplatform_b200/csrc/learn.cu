@@ -659,6 +659,357 @@ __global__ void __launch_bounds__(LT, BLOCKS_PER_SM) ppo1_advantage_kernel(const
     }
 }
 
+// ------------------------------------------------------------------------------------------------ DQN / Double DQN
+// Three kernels on the same tiles and GEMM helpers as the PPO update (64-sample tiles, 256 threads, weights resident in
+// shared memory, fp32 FMA pipe, accurate tanhf; Q-net = tanh hidden layers and an identity head of A <= 64 outputs):
+//   dqn_act_kernel     epsilon-greedy action of n instances from field-major observations [S][n]
+//   dqn_target_kernel  y = r + gamma (1 - done) Q_next for one mini-batch drawn from the replay ring
+//   dqn_grad_kernel    gradient of mse(Q(s)[a], y) into per-block partials, summed by ppo2_reduce_kernel
+//
+// Greedy index: the first maximum over the A outputs (lowest index on ties); a NaN output counts as larger than every
+// number and the first NaN wins, as torch.argmax.
+//
+// Exploration draw of instance i (global index g = offset + i) at step k: ONE Philox4x32-10 block with
+//     key     = (seed lo, seed hi ^ 0x44514E41 "DQNA"),
+//     counter = (g lo, g hi, k lo, (k hi) << 8)
+// (the counter layout of K-POLICY's noise, in a key domain of its own).  Words r0, r1 of the block:
+//     explore  <=>  (r0 >> 8) * 2^-24 < epsilon        (24-bit uniform in [0, 1): epsilon 0 never, 1 always explores)
+//     index     =  (r1 * A) >> 32                      (multiply-high: uniform over [0, A) up to 2^-32 / A)
+// The draw does not depend on n, on the launch geometry or on the instance's position in the batch.
+//
+// Replay sampling: sample j of a mini-batch is ring position p = row * N + i with
+//     h = splitmix64(sample_key + (j + 1) * 0x9E3779B97F4A7C15),  b = (h * V N) >> 64  (a 64-bit multiply-high),
+//     row = (newest_row - b / N) mod R,  i = b mod N
+// i.e. uniform WITH replacement over the V = valid_rows newest rows; a caller-given index[j] (ring positions) overrides
+// it.  The same function runs on the host (b200_dqn_sample_indices).
+#define B200_DQN_KEY_DOMAIN 0x44514E41u
+
+__host__ __device__ __forceinline__ uint64_t dqn_mix(uint64_t key, uint64_t j) {
+    uint64_t z = key + (j + 1) * 0x9E3779B97F4A7C15ull;
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+    return z ^ (z >> 31);
+}
+struct DqnSampler {
+    int64_t R, N, newest, V;
+    const int64_t *index;
+    uint64_t key;
+};
+__host__ __device__ __forceinline__ int64_t dqn_sample_pos(const DqnSampler &p, int64_t j) {
+    if (p.index) return p.index[j];
+    const uint64_t h = dqn_mix(p.key, (uint64_t)j), vn = (uint64_t)(p.V * p.N);
+#ifdef __CUDA_ARCH__
+    const uint64_t b = __umul64hi(h, vn);
+#else
+    const uint64_t b = (uint64_t)(((unsigned __int128)h * vn) >> 64);
+#endif
+    const int64_t back = (int64_t)(b / (uint64_t)p.N), i = (int64_t)b - back * p.N;
+    int64_t row = p.newest - back;
+    if (row < 0) row += p.R;
+    return row * p.N + i;
+}
+
+// weights and biases of `net` -> w (shared memory, the offsets of fill_net), zero-padded
+__device__ __forceinline__ void dqn_load_weights(const LNet &net, float *w, int tid) {
+    for (int l = 0; l < net.n_layers; ++l) {
+        const LLayer &Ly = net.L[l];
+        const int pw = Ly.K + 4;
+        for (int e = tid; e < Ly.N * pw; e += LT) {
+            const int n = e / pw, k = e - n * pw;
+            w[Ly.w_off + e] = (n < Ly.n_real && k < Ly.k_real) ? __ldg(Ly.w + n * Ly.k_real + k) : 0.0f;
+        }
+        for (int n = tid; n < Ly.N; n += LT) w[Ly.b_off + n] = n < Ly.n_real ? __ldg(Ly.b + n) : 0.0f;
+    }
+}
+
+// Forward-only pass of the tile in X: the layers alternate between P and Q (all three [TM][pw]); returns the buffer that
+// holds the output [TM][A].  Ends with a barrier.  X is not written, so a second net can run on the same input.
+__device__ __forceinline__ const float *dqn_forward(const LNet &net, const float *w, const float *X, float *P, float *Q,
+                                                    int pw, int sg, int ng) {
+    const float *in = X;
+    float *out = P;
+#pragma unroll
+    for (int l = 0; l < LMAX; ++l) {
+        if (l < net.n_layers) {
+            const LLayer &Ly = net.L[l];
+            const bool hidden = l + 1 < net.n_layers;
+            const float *W = w + Ly.w_off, *bs = w + Ly.b_off;
+            const int pk = Ly.K + 4;
+            switch (Ly.N >> 3) {
+            case 1: fwd_layer<1>(in, pw, W, pk, bs, Ly.K, out, pw, hidden, sg, ng); break;
+            case 2: fwd_layer<2>(in, pw, W, pk, bs, Ly.K, out, pw, hidden, sg, ng); break;
+            case 4: fwd_layer<4>(in, pw, W, pk, bs, Ly.K, out, pw, hidden, sg, ng); break;
+            default: fwd_layer<8>(in, pw, W, pk, bs, Ly.K, out, pw, hidden, sg, ng); break;
+            }
+            __syncthreads();
+            in = out;
+            out = out == P ? Q : P;
+        }
+    }
+    return in;
+}
+
+// first maximum of z[0 .. A - 1], NaN above every number (torch.argmax)
+__device__ __forceinline__ int dqn_argmax(const float *z, int A) {
+    int best = 0;
+    float bv = z[0];
+    for (int a = 1; a < A; ++a) {
+        const float v = z[a];
+        if (bv == bv && (v > bv || v != v)) { bv = v; best = a; }
+    }
+    return best;
+}
+
+struct DqnActArgs {
+    LNet net;
+    int S, A, pw, wfl;           // wfl: floats of the weights in shared memory; pw: row pitch of X / P / Q
+    int64_t n, off;
+    const float *obs, *table;
+    float epsilon;
+    uint64_t seed, step;
+    int32_t *index;
+    float *value, *q;            // q may be NULL
+};
+__global__ void __launch_bounds__(LT, BLOCKS_PER_SM) dqn_act_kernel(const __grid_constant__ DqnActArgs A) {
+    extern __shared__ __align__(16) float sm[];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int sg = (lane & 3) + 4 * warp, ng = lane >> 2;
+    float *X = sm + A.wfl, *P = X + TM * A.pw, *Q = P + TM * A.pw;
+    dqn_load_weights(A.net, sm, tid);
+    const int64_t tiles = (A.n + TM - 1) / TM;
+    const int K0 = A.net.L[0].K;
+    for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
+        __syncthreads();   // the previous tile's outputs have been read
+        {
+            const int s = tid & (TM - 1), q = tid >> TM_LOG2;
+            const int64_t i = tile * TM + s;
+            for (int k = q; k < K0; k += LT / TM)
+                X[s * A.pw + k] = (i < A.n && k < A.S) ? __ldg(A.obs + (int64_t)k * A.n + i) : 0.0f;
+        }
+        __syncthreads();
+        const float *Z = dqn_forward(A.net, sm, X, P, Q, A.pw, sg, ng);
+        if (tid < TM) {
+            const int64_t i = tile * TM + tid;
+            if (i < A.n) {
+                int idx = dqn_argmax(Z + tid * A.pw, A.A);
+                Philox rng(A.seed, (uint64_t)(A.off + i), (uint32_t)A.step);
+                rng.k1 ^= B200_DQN_KEY_DOMAIN;
+                rng.c3 = (uint32_t)(A.step >> 32) << 8;
+                rng.block();
+                if ((float)(rng.r[0] >> 8) * (1.0f / 16777216.0f) < A.epsilon)
+                    idx = (int)(((uint64_t)rng.r[1] * (uint32_t)A.A) >> 32);
+                A.index[i] = idx;
+                A.value[i] = __ldg(A.table + idx);
+            }
+        }
+        if (A.q) {
+            for (int e = tid; e < A.A * TM; e += LT) {
+                const int a = e >> TM_LOG2, s = e & (TM - 1);
+                const int64_t i = tile * TM + s;
+                if (i < A.n) A.q[(int64_t)a * A.n + i] = Z[s * A.pw + a];
+            }
+        }
+    }
+}
+
+// Target of one mini-batch.  Shared memory: the target net's weights, with double_q the online net's after them, then X /
+// P / Q [64][W + 4] (W = the widest layer or input).  At the largest nets (64 inputs, four 64-wide layers, 64 actions)
+// that is 2 x 70.6 KB + 3 x 17.4 KB = 193.4 KB, under the 227 KB of a block; the demo's 2-64-64-47 nets take 2 x 38.7 KB
+// + 3 x 17.4 KB = 129.6 KB (one block per SM).
+struct DqnTargetArgs {
+    LNet tnet, onet;             // same shapes, hence the same offsets
+    int S, A, pw, wfl, double_q;
+    DqnSampler sp;
+    int64_t count;
+    const float *s_, *r;
+    const uint8_t *done;
+    float gamma;
+    float *y;
+};
+__global__ void __launch_bounds__(LT, BLOCKS_PER_SM) dqn_target_kernel(const __grid_constant__ DqnTargetArgs A) {
+    extern __shared__ __align__(16) float sm[];
+    __shared__ int s_t[TM], s_i[TM], s_arg[TM];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int sg = (lane & 3) + 4 * warp, ng = lane >> 2;
+    float *wo = sm + A.wfl;
+    float *X = sm + (A.double_q ? 2 : 1) * A.wfl, *P = X + TM * A.pw, *Q = P + TM * A.pw;
+    dqn_load_weights(A.tnet, sm, tid);
+    if (A.double_q) dqn_load_weights(A.onet, wo, tid);
+    const int64_t tiles = (A.count + TM - 1) / TM, N = A.sp.N;
+    const int K0 = A.tnet.L[0].K;
+    for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
+        __syncthreads();
+        if (tid < TM) {
+            const int64_t j = tile * TM + tid;
+            int t = -1, i = 0;
+            if (j < A.count) {
+                const int64_t p = dqn_sample_pos(A.sp, j);
+                t = (int)(p / N);
+                i = (int)(p - (int64_t)t * N);
+            }
+            s_t[tid] = t;
+            s_i[tid] = i;
+        }
+        __syncthreads();
+        {
+            const int s = tid & (TM - 1), q = tid >> TM_LOG2;
+            const int t = s_t[s];
+            const int64_t i = s_i[s], tt = t < 0 ? 0 : t;
+            for (int k = q; k < K0; k += LT / TM)
+                X[s * A.pw + k] = (t >= 0 && k < A.S) ? __ldg(A.s_ + (tt * A.S + k) * N + i) : 0.0f;
+        }
+        __syncthreads();
+        if (A.double_q) {
+            const float *Z = dqn_forward(A.onet, wo, X, P, Q, A.pw, sg, ng);
+            if (tid < TM) s_arg[tid] = dqn_argmax(Z + tid * A.pw, A.A);
+            __syncthreads();
+        }
+        const float *Z = dqn_forward(A.tnet, sm, X, P, Q, A.pw, sg, ng);
+        if (tid < TM && s_t[tid] >= 0) {
+            const float *z = Z + tid * A.pw;
+            const float qn = z[A.double_q ? s_arg[tid] : dqn_argmax(z, A.A)];
+            const int64_t p = (int64_t)s_t[tid] * N + s_i[tid];
+            const float r = __ldg(A.r + p);
+            // a done transition (terminal OR time-out) takes y = r: nothing of Q_next, not even a non-finite value
+            A.y[tile * TM + tid] = __ldg(A.done + p) ? r : __fadd_rn(r, __fmul_rn(A.gamma, qn));
+        }
+    }
+}
+
+// Gradient of mean_j (Q(s_j)[a_j] - y_j)^2: ppo2_grad_kernel's tile loop for one net with the squared error at the
+// selected output as the loss (dZ_out[s][n] = n == a_s ? 2 (Q - y) / M : 0).  An action outside [0, A) reads Q = NaN,
+// so the loss shows it.
+struct DqnGradArgs {
+    LNet net;
+    int S, A;
+    DqnSampler sp;
+    int64_t count;
+    const float *s, *y;
+    const int32_t *a;
+    float inv_count;
+    float *partial;              // [gridDim.x][P + 4]
+};
+__global__ void __launch_bounds__(LT, BLOCKS_PER_SM) dqn_grad_kernel(const __grid_constant__ DqnGradArgs A) {
+    extern __shared__ __align__(16) float sm[];
+    __shared__ int s_t[TM], s_i[TM], s_a[TM];
+    __shared__ float s_y[TM];
+    __shared__ float s_red[LT / 32];
+    const LNet &net = A.net;
+    const int L = net.n_layers;
+    const int bx = blockIdx.x, nbx = gridDim.x;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int sg = (lane & 3) + 4 * warp, ng = lane >> 2;
+    dqn_load_weights(net, sm, tid);
+    float loss_acc = 0.0f;
+    float *part = A.partial + (size_t)bx * (size_t)(net.P + 4);
+    const int64_t tiles = (A.count + TM - 1) / TM, N = A.sp.N;
+    const LLayer &L0 = net.L[0];
+    const LLayer &LO = net.L[L - 1];
+    float *gout = sm + net.gout_off;
+    const int pgo = LO.N + 4;
+    for (int64_t tile = bx; tile < tiles; tile += nbx) {
+        __syncthreads();
+        if (tid < TM) {
+            const int64_t j = tile * TM + tid;
+            int t = -1, i = 0, act = 0;
+            float y = 0.0f;
+            if (j < A.count) {
+                const int64_t p = dqn_sample_pos(A.sp, j);
+                t = (int)(p / N);
+                i = (int)(p - (int64_t)t * N);
+                act = __ldg(A.a + p);
+                y = __ldg(A.y + j);
+            }
+            s_t[tid] = t; s_i[tid] = i; s_a[tid] = act; s_y[tid] = y;
+        }
+        __syncthreads();
+        {
+            float *H0 = sm + L0.h_off;
+            const int p0 = L0.K + 4;
+            const int s = tid & (TM - 1), q = tid >> TM_LOG2;
+            const int t = s_t[s];
+            const int64_t i = s_i[s], tt = t < 0 ? 0 : t;
+            for (int k = q; k < L0.K; k += LT / TM)
+                H0[s * p0 + k] = (t >= 0 && k < A.S) ? __ldg(A.s + (tt * A.S + k) * N + i) : 0.0f;
+        }
+        __syncthreads();
+#pragma unroll
+        for (int l = 0; l < LMAX; ++l) {
+            if (l < L) {
+                const LLayer &Ly = net.L[l];
+                const bool last = l == L - 1;
+                float *out = last ? gout : sm + net.L[l + 1 < LMAX ? l + 1 : l].h_off;
+                const float *H = sm + Ly.h_off, *W = sm + Ly.w_off, *bs = sm + Ly.b_off;
+                const int ph = Ly.K + 4, po = Ly.N + 4;
+                switch (Ly.N >> 3) {
+                case 1: fwd_layer<1>(H, ph, W, ph, bs, Ly.K, out, po, !last, sg, ng); break;
+                case 2: fwd_layer<2>(H, ph, W, ph, bs, Ly.K, out, po, !last, sg, ng); break;
+                case 4: fwd_layer<4>(H, ph, W, ph, bs, Ly.K, out, po, !last, sg, ng); break;
+                default: fwd_layer<8>(H, ph, W, ph, bs, Ly.K, out, po, !last, sg, ng); break;
+                }
+                __syncthreads();
+            }
+        }
+        {   // four lanes per sample, in one warp: all read Q[a] before any of them writes dZ over the row
+            const int sx = tid >> 2, q = tid & 3;
+            float *z = gout + sx * pgo;
+            const bool live = s_t[sx] >= 0;
+            const int act = s_a[sx];
+            const float qa = (unsigned)act < (unsigned)A.A ? z[act] : __int_as_float(0x7fc00000);
+            const float e = qa - s_y[sx];
+            __syncwarp();
+            if (live && q == 0) loss_acc += e * e;
+            const float c = live ? 2.0f * e * A.inv_count : 0.0f;
+            for (int d = q; d < LO.N; d += 4) z[d] = d == act ? c : 0.0f;
+        }
+        __syncthreads();
+#pragma unroll
+        for (int l = LMAX - 1; l >= 0; --l) {
+            if (l < L) {
+                const LLayer &Ly = net.L[l];
+                const float *G = (l == L - 1) ? gout : sm + net.L[l + 1 < LMAX ? l + 1 : l].h_off;
+                float *H = sm + Ly.h_off;
+                const int pg = Ly.N + 4, ph = Ly.K + 4;
+                const int kgs = Ly.K >> 2;
+                {
+                    const int kt = Ly.K / Ly.rk, nt = Ly.N / Ly.rn;
+                    if (tid < nt * kt) {
+                        const int tk = tid / nt, tn = tid - tk * nt;
+                        float dw[16], db[4];
+#pragma unroll
+                        for (int e = 0; e < 16; ++e) dw[e] = 0.0f;
+#pragma unroll
+                        for (int e = 0; e < 4; ++e) db[e] = 0.0f;
+                        const bool first = tile == bx;
+                        switch (Ly.rn * 8 + Ly.rk) {
+                        case 4 * 8 + 4: dw_layer<4, 4>(G, pg, H, ph, tn, tk, dw, db); dw_store<4, 4>(Ly, part, tn, tk, dw, db, first); break;
+                        case 2 * 8 + 4: dw_layer<2, 4>(G, pg, H, ph, tn, tk, dw, db); dw_store<2, 4>(Ly, part, tn, tk, dw, db, first); break;
+                        case 1 * 8 + 4: dw_layer<1, 4>(G, pg, H, ph, tn, tk, dw, db); dw_store<1, 4>(Ly, part, tn, tk, dw, db, first); break;
+                        case 1 * 8 + 2: dw_layer<1, 2>(G, pg, H, ph, tn, tk, dw, db); dw_store<1, 2>(Ly, part, tn, tk, dw, db, first); break;
+                        default: dw_layer<1, 1>(G, pg, H, ph, tn, tk, dw, db); dw_store<1, 1>(Ly, part, tn, tk, dw, db, first); break;
+                        }
+                    }
+                }
+                if (l > 0) {
+                    __syncthreads();
+                    if (kgs == 16) bwd_layer<2>(G, pg, sm + Ly.w_off, ph, Ly.N, H, ph, kgs, sg, ng);
+                    else bwd_layer<1>(G, pg, sm + Ly.w_off, ph, Ly.N, H, ph, kgs, sg, ng);
+                    __syncthreads();
+                }
+            }
+        }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) loss_acc += __shfl_xor_sync(0xffffffffu, loss_acc, o);
+    if (lane == 0) s_red[warp] = loss_acc;
+    __syncthreads();
+    if (tid == 0) {
+        float t = 0.0f;
+        for (int w = 0; w < LT / 32; ++w) t += s_red[w];
+        part[net.P] = t;
+    }
+}
+
 // ------------------------------------------------------------------------------------------------ clip + Adam
 struct AdamArgs {
     int64_t off[2], len[2];
@@ -713,7 +1064,8 @@ __global__ void __launch_bounds__(AT) adam_kernel(const __grid_constant__ AdamAr
 // ------------------------------------------------------------------------------------------------ host side
 int pad_n(int n) { return n <= 8 ? 8 : n <= 16 ? 16 : n <= 32 ? 32 : 64; }
 
-int fill_net(const b200_mlp *m, bool is_actor, LNet *net) {
+// max_out: the widest output layer the caller's loss handles (16 for the PPO heads, 64 for a Q-net)
+int fill_net(const b200_mlp *m, int max_out, LNet *net) {
     *net = LNet{};
     if (m->n_layers < 1 || m->n_layers > LMAX) return B200ENV_ESIZE;
     net->n_layers = m->n_layers;
@@ -725,7 +1077,7 @@ int fill_net(const b200_mlp *m, bool is_actor, LNet *net) {
         if (!m->w[l] || !m->b[l]) return B200ENV_ENULL;
         LLayer &Ly = net->L[l];
         const bool last = l + 1 == m->n_layers;
-        if (last && out > 16) return B200ENV_ESIZE;
+        if (last && out > max_out) return B200ENV_ESIZE;
         Ly.k_real = in;
         Ly.n_real = out;
         Ly.K = l == 0 ? (in + 7) / 8 * 8 : net->L[l - 1].N;
@@ -752,7 +1104,6 @@ int fill_net(const b200_mlp *m, bool is_actor, LNet *net) {
     off += TM * (net->L[m->n_layers - 1].N + 4);
     net->P = P;
     net->smem_floats = off;
-    (void)is_actor;
     return B200ENV_OK;
 }
 
@@ -796,7 +1147,7 @@ int make_plan(const b200_ppo2_batch *bt, const b200_mlp *actor, const b200_mlp *
         if (!std_vec && !(std_ > 0.0f)) return B200ENV_EPARAMS;
         if (actor->out_act < 0 || actor->out_act > 2) return B200ENV_EPARAMS;
         if (actor->out_act == 2 && (!a_min || !a_max)) return B200ENV_ENULL;
-        if ((rc = fill_net(actor, true, &a.net[0]))) return rc;
+        if ((rc = fill_net(actor, 16, &a.net[0]))) return rc;
         a.net_of_y[pl->nets++] = 0;
         smem_f = a.net[0].smem_floats;
         a.partial[0] = reinterpret_cast<float *>(static_cast<char *>(workspace) + ws);
@@ -808,7 +1159,7 @@ int make_plan(const b200_ppo2_batch *bt, const b200_mlp *actor, const b200_mlp *
         if (!grad_critic) return B200ENV_ENULL;
         if (critic->dims[critic->n_layers > 0 && critic->n_layers <= 4 ? critic->n_layers : 0] != 1) return B200ENV_EPARAMS;
         if (actor && actor->dims[0] != critic->dims[0]) return B200ENV_EPARAMS;
-        if ((rc = fill_net(critic, false, &a.net[1]))) return rc;
+        if ((rc = fill_net(critic, 16, &a.net[1]))) return rc;
         a.net[1].out_act = 0;
         a.net_of_y[pl->nets++] = 1;
         if ((size_t)a.net[1].smem_floats > smem_f) smem_f = a.net[1].smem_floats;
@@ -923,11 +1274,11 @@ extern "C" B200_API size_t b200_ppo2_workspace_bytes(const b200_mlp *actor, cons
     size_t ws = 64;
     LNet n;
     if (actor) {
-        if (fill_net(actor, true, &n)) return 0;
+        if (fill_net(actor, 16, &n)) return 0;
         ws += partial_floats(n) * 4;
     }
     if (critic) {
-        if (fill_net(critic, false, &n)) return 0;
+        if (fill_net(critic, 16, &n)) return 0;
         ws += partial_floats(n) * 4;
     }
     return (actor || critic) ? ws : 0;
@@ -1025,7 +1376,7 @@ extern "C" B200_API int b200_ppo2_learn(const b200_ppo2_batch *batch, const b200
     const int64_t B = batch->T * batch->N;
     LNet na, nc;
     int rc;
-    if ((rc = fill_net(actor, true, &na)) || (rc = fill_net(critic, false, &nc))) return rc;
+    if ((rc = fill_net(actor, 16, &na)) || (rc = fill_net(critic, 16, &nc))) return rc;
     const int64_t seg_off[2] = {0, na.P}, seg_len[2] = {na.P, nc.P};
     const float lr[2] = {lr_actor, lr_critic};
     cudaStream_t stream = (cudaStream_t)cuda_stream;
@@ -1052,6 +1403,180 @@ extern "C" B200_API int b200_ppo2_permutation(uint64_t perm_key, int64_t B, int6
     if (!out_host && count) return B200ENV_ENULL;
     const int hb = half_bits_for(B);
     for (int64_t j = 0; j < count; ++j) out_host[j] = perm_index(perm_key, first + j, B, hb);
+    return B200ENV_OK;
+}
+
+// ------------------------------------------------------------------------------------------------ DQN host side
+namespace {
+constexpr size_t SMEM_MAX = 227 * 1024 - 12 * 1024;   // as make_plan: room for the kernels' static shared memory
+
+// a Q-net: fill_net with heads up to 64 wide, identity head
+int dqn_fill(const b200_mlp *m, LNet *n) {
+    int rc = fill_net(m, WMAX, n);
+    if (rc) return rc;
+    return m->out_act == 0 ? B200ENV_OK : B200ENV_EPARAMS;
+}
+int dqn_weight_floats(const LNet &n) { return n.L[0].h_off; }
+// row pitch of the forward-only kernels' X / P / Q buffers: the widest input or output + 4
+int dqn_pitch(const LNet &n) {
+    int w = n.L[0].K;
+    for (int l = 0; l < n.n_layers; ++l) w = n.L[l].N > w ? n.L[l].N : w;
+    return w + 4;
+}
+size_t dqn_y_bytes(int64_t count) { return ((size_t)count * 4 + 63) / 64 * 64; }
+
+bool overlaps_net(const void *x, size_t bytes, const b200_mlp *m) {
+    for (int l = 0; l < m->n_layers; ++l)
+        if (overlaps(x, bytes, m->w[l], (size_t)m->dims[l] * m->dims[l + 1] * 4) ||
+            overlaps(x, bytes, m->b[l], (size_t)m->dims[l + 1] * 4)) return true;
+    return false;
+}
+
+template <typename Kernel>
+int set_smem(Kernel k, size_t smem, size_t (&configured)[64]) {
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (dev < 0 || dev >= 64) dev = 0;
+    if (smem > 48 * 1024 && smem > configured[dev]) {
+        if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+            return b200_check_launch();
+        configured[dev] = smem;
+    }
+    return B200ENV_OK;
+}
+} // namespace
+
+extern "C" B200_API int b200_dqn_act(int64_t n, const b200_mlp *q, const float *obs, const float *table, float epsilon,
+                                     uint64_t seed, uint64_t step, int64_t offset, int32_t *action_index,
+                                     float *action_value, float *q_out, void *cuda_stream) {
+    if (!q || !obs || !table || !action_index || !action_value) return B200ENV_ENULL;
+    if (n <= 0 || n >= ((int64_t)1 << 31)) return B200ENV_ESIZE;
+    DqnActArgs a = {};
+    int rc = dqn_fill(q, &a.net);
+    if (rc) return rc;
+    if (!(epsilon >= 0.0f && epsilon <= 1.0f)) return B200ENV_EPARAMS;
+    a.S = q->dims[0];
+    a.A = q->dims[q->n_layers];
+    {   // outputs against inputs and against each other
+        const size_t nb = (size_t)n * 4;
+        const void *out[3] = {action_index, action_value, q_out};
+        const size_t out_b[3] = {nb, nb, nb * (size_t)a.A};
+        for (int o = 0; o < 3; ++o) {
+            if (!out[o]) continue;
+            if (overlaps(out[o], out_b[o], obs, nb * (size_t)a.S) || overlaps(out[o], out_b[o], table, (size_t)a.A * 4) ||
+                overlaps_net(out[o], out_b[o], q)) return B200ENV_EPARAMS;
+            for (int p = o + 1; p < 3; ++p)
+                if (out[p] && overlaps(out[o], out_b[o], out[p], out_b[p])) return B200ENV_EPARAMS;
+        }
+    }
+    a.wfl = dqn_weight_floats(a.net);
+    a.pw = dqn_pitch(a.net);
+    const size_t smem = ((size_t)a.wfl + 3 * (size_t)TM * a.pw) * sizeof(float);
+    if (smem > SMEM_MAX) return B200ENV_ESIZE;
+    a.n = n; a.off = offset;
+    a.obs = obs; a.table = table;
+    a.epsilon = epsilon;
+    a.seed = seed; a.step = step;
+    a.index = action_index; a.value = action_value; a.q = q_out;
+    static size_t configured[64] = {0};
+    if ((rc = set_smem(dqn_act_kernel, smem, configured))) return rc;
+    const int64_t tiles = (n + TM - 1) / TM;
+    const int cap = grid_cap();
+    dqn_act_kernel<<<(unsigned)(tiles < cap ? tiles : cap), LT, smem, (cudaStream_t)cuda_stream>>>(a);
+    return b200_check_launch();
+}
+
+extern "C" B200_API size_t b200_dqn_workspace_bytes(const b200_mlp *q, int64_t count) {
+    LNet n;
+    if (!q || count <= 0 || dqn_fill(q, &n)) return 0;
+    return dqn_y_bytes(count) + partial_floats(n) * 4;
+}
+
+extern "C" B200_API int b200_dqn_grad(const b200_dqn_batch *bt, const b200_mlp *q, const b200_mlp *q_target, float gamma,
+                                      int double_q, float *grad, float *loss_out, void *workspace,
+                                      size_t workspace_bytes, void *cuda_stream) {
+    if (!bt || !q || !q_target || !grad || !loss_out || !workspace) return B200ENV_ENULL;
+    if (!bt->s || !bt->r || !bt->s_ || !bt->a || !bt->done) return B200ENV_ENULL;
+    if (bt->R < 2 || bt->N <= 0 || bt->R >= ((int64_t)1 << 31) || bt->N >= ((int64_t)1 << 31) || bt->count <= 0)
+        return B200ENV_ESIZE;
+    DqnTargetArgs t = {};
+    int rc;
+    if ((rc = dqn_fill(q, &t.onet)) || (rc = dqn_fill(q_target, &t.tnet))) return rc;
+    if (q->n_layers != q_target->n_layers) return B200ENV_EPARAMS;
+    for (int l = 0; l <= q->n_layers; ++l)
+        if (q->dims[l] != q_target->dims[l]) return B200ENV_EPARAMS;
+    if (gamma != gamma) return B200ENV_EPARAMS;
+    if (bt->valid_rows < 1 || bt->valid_rows > bt->R - 1 || bt->newest_row < 0 || bt->newest_row >= bt->R)
+        return B200ENV_EPARAMS;
+    const int S = q->dims[0], A = q->dims[q->n_layers];
+    const int64_t count = bt->count;
+    if (workspace_bytes < b200_dqn_workspace_bytes(q, count)) return B200ENV_ESIZE;
+    {   // grad, loss_out and the workspace are written; the ring, the index and both nets are read
+        const size_t rn = (size_t)bt->R * (size_t)bt->N, P = (size_t)t.onet.P;
+        const void *in[6] = {bt->s, bt->s_, bt->r, bt->a, bt->done, bt->index};
+        const size_t in_b[6] = {rn * S * 4, rn * S * 4, rn * 4, rn * 4, rn, (size_t)count * 8};
+        const void *out[3] = {grad, loss_out, workspace};
+        const size_t out_b[3] = {P * 4, 4, workspace_bytes};
+        for (int o = 0; o < 3; ++o) {
+            for (int k = 0; k < 6; ++k)
+                if (in[k] && overlaps(out[o], out_b[o], in[k], in_b[k])) return B200ENV_EPARAMS;
+            if (overlaps_net(out[o], out_b[o], q) || overlaps_net(out[o], out_b[o], q_target)) return B200ENV_EPARAMS;
+            for (int p = o + 1; p < 3; ++p)
+                if (overlaps(out[o], out_b[o], out[p], out_b[p])) return B200ENV_EPARAMS;
+        }
+    }
+    DqnSampler sp = {bt->R, bt->N, bt->newest_row, bt->valid_rows, bt->index, bt->sample_key};
+    float *y = static_cast<float *>(workspace);
+    t.S = S; t.A = A;
+    t.wfl = dqn_weight_floats(t.tnet);
+    t.pw = dqn_pitch(t.tnet);
+    t.double_q = double_q ? 1 : 0;
+    t.sp = sp; t.count = count;
+    t.s_ = bt->s_; t.r = bt->r; t.done = bt->done;
+    t.gamma = gamma;
+    t.y = y;
+    const size_t smem_t = ((size_t)(1 + t.double_q) * t.wfl + 3 * (size_t)TM * t.pw) * sizeof(float);
+    DqnGradArgs g = {};
+    g.net = t.onet;
+    g.S = S; g.A = A;
+    g.sp = sp; g.count = count;
+    g.s = bt->s; g.a = bt->a; g.y = y;
+    g.inv_count = 1.0f / (float)count;
+    g.partial = reinterpret_cast<float *>(static_cast<char *>(workspace) + dqn_y_bytes(count));
+    const size_t smem_g = (size_t)g.net.smem_floats * sizeof(float);
+    if (smem_t > SMEM_MAX || smem_g > SMEM_MAX) return B200ENV_ESIZE;
+    cudaStream_t stream = (cudaStream_t)cuda_stream;
+    static size_t conf_t[64] = {0}, conf_g[64] = {0};
+    if ((rc = set_smem(dqn_target_kernel, smem_t, conf_t)) || (rc = set_smem(dqn_grad_kernel, smem_g, conf_g))) return rc;
+    const int64_t tiles = (count + TM - 1) / TM;
+    const int cap = grid_cap();
+    const int blocks = (int)(tiles < cap ? tiles : cap);
+    dqn_target_kernel<<<blocks, LT, smem_t, stream>>>(t);
+    if ((rc = b200_check_launch())) return rc;
+    dqn_grad_kernel<<<blocks, LT, smem_g, stream>>>(g);
+    if ((rc = b200_check_launch())) return rc;
+    ReduceArgs r = {};
+    r.partial[0] = g.partial;
+    r.grad[0] = grad;
+    r.loss_out = loss_out;
+    r.P[0] = g.net.P;
+    r.nets = 1;
+    r.nblk[0] = blocks;
+    r.inv_count = g.inv_count;
+    r.scale1 = 1.0f;
+    r.ent_slot = -1;
+    ppo2_reduce_kernel<<<(g.net.P + 1 + 255) / 256, 256, 0, stream>>>(r);
+    return b200_check_launch();
+}
+
+extern "C" B200_API int b200_dqn_sample_indices(uint64_t sample_key, int64_t newest_row, int64_t valid_rows, int64_t R,
+                                                int64_t N, int64_t first, int64_t count, int64_t *out_host) {
+    if (R < 2 || N <= 0 || R >= ((int64_t)1 << 31) || N >= ((int64_t)1 << 31) || first < 0 || count < 0)
+        return B200ENV_ESIZE;
+    if (valid_rows < 1 || valid_rows > R - 1 || newest_row < 0 || newest_row >= R) return B200ENV_EPARAMS;
+    if (!out_host && count) return B200ENV_ENULL;
+    const DqnSampler sp = {R, N, newest_row, valid_rows, nullptr, sample_key};
+    for (int64_t j = 0; j < count; ++j) out_host[j] = dqn_sample_pos(sp, first + j);
     return B200ENV_OK;
 }
 
