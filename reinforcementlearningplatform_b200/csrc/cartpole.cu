@@ -152,7 +152,7 @@ __device__ __forceinline__ void cartpole_step_body(CartPole<T> &e, const b200_ca
         if (e.x > (T)p.x_max || e.x < -(T)p.x_max) { flag = 2; done = true; }
         if (e.time > p.time_max) { flag = 3; done = true; }
         const T ex = (T)0 - e.x, eth = (T)0 - e.theta;
-        if (Mth<T>::sqrt(ex * ex + e.dx * e.dx + eth * eth + e.dtheta * e.dtheta) < (T)1e-2) { flag = 4; done = true; }
+        if (Mth<T>::sqrt(sumsq_rn(ex, e.dx, eth, e.dtheta)) < (T)1e-2) { flag = 4; done = true; } // no FMA: common.cuh
     } else if (p.variant == 1) { // CartPoleAngleOnly.py:144-166: returns at the first true test
         if (angle_out) { flag = 1; done = true; }
         else if (e.time > p.time_max) { flag = 3; done = true; }
@@ -160,7 +160,7 @@ __device__ __forceinline__ void cartpole_step_body(CartPole<T> &e, const b200_ca
         if (angle_out) { flag = 1; done = true; }
         if (e.time > p.time_max) { flag = 3; done = true; }
         const T eth = (T)0 - e.theta;
-        if (Mth<T>::sqrt(eth * eth + e.dtheta * e.dtheta) < (T)1e-2) { flag = 4; done = true; }
+        if (Mth<T>::sqrt(sumsq_rn(eth, e.dtheta)) < (T)1e-2) { flag = 4; done = true; }
     }
 
     e.observe(p, nxt);

@@ -176,6 +176,21 @@ __device__ __forceinline__ void stio_idx(void *base, I n, int field, I i, T v) {
 template <typename T>
 __device__ __forceinline__ T np_norm2(T a, T b) { return Mth<T>::sqrt(Mth<T>::fma(b, b, a * a)); }
 
+// Sum of squares a^2 + b^2 (+ c^2 + d^2), left to right with every product and sum rounded on its own, as a Python
+// expression `a * a + b * b + ...` evaluates it.  The _rn intrinsics are never contracted into FMAs, so the result does
+// not depend on -fmad: a decision such as CartPole's `sqrt(...) < 1e-2` then takes the reference's side at the threshold
+// (contracted, it flips in a few percent of the states within an ulp of it; tests/test_env_edges_gpu.py).
+__device__ __forceinline__ double mul_rn(double a, double b) { return __dmul_rn(a, b); }
+__device__ __forceinline__ float mul_rn(float a, float b) { return __fmul_rn(a, b); }
+__device__ __forceinline__ double add_rn(double a, double b) { return __dadd_rn(a, b); }
+__device__ __forceinline__ float add_rn(float a, float b) { return __fadd_rn(a, b); }
+template <typename T>
+__device__ __forceinline__ T sumsq_rn(T a, T b) { return add_rn(mul_rn(a, a), mul_rn(b, b)); }
+template <typename T>
+__device__ __forceinline__ T sumsq_rn(T a, T b, T c, T d) {
+    return add_rn(add_rn(sumsq_rn(a, b), mul_rn(c, c)), mul_rn(d, d));
+}
+
 // clamp against bounds that are never NaN: two compare-selects instead of the NaN-aware fmin / fmax pair (6 instructions
 // each in fp64).  A NaN x passes through, like np.clip.
 template <typename T>
