@@ -61,25 +61,6 @@ struct LNet {
     LLayer L[LMAX];
 };
 
-struct LearnArgs {
-    LNet net[2];                 // 0 actor, 1 critic
-    int net_of_y[2];             // slot -> net: blocks 0 .. nblk[0] - 1 work on slot 0, the next nblk[1] on slot 1
-    int nblk[2];
-    int S, A;
-    int64_t T, N, first, count;
-    const float *s, *a, *a_lp, *adv, *v_target;
-    const int64_t *index;
-    uint64_t perm_key;
-    int perm_half_bits;
-    float eps_clip, inv_count, entropy_coef;
-    float std_;
-    const float *std_vec, *a_min, *a_max;
-    float *partial[2];           // [gridDim.x][P + 4]
-    float *grad[2];
-    float *loss_out;             // [2]
-    unsigned int *counter;       // [2]
-};
-
 // ------------------------------------------------------------------------------------------------ sample permutation
 __host__ __device__ __forceinline__ uint32_t feistel_round(uint32_t r, uint32_t k) {
     uint32_t h = (r + k) * 0x9E3779B1u;
@@ -111,6 +92,34 @@ int half_bits_for(int64_t B) {
     while (((int64_t)1 << bits) < B) ++bits;
     return (bits + 1) / 2 < 1 ? 1 : (bits + 1) / 2;
 }
+
+// sample j of a PPO mini-batch: batch position index[first + j] if the caller gave an index, else the keyed permutation
+// of [0, T N) at first + j
+struct PpoSampler {
+    int64_t T, N, first;
+    const int64_t *index;
+    uint64_t perm_key;
+    int half_bits;
+    __device__ __forceinline__ int64_t pos(int64_t j) const {
+        return index ? index[first + j] : perm_index(perm_key, first + j, T * N, half_bits);
+    }
+};
+
+struct LearnArgs {
+    LNet net[2];                 // 0 actor, 1 critic
+    int net_of_y[2];             // slot -> net: blocks 0 .. nblk[0] - 1 work on slot 0, the next nblk[1] on slot 1
+    int nblk[2];
+    int S, A;
+    PpoSampler sp;
+    int64_t count;
+    const float *s, *a, *a_lp, *adv, *v_target;
+    float eps_clip, inv_count, entropy_coef;
+    float std_;
+    const float *std_vec, *a_min, *a_max;
+    float *partial[2];           // [gridDim.x][P + 4]
+    float *grad[2];
+    float *loss_out;             // [2]
+};
 
 // ------------------------------------------------------------------------------------------------ tile GEMMs
 // thread coordinates of the sample-by-feature products: sg = 0..31 -> samples sg + 32 i, ng = 0..7 -> features ng + 8 j
@@ -270,19 +279,166 @@ __device__ __forceinline__ void dw_store(const LLayer &Ly, float *part, int ng, 
 // -DLEARN_TRACE (tools/build_variant.sh): thread 0 of block 0 adds up the cycles between the phase barriers of its tiles
 // (phase ids: 0 sample indices, 1 gather, 2 + l forward layer l, 6 loss, 7 + 2 l dW_l, 8 + 2 l dH_l + dZ write) ->
 // b200_learn_trace_read.  How profiles/r2/learn.md's phase table was measured.  Compiled out of the shipped library.
+// The timestamp lives in shared memory so that the tile helpers below can mark their phases too; every kernel that
+// runs them starts it with LTRACE_START, and their block 0 adds to the same table (tools/learn_trace.py runs PPO2 alone).
 #ifdef LEARN_TRACE
 __device__ long long g_learn_trace[16];
+__shared__ long long s_lt_prev;
+#define LTRACE_START()                                                      \
+    do {                                                                    \
+        if (blockIdx.x == 0 && threadIdx.x == 0) s_lt_prev = clock64();     \
+    } while (0)
 #define LTRACE(id)                                                          \
     do {                                                                    \
-        if (blockIdx.x == 0 && tid == 0) {                                  \
+        if (blockIdx.x == 0 && threadIdx.x == 0) {                          \
             const long long now = clock64();                                \
-            g_learn_trace[id] += now - lt_prev;                             \
-            lt_prev = now;                                                  \
+            g_learn_trace[id] += now - s_lt_prev;                           \
+            s_lt_prev = now;                                                \
         }                                                                   \
     } while (0)
 #else
+#define LTRACE_START() do { } while (0)
 #define LTRACE(id) do { } while (0)
 #endif
+
+// ------------------------------------------------------------------------------------------------ tile phases
+// The phases every tile kernel shares.  One copy each: ppo1_advantage_kernel's V is bit-identical to the critic blocks'
+// of ppo2_grad_kernel, and dqn_grad_kernel's backward is ppo2_grad_kernel's, because they run the same code.
+
+// weights and biases of `net` -> w (shared memory, the offsets of fill_net), zero-padded
+__device__ __forceinline__ void load_weights(const LNet &net, float *w, int tid) {
+    for (int l = 0; l < net.n_layers; ++l) {
+        const LLayer &Ly = net.L[l];
+        const int pw = Ly.K + 4;
+        for (int e = tid; e < Ly.N * pw; e += LT) {
+            const int n = e / pw, k = e - n * pw;
+            w[Ly.w_off + e] = (n < Ly.n_real && k < Ly.k_real) ? __ldg(Ly.w + n * Ly.k_real + k) : 0.0f;
+        }
+        for (int n = tid; n < Ly.N; n += LT) w[Ly.b_off + n] = n < Ly.n_real ? __ldg(Ly.b + n) : 0.0f;
+    }
+}
+
+// layer Ly of the forward: out [TM][po] = act(H [TM][ph] W^T + b), with W and b at Ly's offsets in w
+__device__ __forceinline__ void fwd_any(const LLayer &Ly, const float *w, const float *H, int ph, float *out, int po,
+                                        bool hidden, int sg, int ng) {
+    const float *W = w + Ly.w_off, *bs = w + Ly.b_off;
+    const int pw = Ly.K + 4;
+    switch (Ly.N >> 3) {
+    case 1: fwd_layer<1>(H, ph, W, pw, bs, Ly.K, out, po, hidden, sg, ng); break;
+    case 2: fwd_layer<2>(H, ph, W, pw, bs, Ly.K, out, po, hidden, sg, ng); break;
+    case 4: fwd_layer<4>(H, ph, W, pw, bs, Ly.K, out, po, hidden, sg, ng); break;
+    default: fwd_layer<8>(H, ph, W, pw, bs, Ly.K, out, po, hidden, sg, ng); break;
+    }
+}
+
+// sample j = tile TM + tid of the mini-batch -> (t, i) in s_t / s_i (t = -1 past `count`); returns its position
+// t N + i in the batch (-1 for none)
+template <typename Sampler>
+__device__ __forceinline__ int64_t tile_samples(const Sampler &sp, int64_t tile, int64_t count, int *s_t, int *s_i,
+                                                int tid) {
+    int64_t b = -1;
+    if (tid < TM) {
+        const int64_t j = tile * TM + tid;
+        int t = -1, i = 0;
+        if (j < count) {
+            b = sp.pos(j);
+            t = (int)(b / sp.N);
+            i = (int)(b - (int64_t)t * sp.N);
+        }
+        s_t[tid] = t;
+        s_i[tid] = i;
+    }
+    return b;
+}
+
+// X [TM][px] = the tile's observations s [T][S][N], zero-padded to K0 fields and for samples t < 0
+// (thread = sample s, fields q, q + 4, ...)
+__device__ __forceinline__ void gather_obs(const float *s, int S, int64_t N, int K0, const int *s_t, const int *s_i,
+                                           float *X, int px, int tid) {
+    const int sx = tid & (TM - 1), q = tid >> TM_LOG2;
+    const int t = s_t[sx];
+    const int64_t i = s_i[sx], tt = t < 0 ? 0 : t;
+    for (int k = q; k < K0; k += LT / TM)
+        X[sx * px + k] = (t >= 0 && k < S) ? __ldg(s + (tt * S + k) * N + i) : 0.0f;
+}
+
+// tile_forward / tile_backward take L = net.n_layers and gout = sm + net.gout_off from the kernel, which reads them once
+// before its tile loop.  Read from `net` inside the helpers instead, they made ptxas rebuild the shared-memory base
+// (S2UR + ULEA) at every layer: 2.2 % more instructions in ppo1_advantage_kernel and dqn_grad_kernel.
+
+// forward of the tile in H_0 through the net's H_l buffers (fill_net's layout); the output layer's Z goes to gout.
+// Ends with a barrier.
+__device__ __forceinline__ void tile_forward(const LNet &net, int L, float *sm, float *gout, int sg, int ng) {
+#pragma unroll
+    for (int l = 0; l < LMAX; ++l) {
+        if (l < L) {
+            const LLayer &Ly = net.L[l];
+            const bool last = l == L - 1;
+            float *out = last ? gout : sm + net.L[l + 1 < LMAX ? l + 1 : l].h_off;
+            fwd_any(Ly, sm, sm + Ly.h_off, Ly.K + 4, out, Ly.N + 4, !last, sg, ng);
+            __syncthreads();
+            LTRACE(2 + l);
+        }
+    }
+}
+
+// backward of the tile from dZ of the output layer (in gout): per layer, dW / db added to the block's partial gradient
+// `part` (`first`: the block's first tile, see dw_store), then dZ_{l-1} written over H_l.  No barrier after the last dW.
+__device__ __forceinline__ void tile_backward(const LNet &net, int L, float *sm, const float *gout, float *part, bool first,
+                                              int tid, int sg, int ng) {
+#pragma unroll
+    for (int l = LMAX - 1; l >= 0; --l) {
+        if (l < L) {
+            const LLayer &Ly = net.L[l];
+            const float *G = (l == L - 1) ? gout : sm + net.L[l + 1 < LMAX ? l + 1 : l].h_off;
+            float *H = sm + Ly.h_off;
+            const int pg = Ly.N + 4, ph = Ly.K + 4;
+            const int kgs = Ly.K >> 2;
+            {
+                const int kt = Ly.K / Ly.rk, nt = Ly.N / Ly.rn;
+                if (tid < nt * kt) {
+                    // tn runs fastest: the threads that also sum the bias gradient (tk == 0) are the first nt of the
+                    // block, so the other warps skip those adds (they were 5 % of all issued instructions)
+                    const int tk = tid / nt, tn = tid - tk * nt;
+                    float dw[16], db[4];
+#pragma unroll
+                    for (int e = 0; e < 16; ++e) dw[e] = 0.0f;
+#pragma unroll
+                    for (int e = 0; e < 4; ++e) db[e] = 0.0f;
+                    switch (Ly.rn * 8 + Ly.rk) {
+                    case 4 * 8 + 4: dw_layer<4, 4>(G, pg, H, ph, tn, tk, dw, db); dw_store<4, 4>(Ly, part, tn, tk, dw, db, first); break;
+                    case 2 * 8 + 4: dw_layer<2, 4>(G, pg, H, ph, tn, tk, dw, db); dw_store<2, 4>(Ly, part, tn, tk, dw, db, first); break;
+                    case 1 * 8 + 4: dw_layer<1, 4>(G, pg, H, ph, tn, tk, dw, db); dw_store<1, 4>(Ly, part, tn, tk, dw, db, first); break;
+                    case 1 * 8 + 2: dw_layer<1, 2>(G, pg, H, ph, tn, tk, dw, db); dw_store<1, 2>(Ly, part, tn, tk, dw, db, first); break;
+                    default: dw_layer<1, 1>(G, pg, H, ph, tn, tk, dw, db); dw_store<1, 1>(Ly, part, tn, tk, dw, db, first); break;
+                    }
+                }
+            }
+            if (l > 0) {
+                __syncthreads();
+                LTRACE(7 + 2 * l);
+                if (kgs == 16) bwd_layer<2>(G, pg, sm + Ly.w_off, ph, Ly.N, H, ph, kgs, sg, ng);
+                else bwd_layer<1>(G, pg, sm + Ly.w_off, ph, Ly.N, H, ph, kgs, sg, ng);
+                __syncthreads();
+                LTRACE(8 + 2 * l);
+            }
+        }
+    }
+}
+
+// block sum of every thread's loss_acc in a fixed order -> *out
+__device__ __forceinline__ void block_loss_to(float *out, float loss_acc, int tid) {
+    __shared__ float s_red[LT / 32];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) loss_acc += __shfl_xor_sync(0xffffffffu, loss_acc, o);
+    if ((tid & 31) == 0) s_red[tid >> 5] = loss_acc;
+    __syncthreads();
+    if (tid == 0) {
+        float t = 0.0f;
+        for (int w = 0; w < LT / 32; ++w) t += s_red[w];
+        *out = t;
+    }
+}
 
 // ------------------------------------------------------------------------------------------------ the gradient kernel
 __global__ void __launch_bounds__(LT, BLOCKS_PER_SM) ppo2_grad_kernel(const __grid_constant__ LearnArgs A) {
@@ -290,7 +446,6 @@ __global__ void __launch_bounds__(LT, BLOCKS_PER_SM) ppo2_grad_kernel(const __gr
     __shared__ int s_t[TM], s_i[TM];
     __shared__ float s_act[16 * TM], s_alp[16 * TM], s_tgt[TM];   // the tile's actions, old log-probs [d][s]; adv / v_target
     __shared__ float s_cst[16][4];                                 // per action dimension: var, log std, gain, offset
-    __shared__ float s_red[LT / 32];
     const int slot = (int)blockIdx.x >= A.nblk[0] ? 1 : 0;
     const int bx = (int)blockIdx.x - (slot ? A.nblk[0] : 0), nbx = A.nblk[slot];
     const int net_id = A.net_of_y[slot];
@@ -299,17 +454,7 @@ __global__ void __launch_bounds__(LT, BLOCKS_PER_SM) ppo2_grad_kernel(const __gr
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int sg = (lane & 3) + 4 * warp, ng = lane >> 2;
 
-    // weights and biases -> shared memory, zero-padded
-    for (int l = 0; l < L; ++l) {
-        const LLayer &Ly = net.L[l];
-        const int pw = Ly.K + 4;
-        for (int e = tid; e < Ly.N * pw; e += LT) {
-            const int n = e / pw, k = e - n * pw;
-            sm[Ly.w_off + e] = (n < Ly.n_real && k < Ly.k_real) ? __ldg(Ly.w + n * Ly.k_real + k) : 0.0f;
-        }
-        for (int n = tid; n < Ly.N; n += LT) sm[Ly.b_off + n] = n < Ly.n_real ? __ldg(Ly.b + n) : 0.0f;
-    }
-
+    load_weights(net, sm, tid);
     if (net_id == 0 && tid < 16) {
         const int d = tid;
         const float sd = d < A.A ? (A.std_vec ? __ldg(A.std_vec + d) : A.std_) : 1.0f;
@@ -329,30 +474,19 @@ __global__ void __launch_bounds__(LT, BLOCKS_PER_SM) ppo2_grad_kernel(const __gr
     const LLayer &LO = net.L[L - 1];
     float *gout = sm + net.gout_off;
     const int pgo = LO.N + 4;
+    const int64_t N = A.sp.N;
 
-#ifdef LEARN_TRACE
-    long long lt_prev = clock64();
-#endif
+    LTRACE_START();
     for (int64_t tile = bx; tile < tiles; tile += nbx) {
         __syncthreads();   // the previous tile's last phase has finished with H and s_t / s_i
         LTRACE(15);
-        if (tid < TM) {
-            const int64_t j = tile * TM + tid;
-            int t = -1, i = 0;
-            if (j < A.count) {
-                const int64_t b = A.index ? A.index[A.first + j] : perm_index(A.perm_key, A.first + j, A.T * A.N, A.perm_half_bits);
-                t = (int)(b / A.N);
-                i = (int)(b - (int64_t)t * A.N);
-            }
-            s_t[tid] = t;
-            s_i[tid] = i;
-        }
+        tile_samples(A.sp, tile, A.count, s_t, s_i, tid);
         __syncthreads();
         LTRACE(0);
         {   // gather: H_0[s][k] (observations) and the loss phase's inputs (actions, old log-probs, adv / v_target).
             // Thread = (sample s, field lane q): its fields are q, q + 4, ...; ALL its loads are issued before the first
-            // store to shared memory -- the obvious load-store loop serialised six DRAM round trips per tile (phase
-            // trace: 9.5 k of 82 k cycles per tile)
+            // store to shared memory -- the obvious load-store loop (gather_obs) serialised six DRAM round trips per tile
+            // (phase trace: 9.5 k of 82 k cycles per tile)
             static_assert(LT % TM == 0 && LT / TM == 4, "4 field lanes per sample");
             float *H0 = sm + L0.h_off;
             const int p0 = L0.K + 4;
@@ -363,17 +497,17 @@ __global__ void __launch_bounds__(LT, BLOCKS_PER_SM) ppo2_grad_kernel(const __gr
 #pragma unroll
             for (int j = 0; j < WMAX / 4; ++j) {
                 const int k = q + 4 * j;
-                vo[j] = (t >= 0 && k < A.S) ? __ldg(A.s + (tt * A.S + k) * A.N + i) : 0.0f;
+                vo[j] = (t >= 0 && k < A.S) ? __ldg(A.s + (tt * A.S + k) * N + i) : 0.0f;
             }
 #pragma unroll
             for (int j = 0; j < 4; ++j) {
                 const int d = q + 4 * j;
                 const bool on = net_id == 0 && t >= 0 && d < A.A;
-                const int64_t off = (tt * A.A + (on ? d : 0)) * A.N + i;
+                const int64_t off = (tt * A.A + (on ? d : 0)) * N + i;
                 va[j] = on ? __ldg(A.a + off) : 0.0f;
                 vl[j] = on ? __ldg(A.a_lp + off) : 0.0f;
             }
-            if (q == 0 && t >= 0) vt = __ldg((net_id == 0 ? A.adv : A.v_target) + tt * A.N + i);
+            if (q == 0 && t >= 0) vt = __ldg((net_id == 0 ? A.adv : A.v_target) + tt * N + i);
 #pragma unroll
             for (int j = 0; j < WMAX / 4; ++j) {
                 const int k = q + 4 * j;
@@ -390,25 +524,7 @@ __global__ void __launch_bounds__(LT, BLOCKS_PER_SM) ppo2_grad_kernel(const __gr
         }
         __syncthreads();
         LTRACE(1);
-        // ---------------------------------------------------------------- forward
-#pragma unroll
-        for (int l = 0; l < LMAX; ++l) {
-            if (l < L) {
-                const LLayer &Ly = net.L[l];
-                const bool last = l == L - 1;
-                float *out = last ? gout : sm + net.L[l + 1 < LMAX ? l + 1 : l].h_off;
-                const float *H = sm + Ly.h_off, *W = sm + Ly.w_off, *bs = sm + Ly.b_off;
-                const int ph = Ly.K + 4, po = Ly.N + 4;
-                switch (Ly.N >> 3) {
-                case 1: fwd_layer<1>(H, ph, W, ph, bs, Ly.K, out, po, !last, sg, ng); break;
-                case 2: fwd_layer<2>(H, ph, W, ph, bs, Ly.K, out, po, !last, sg, ng); break;
-                case 4: fwd_layer<4>(H, ph, W, ph, bs, Ly.K, out, po, !last, sg, ng); break;
-                default: fwd_layer<8>(H, ph, W, ph, bs, Ly.K, out, po, !last, sg, ng); break;
-                }
-                __syncthreads();
-                LTRACE(2 + l);
-            }
-        }
+        tile_forward(net, L, sm, gout, sg, ng);
         // ---------------------------------------------------------------- loss and its gradient at the net's output
         {   // two threads per sample: thread `half` takes the action dimensions half, half + 2, ...
             const int sx = tid >> 1, half = tid & 1;
@@ -466,58 +582,9 @@ __global__ void __launch_bounds__(LT, BLOCKS_PER_SM) ppo2_grad_kernel(const __gr
         }
         __syncthreads();
         LTRACE(6);
-        // ---------------------------------------------------------------- backward
-#pragma unroll
-        for (int l = LMAX - 1; l >= 0; --l) {
-            if (l < L) {
-                const LLayer &Ly = net.L[l];
-                const float *G = (l == L - 1) ? gout : sm + net.L[l + 1 < LMAX ? l + 1 : l].h_off;
-                float *H = sm + Ly.h_off;
-                const int pg = Ly.N + 4, ph = Ly.K + 4;
-                const int kgs = Ly.K >> 2;
-                {
-                    const int kt = Ly.K / Ly.rk, nt = Ly.N / Ly.rn;
-                    if (tid < nt * kt) {
-                        // tn runs fastest: the threads that also sum the bias gradient (tk == 0) are the first nt of
-                        // the block, so the other warps skip those adds (they were 5 % of all issued instructions)
-                        const int tk = tid / nt, tn = tid - tk * nt;
-                        float dw[16], db[4];
-#pragma unroll
-                        for (int e = 0; e < 16; ++e) dw[e] = 0.0f;
-#pragma unroll
-                        for (int e = 0; e < 4; ++e) db[e] = 0.0f;
-                        const bool first = tile == bx;
-                        switch (Ly.rn * 8 + Ly.rk) {
-                        case 4 * 8 + 4: dw_layer<4, 4>(G, pg, H, ph, tn, tk, dw, db); dw_store<4, 4>(Ly, part, tn, tk, dw, db, first); break;
-                        case 2 * 8 + 4: dw_layer<2, 4>(G, pg, H, ph, tn, tk, dw, db); dw_store<2, 4>(Ly, part, tn, tk, dw, db, first); break;
-                        case 1 * 8 + 4: dw_layer<1, 4>(G, pg, H, ph, tn, tk, dw, db); dw_store<1, 4>(Ly, part, tn, tk, dw, db, first); break;
-                        case 1 * 8 + 2: dw_layer<1, 2>(G, pg, H, ph, tn, tk, dw, db); dw_store<1, 2>(Ly, part, tn, tk, dw, db, first); break;
-                        default: dw_layer<1, 1>(G, pg, H, ph, tn, tk, dw, db); dw_store<1, 1>(Ly, part, tn, tk, dw, db, first); break;
-                        }
-                    }
-                }
-                if (l > 0) {
-                    __syncthreads();
-                    LTRACE(7 + 2 * l);
-                    if (kgs == 16) bwd_layer<2>(G, pg, sm + Ly.w_off, ph, Ly.N, H, ph, kgs, sg, ng);
-                    else bwd_layer<1>(G, pg, sm + Ly.w_off, ph, Ly.N, H, ph, kgs, sg, ng);
-                    __syncthreads();
-                    LTRACE(8 + 2 * l);
-                }
-            }
-        }
+        tile_backward(net, L, sm, gout, part, tile == bx, tid, sg, ng);
     }
-
-    // block sum of the loss in a fixed order
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) loss_acc += __shfl_xor_sync(0xffffffffu, loss_acc, o);
-    if (lane == 0) s_red[warp] = loss_acc;
-    __syncthreads();
-    if (tid == 0) {
-        float t = 0.0f;
-        for (int w = 0; w < LT / 32; ++w) t += s_red[w];
-        part[net.P] = t;
-    }
+    block_loss_to(part + net.P, loss_acc, tid);
 }
 
 // Sum of the per-block partial gradients in block order: one thread per parameter (consecutive threads read consecutive
@@ -575,18 +642,17 @@ __global__ void __launch_bounds__(256) ppo2_reduce_kernel(const __grid_constant_
 }
 
 // PPO v1 advantage (the joint loss of b200_ppo1_grad): adv = R_hat - V(s) with the CURRENT critic at the batch's samples,
-// before ppo2_grad_kernel reads adv.  Same sample selection, tile, shared-memory layout and fwd_layer calls as the critic
-// blocks of ppo2_grad_kernel, so V is bit-identical to the V those blocks compute from the same weights.  A separate
-// launch rather than the critic forward inside the actor's blocks: that would put both nets' weights into those blocks
-// and change the shipped gradient kernel; this costs one more read of the observations.
+// before ppo2_grad_kernel reads adv.  The critic blocks of ppo2_grad_kernel run the same tile_samples and tile_forward on
+// the same shared-memory layout, and the observations reach H_0 unchanged on both paths, so V is bit-identical to the V
+// those blocks compute from the same weights.  A separate launch rather than the critic forward inside the actor's
+// blocks: that would put both nets' weights into those blocks and change the shipped gradient kernel; this costs one more
+// read of the observations.
 struct AdvArgs {
     LNet net;                    // the critic
     int S;
-    int64_t T, N, first, count;
+    PpoSampler sp;
+    int64_t count;
     const float *s, *ret_hat;
-    const int64_t *index;
-    uint64_t perm_key;
-    int perm_half_bits;
     float *adv, *value;          // value may be NULL
 };
 __global__ void __launch_bounds__(LT, BLOCKS_PER_SM) ppo1_advantage_kernel(const __grid_constant__ AdvArgs A) {
@@ -596,62 +662,21 @@ __global__ void __launch_bounds__(LT, BLOCKS_PER_SM) ppo1_advantage_kernel(const
     const int L = net.n_layers;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int sg = (lane & 3) + 4 * warp, ng = lane >> 2;
-    for (int l = 0; l < L; ++l) {
-        const LLayer &Ly = net.L[l];
-        const int pw = Ly.K + 4;
-        for (int e = tid; e < Ly.N * pw; e += LT) {
-            const int n = e / pw, k = e - n * pw;
-            sm[Ly.w_off + e] = (n < Ly.n_real && k < Ly.k_real) ? __ldg(Ly.w + n * Ly.k_real + k) : 0.0f;
-        }
-        for (int n = tid; n < Ly.N; n += LT) sm[Ly.b_off + n] = n < Ly.n_real ? __ldg(Ly.b + n) : 0.0f;
-    }
-    const int64_t tiles = (A.count + TM - 1) / TM;
+    load_weights(net, sm, tid);
+    const int64_t tiles = (A.count + TM - 1) / TM, N = A.sp.N;
     const LLayer &L0 = net.L[0];
     float *gout = sm + net.gout_off;
     const int pgo = net.L[L - 1].N + 4;
+    LTRACE_START();
     for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
         __syncthreads();   // the previous tile's last reads of H and s_t / s_i are done
-        if (tid < TM) {
-            const int64_t j = tile * TM + tid;
-            int t = -1, i = 0;
-            if (j < A.count) {
-                const int64_t b = A.index ? A.index[A.first + j] : perm_index(A.perm_key, A.first + j, A.T * A.N, A.perm_half_bits);
-                t = (int)(b / A.N);
-                i = (int)(b - (int64_t)t * A.N);
-            }
-            s_t[tid] = t;
-            s_i[tid] = i;
-        }
+        tile_samples(A.sp, tile, A.count, s_t, s_i, tid);
         __syncthreads();
-        {   // H_0 = the gathered observations, zero-padded to K_0 (thread = sample s, fields q, q + 4, ...)
-            float *H0 = sm + L0.h_off;
-            const int p0 = L0.K + 4;
-            const int s = tid & (TM - 1), q = tid >> TM_LOG2;
-            const int t = s_t[s];
-            const int64_t i = s_i[s], tt = t < 0 ? 0 : t;
-            for (int k = q; k < L0.K; k += LT / TM)
-                H0[s * p0 + k] = (t >= 0 && k < A.S) ? __ldg(A.s + (tt * A.S + k) * A.N + i) : 0.0f;
-        }
+        gather_obs(A.s, A.S, N, L0.K, s_t, s_i, sm + L0.h_off, L0.K + 4, tid);
         __syncthreads();
-#pragma unroll
-        for (int l = 0; l < LMAX; ++l) {
-            if (l < L) {
-                const LLayer &Ly = net.L[l];
-                const bool last = l == L - 1;
-                float *out = last ? gout : sm + net.L[l + 1 < LMAX ? l + 1 : l].h_off;
-                const float *H = sm + Ly.h_off, *W = sm + Ly.w_off, *bs = sm + Ly.b_off;
-                const int ph = Ly.K + 4, po = Ly.N + 4;
-                switch (Ly.N >> 3) {
-                case 1: fwd_layer<1>(H, ph, W, ph, bs, Ly.K, out, po, !last, sg, ng); break;
-                case 2: fwd_layer<2>(H, ph, W, ph, bs, Ly.K, out, po, !last, sg, ng); break;
-                case 4: fwd_layer<4>(H, ph, W, ph, bs, Ly.K, out, po, !last, sg, ng); break;
-                default: fwd_layer<8>(H, ph, W, ph, bs, Ly.K, out, po, !last, sg, ng); break;
-                }
-                __syncthreads();
-            }
-        }
+        tile_forward(net, L, sm, gout, sg, ng);
         if (tid < TM && s_t[tid] >= 0) {
-            const int64_t b = (int64_t)s_t[tid] * A.N + s_i[tid];
+            const int64_t b = (int64_t)s_t[tid] * N + s_i[tid];
             const float v = gout[tid * pgo];
             A.adv[b] = __fsub_rn(__ldg(A.ret_hat + b), v);
             if (A.value) A.value[b] = v;
@@ -694,33 +719,20 @@ struct DqnSampler {
     int64_t R, N, newest, V;
     const int64_t *index;
     uint64_t key;
-};
-__host__ __device__ __forceinline__ int64_t dqn_sample_pos(const DqnSampler &p, int64_t j) {
-    if (p.index) return p.index[j];
-    const uint64_t h = dqn_mix(p.key, (uint64_t)j), vn = (uint64_t)(p.V * p.N);
+    __host__ __device__ __forceinline__ int64_t pos(int64_t j) const {
+        if (index) return index[j];
+        const uint64_t h = dqn_mix(key, (uint64_t)j), vn = (uint64_t)(V * N);
 #ifdef __CUDA_ARCH__
-    const uint64_t b = __umul64hi(h, vn);
+        const uint64_t b = __umul64hi(h, vn);
 #else
-    const uint64_t b = (uint64_t)(((unsigned __int128)h * vn) >> 64);
+        const uint64_t b = (uint64_t)(((unsigned __int128)h * vn) >> 64);
 #endif
-    const int64_t back = (int64_t)(b / (uint64_t)p.N), i = (int64_t)b - back * p.N;
-    int64_t row = p.newest - back;
-    if (row < 0) row += p.R;
-    return row * p.N + i;
-}
-
-// weights and biases of `net` -> w (shared memory, the offsets of fill_net), zero-padded
-__device__ __forceinline__ void dqn_load_weights(const LNet &net, float *w, int tid) {
-    for (int l = 0; l < net.n_layers; ++l) {
-        const LLayer &Ly = net.L[l];
-        const int pw = Ly.K + 4;
-        for (int e = tid; e < Ly.N * pw; e += LT) {
-            const int n = e / pw, k = e - n * pw;
-            w[Ly.w_off + e] = (n < Ly.n_real && k < Ly.k_real) ? __ldg(Ly.w + n * Ly.k_real + k) : 0.0f;
-        }
-        for (int n = tid; n < Ly.N; n += LT) w[Ly.b_off + n] = n < Ly.n_real ? __ldg(Ly.b + n) : 0.0f;
+        const int64_t back = (int64_t)(b / (uint64_t)N), i = (int64_t)b - back * N;
+        int64_t row = newest - back;
+        if (row < 0) row += R;
+        return row * N + i;
     }
-}
+};
 
 // Forward-only pass of the tile in X: the layers alternate between P and Q (all three [TM][pw]); returns the buffer that
 // holds the output [TM][A].  Ends with a barrier.  X is not written, so a second net can run on the same input.
@@ -731,16 +743,7 @@ __device__ __forceinline__ const float *dqn_forward(const LNet &net, const float
 #pragma unroll
     for (int l = 0; l < LMAX; ++l) {
         if (l < net.n_layers) {
-            const LLayer &Ly = net.L[l];
-            const bool hidden = l + 1 < net.n_layers;
-            const float *W = w + Ly.w_off, *bs = w + Ly.b_off;
-            const int pk = Ly.K + 4;
-            switch (Ly.N >> 3) {
-            case 1: fwd_layer<1>(in, pw, W, pk, bs, Ly.K, out, pw, hidden, sg, ng); break;
-            case 2: fwd_layer<2>(in, pw, W, pk, bs, Ly.K, out, pw, hidden, sg, ng); break;
-            case 4: fwd_layer<4>(in, pw, W, pk, bs, Ly.K, out, pw, hidden, sg, ng); break;
-            default: fwd_layer<8>(in, pw, W, pk, bs, Ly.K, out, pw, hidden, sg, ng); break;
-            }
+            fwd_any(net.L[l], w, in, pw, out, pw, l + 1 < net.n_layers, sg, ng);
             __syncthreads();
             in = out;
             out = out == P ? Q : P;
@@ -775,7 +778,7 @@ __global__ void __launch_bounds__(LT, BLOCKS_PER_SM) dqn_act_kernel(const __grid
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int sg = (lane & 3) + 4 * warp, ng = lane >> 2;
     float *X = sm + A.wfl, *P = X + TM * A.pw, *Q = P + TM * A.pw;
-    dqn_load_weights(A.net, sm, tid);
+    load_weights(A.net, sm, tid);
     const int64_t tiles = (A.n + TM - 1) / TM;
     const int K0 = A.net.L[0].K;
     for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
@@ -833,31 +836,15 @@ __global__ void __launch_bounds__(LT, BLOCKS_PER_SM) dqn_target_kernel(const __g
     const int sg = (lane & 3) + 4 * warp, ng = lane >> 2;
     float *wo = sm + A.wfl;
     float *X = sm + (A.double_q ? 2 : 1) * A.wfl, *P = X + TM * A.pw, *Q = P + TM * A.pw;
-    dqn_load_weights(A.tnet, sm, tid);
-    if (A.double_q) dqn_load_weights(A.onet, wo, tid);
+    load_weights(A.tnet, sm, tid);
+    if (A.double_q) load_weights(A.onet, wo, tid);
     const int64_t tiles = (A.count + TM - 1) / TM, N = A.sp.N;
     const int K0 = A.tnet.L[0].K;
     for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
         __syncthreads();
-        if (tid < TM) {
-            const int64_t j = tile * TM + tid;
-            int t = -1, i = 0;
-            if (j < A.count) {
-                const int64_t p = dqn_sample_pos(A.sp, j);
-                t = (int)(p / N);
-                i = (int)(p - (int64_t)t * N);
-            }
-            s_t[tid] = t;
-            s_i[tid] = i;
-        }
+        tile_samples(A.sp, tile, A.count, s_t, s_i, tid);
         __syncthreads();
-        {
-            const int s = tid & (TM - 1), q = tid >> TM_LOG2;
-            const int t = s_t[s];
-            const int64_t i = s_i[s], tt = t < 0 ? 0 : t;
-            for (int k = q; k < K0; k += LT / TM)
-                X[s * A.pw + k] = (t >= 0 && k < A.S) ? __ldg(A.s_ + (tt * A.S + k) * N + i) : 0.0f;
-        }
+        gather_obs(A.s_, A.S, N, K0, s_t, s_i, X, A.pw, tid);
         __syncthreads();
         if (A.double_q) {
             const float *Z = dqn_forward(A.onet, wo, X, P, Q, A.pw, sg, ng);
@@ -893,13 +880,12 @@ __global__ void __launch_bounds__(LT, BLOCKS_PER_SM) dqn_grad_kernel(const __gri
     extern __shared__ __align__(16) float sm[];
     __shared__ int s_t[TM], s_i[TM], s_a[TM];
     __shared__ float s_y[TM];
-    __shared__ float s_red[LT / 32];
     const LNet &net = A.net;
     const int L = net.n_layers;
     const int bx = blockIdx.x, nbx = gridDim.x;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int sg = (lane & 3) + 4 * warp, ng = lane >> 2;
-    dqn_load_weights(net, sm, tid);
+    load_weights(net, sm, tid);
     float loss_acc = 0.0f;
     float *part = A.partial + (size_t)bx * (size_t)(net.P + 4);
     const int64_t tiles = (A.count + TM - 1) / TM, N = A.sp.N;
@@ -907,49 +893,18 @@ __global__ void __launch_bounds__(LT, BLOCKS_PER_SM) dqn_grad_kernel(const __gri
     const LLayer &LO = net.L[L - 1];
     float *gout = sm + net.gout_off;
     const int pgo = LO.N + 4;
+    LTRACE_START();
     for (int64_t tile = bx; tile < tiles; tile += nbx) {
         __syncthreads();
+        const int64_t p = tile_samples(A.sp, tile, A.count, s_t, s_i, tid);
         if (tid < TM) {
-            const int64_t j = tile * TM + tid;
-            int t = -1, i = 0, act = 0;
-            float y = 0.0f;
-            if (j < A.count) {
-                const int64_t p = dqn_sample_pos(A.sp, j);
-                t = (int)(p / N);
-                i = (int)(p - (int64_t)t * N);
-                act = __ldg(A.a + p);
-                y = __ldg(A.y + j);
-            }
-            s_t[tid] = t; s_i[tid] = i; s_a[tid] = act; s_y[tid] = y;
+            s_a[tid] = p >= 0 ? __ldg(A.a + p) : 0;
+            s_y[tid] = p >= 0 ? __ldg(A.y + tile * TM + tid) : 0.0f;
         }
         __syncthreads();
-        {
-            float *H0 = sm + L0.h_off;
-            const int p0 = L0.K + 4;
-            const int s = tid & (TM - 1), q = tid >> TM_LOG2;
-            const int t = s_t[s];
-            const int64_t i = s_i[s], tt = t < 0 ? 0 : t;
-            for (int k = q; k < L0.K; k += LT / TM)
-                H0[s * p0 + k] = (t >= 0 && k < A.S) ? __ldg(A.s + (tt * A.S + k) * N + i) : 0.0f;
-        }
+        gather_obs(A.s, A.S, N, L0.K, s_t, s_i, sm + L0.h_off, L0.K + 4, tid);
         __syncthreads();
-#pragma unroll
-        for (int l = 0; l < LMAX; ++l) {
-            if (l < L) {
-                const LLayer &Ly = net.L[l];
-                const bool last = l == L - 1;
-                float *out = last ? gout : sm + net.L[l + 1 < LMAX ? l + 1 : l].h_off;
-                const float *H = sm + Ly.h_off, *W = sm + Ly.w_off, *bs = sm + Ly.b_off;
-                const int ph = Ly.K + 4, po = Ly.N + 4;
-                switch (Ly.N >> 3) {
-                case 1: fwd_layer<1>(H, ph, W, ph, bs, Ly.K, out, po, !last, sg, ng); break;
-                case 2: fwd_layer<2>(H, ph, W, ph, bs, Ly.K, out, po, !last, sg, ng); break;
-                case 4: fwd_layer<4>(H, ph, W, ph, bs, Ly.K, out, po, !last, sg, ng); break;
-                default: fwd_layer<8>(H, ph, W, ph, bs, Ly.K, out, po, !last, sg, ng); break;
-                }
-                __syncthreads();
-            }
-        }
+        tile_forward(net, L, sm, gout, sg, ng);
         {   // four lanes per sample, in one warp: all read Q[a] before any of them writes dZ over the row
             const int sx = tid >> 2, q = tid & 3;
             float *z = gout + sx * pgo;
@@ -963,51 +918,9 @@ __global__ void __launch_bounds__(LT, BLOCKS_PER_SM) dqn_grad_kernel(const __gri
             for (int d = q; d < LO.N; d += 4) z[d] = d == act ? c : 0.0f;
         }
         __syncthreads();
-#pragma unroll
-        for (int l = LMAX - 1; l >= 0; --l) {
-            if (l < L) {
-                const LLayer &Ly = net.L[l];
-                const float *G = (l == L - 1) ? gout : sm + net.L[l + 1 < LMAX ? l + 1 : l].h_off;
-                float *H = sm + Ly.h_off;
-                const int pg = Ly.N + 4, ph = Ly.K + 4;
-                const int kgs = Ly.K >> 2;
-                {
-                    const int kt = Ly.K / Ly.rk, nt = Ly.N / Ly.rn;
-                    if (tid < nt * kt) {
-                        const int tk = tid / nt, tn = tid - tk * nt;
-                        float dw[16], db[4];
-#pragma unroll
-                        for (int e = 0; e < 16; ++e) dw[e] = 0.0f;
-#pragma unroll
-                        for (int e = 0; e < 4; ++e) db[e] = 0.0f;
-                        const bool first = tile == bx;
-                        switch (Ly.rn * 8 + Ly.rk) {
-                        case 4 * 8 + 4: dw_layer<4, 4>(G, pg, H, ph, tn, tk, dw, db); dw_store<4, 4>(Ly, part, tn, tk, dw, db, first); break;
-                        case 2 * 8 + 4: dw_layer<2, 4>(G, pg, H, ph, tn, tk, dw, db); dw_store<2, 4>(Ly, part, tn, tk, dw, db, first); break;
-                        case 1 * 8 + 4: dw_layer<1, 4>(G, pg, H, ph, tn, tk, dw, db); dw_store<1, 4>(Ly, part, tn, tk, dw, db, first); break;
-                        case 1 * 8 + 2: dw_layer<1, 2>(G, pg, H, ph, tn, tk, dw, db); dw_store<1, 2>(Ly, part, tn, tk, dw, db, first); break;
-                        default: dw_layer<1, 1>(G, pg, H, ph, tn, tk, dw, db); dw_store<1, 1>(Ly, part, tn, tk, dw, db, first); break;
-                        }
-                    }
-                }
-                if (l > 0) {
-                    __syncthreads();
-                    if (kgs == 16) bwd_layer<2>(G, pg, sm + Ly.w_off, ph, Ly.N, H, ph, kgs, sg, ng);
-                    else bwd_layer<1>(G, pg, sm + Ly.w_off, ph, Ly.N, H, ph, kgs, sg, ng);
-                    __syncthreads();
-                }
-            }
-        }
+        tile_backward(net, L, sm, gout, part, tile == bx, tid, sg, ng);
     }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) loss_acc += __shfl_xor_sync(0xffffffffu, loss_acc, o);
-    if (lane == 0) s_red[warp] = loss_acc;
-    __syncthreads();
-    if (tid == 0) {
-        float t = 0.0f;
-        for (int w = 0; w < LT / 32; ++w) t += s_red[w];
-        part[net.P] = t;
-    }
+    block_loss_to(part + net.P, loss_acc, tid);
 }
 
 // ------------------------------------------------------------------------------------------------ clip + Adam
@@ -1121,6 +1034,29 @@ int grid_cap() {
     return sms[dev];
 }
 
+// blocks of a launch over `count` samples: one per tile, at most grid_cap()
+int grid_for(int64_t count) {
+    const int64_t tiles = (count + TM - 1) / TM;
+    const int cap = grid_cap();
+    return (int)(tiles < cap ? tiles : cap);
+}
+
+// raises `k`'s dynamic shared-memory limit to `smem` once per device (configured: the kernel's limit per device)
+template <typename Kernel>
+int set_smem(Kernel k, size_t smem, size_t (&configured)[64]) {
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (dev < 0 || dev >= 64) dev = 0;
+    if (smem > 48 * 1024 && smem > configured[dev]) {
+        if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+            return b200_check_launch();
+        configured[dev] = smem;
+    }
+    return B200ENV_OK;
+}
+
+constexpr size_t SMEM_MAX = 227 * 1024 - 12 * 1024;   // room for the kernels' static shared memory (~10 KB) next to it
+
 size_t partial_floats(const LNet &n) { return (size_t)GRID_CAP * (size_t)(n.P + 4); }
 
 struct Plan {
@@ -1141,7 +1077,7 @@ int make_plan(const b200_ppo2_batch *bt, const b200_mlp *actor, const b200_mlp *
     a = LearnArgs{};
     int rc;
     pl->nets = 0;
-    size_t smem_f = 0, ws = 64;
+    size_t smem_f = 0, ws = 64;   // the partials start after 64 unused bytes, as b200_ppo2_workspace_bytes counts them
     if (actor) {
         if (!grad_actor || !bt->a || !bt->a_lp) return B200ENV_ENULL;
         if (!std_vec && !(std_ > 0.0f)) return B200ENV_EPARAMS;
@@ -1169,62 +1105,63 @@ int make_plan(const b200_ppo2_batch *bt, const b200_mlp *actor, const b200_mlp *
     }
     if (ws > workspace_bytes) return B200ENV_ESIZE;
     pl->smem = smem_f * sizeof(float);
-    if (pl->smem > 227 * 1024 - 12 * 1024) return B200ENV_ESIZE;   // ~10 KB of static shared memory next to it
-    a.T = bt->T; a.N = bt->N; a.first = bt->first; a.count = bt->count;
+    if (pl->smem > SMEM_MAX) return B200ENV_ESIZE;
+    a.sp = {bt->T, bt->N, bt->first, bt->index, bt->perm_key, half_bits_for(B)};
+    a.count = bt->count;
     a.s = bt->s; a.a = bt->a; a.a_lp = bt->a_lp; a.adv = bt->adv; a.v_target = bt->v_target;
-    a.index = bt->index;
-    a.perm_key = bt->perm_key;
-    a.perm_half_bits = half_bits_for(B);
     a.eps_clip = eps_clip;
     a.inv_count = 1.0f / (float)bt->count;
     a.std_ = std_; a.std_vec = std_vec; a.a_min = a_min; a.a_max = a_max;
     a.entropy_coef = entropy_coef;
     a.grad[0] = grad_actor; a.grad[1] = grad_critic;
     a.loss_out = loss_out;
-    a.counter = static_cast<unsigned int *>(workspace);
     return B200ENV_OK;
+}
+
+// ppo2_reduce_kernel over r.nets slots: r gives everything but the launch's block layout (first_block)
+int launch_reduce(ReduceArgs r, cudaStream_t stream) {
+    int blocks = 0;
+    for (int y = 0; y < r.nets; ++y) {
+        r.first_block[y] = blocks;
+        blocks += (r.P[y] + 1 + 255) / 256;
+    }
+    ppo2_reduce_kernel<<<blocks, 256, 0, stream>>>(r);
+    return b200_check_launch();
 }
 
 int launch_grad(Plan &pl, cudaStream_t stream, float critic_scale = 1.0f) {
     static size_t configured[64] = {0};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64) dev = 0;
-    if (pl.smem > 48 * 1024 && pl.smem > configured[dev]) {
-        if (cudaFuncSetAttribute(ppo2_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem) != cudaSuccess)
-            return b200_check_launch();
-        configured[dev] = pl.smem;
-    }
-    const int64_t tiles = (pl.a.count + TM - 1) / TM;
-    // one block per SM; the SMs are dealt to the two nets in proportion to their work per sample (3 x sum K N), so that
-    // the actor's and the critic's blocks finish together (an even split left the critic's SMs idle 60 % of the time)
-    const int cap = grid_cap();
-    double work[2] = {0.0, 0.0};
-    for (int y = 0; y < pl.nets; ++y) {
-        const LNet &n = pl.a.net[pl.a.net_of_y[y]];
-        for (int l = 0; l < n.n_layers; ++l) work[y] += (double)n.L[l].K * n.L[l].N;
-        work[y] += 2200.0;   // per-tile fixed part (indices, gather, loss, barriers) in units of one K x N product term:
-                             // phase trace, ~20 k of an actor tile's 82 k cycles; with 64 the critic's blocks were the tail
-    }
+    int rc = set_smem(ppo2_grad_kernel, pl.smem, configured);
+    if (rc) return rc;
     pl.a.nblk[1] = 0;
     if (pl.nets == 2) {
+        // one block per SM; the SMs are dealt to the two nets in proportion to their work per sample (3 x sum K N), so
+        // that the actor's and the critic's blocks finish together (an even split left the critic's SMs idle 60 % of the
+        // time)
+        const int64_t tiles = (pl.a.count + TM - 1) / TM;
+        const int cap = grid_cap();
+        double work[2] = {0.0, 0.0};
+        for (int y = 0; y < 2; ++y) {
+            const LNet &n = pl.a.net[pl.a.net_of_y[y]];
+            for (int l = 0; l < n.n_layers; ++l) work[y] += (double)n.L[l].K * n.L[l].N;
+            work[y] += 2200.0;   // per-tile fixed part (indices, gather, loss, barriers) in units of one K x N product
+                                 // term: phase trace, ~20 k of an actor tile's 82 k cycles; with 64 the critic's blocks
+                                 // were the tail
+        }
         int nb1 = (int)(cap * work[1] / (work[0] + work[1]) + 0.5);
         nb1 = nb1 < 1 ? 1 : (nb1 > cap - 1 ? cap - 1 : nb1);
         pl.a.nblk[0] = (int)(tiles < cap - nb1 ? tiles : cap - nb1);
         pl.a.nblk[1] = (int)(tiles < nb1 ? tiles : nb1);
     } else {
-        pl.a.nblk[0] = (int)(tiles < cap ? tiles : cap);
+        pl.a.nblk[0] = grid_for(pl.a.count);
     }
     ppo2_grad_kernel<<<pl.a.nblk[0] + pl.a.nblk[1], LT, pl.smem, stream>>>(pl.a);
     ReduceArgs r = {};
-    int blocks = 0;
     for (int y = 0; y < pl.nets; ++y) {
         const int id = pl.a.net_of_y[y];
         r.partial[y] = pl.a.partial[id];
         r.grad[y] = pl.a.grad[id];
         r.P[y] = pl.a.net[id].P;
-        r.first_block[y] = blocks;
-        blocks += (pl.a.net[id].P + 1 + 255) / 256;
     }
     // loss_out is indexed by net id (0 actor, 1 critic): with a single net present its slot is selected here
     r.loss_out = pl.a.loss_out + (pl.nets == 1 ? pl.a.net_of_y[0] : 0);
@@ -1234,8 +1171,7 @@ int launch_grad(Plan &pl, cudaStream_t stream, float critic_scale = 1.0f) {
     r.scale1 = critic_scale;   // slot 1 exists only in two-net launches, and is the critic there
     r.ent_slot = (pl.a.net_of_y[0] == 0 && pl.a.entropy_coef != 0.0f) ? 0 : -1;
     r.A = pl.a.A; r.ent_coef = pl.a.entropy_coef; r.std_ = pl.a.std_; r.std_vec = pl.a.std_vec;
-    ppo2_reduce_kernel<<<blocks, 256, 0, stream>>>(r);
-    return b200_check_launch();
+    return launch_reduce(r, stream);
 }
 
 int launch_adam(int n_seg, const int64_t *seg_off, const int64_t *seg_len, const float *lr, float *param, const float *grad,
@@ -1315,10 +1251,10 @@ extern "C" B200_API int b200_ppo1_grad(const b200_ppo2_batch *batch, const b200_
     if (rc) return rc;
     {   // adv and value are written by the advantage launch while R_hat, s, a, a_lp and the index are read by both launches:
         // an output that overlaps an input (e.g. adv == v_target for an in-place call) would be read back as that input
-        const size_t tn = (size_t)pl.a.T * (size_t)pl.a.N * sizeof(float);
+        const size_t tn = (size_t)pl.a.sp.T * (size_t)pl.a.sp.N * sizeof(float);
         const size_t tan_ = tn * (size_t)pl.a.A, tsn = tn * (size_t)pl.a.S;
         const void *in[5] = {batch->v_target, batch->s, batch->a, batch->a_lp, batch->index};
-        const size_t in_bytes[5] = {tn, tsn, tan_, tan_, (size_t)(pl.a.first + pl.a.count) * sizeof(int64_t)};
+        const size_t in_bytes[5] = {tn, tsn, tan_, tan_, (size_t)(pl.a.sp.first + pl.a.count) * sizeof(int64_t)};
         const void *out[2] = {batch->adv, value};
         for (int o = 0; o < 2; ++o) {
             if (!out[o]) continue;
@@ -1330,27 +1266,16 @@ extern "C" B200_API int b200_ppo1_grad(const b200_ppo2_batch *batch, const b200_
     AdvArgs v = {};
     v.net = pl.a.net[1];
     v.S = pl.a.S;
-    v.T = pl.a.T; v.N = pl.a.N; v.first = pl.a.first; v.count = pl.a.count;
+    v.sp = pl.a.sp;
+    v.count = pl.a.count;
     v.s = batch->s; v.ret_hat = batch->v_target;
-    v.index = batch->index;
-    v.perm_key = pl.a.perm_key;
-    v.perm_half_bits = pl.a.perm_half_bits;
     v.adv = const_cast<float *>(batch->adv);   // the caller-owned [T][N] buffer this call fills
     v.value = value;
     const size_t smem = (size_t)v.net.smem_floats * sizeof(float);
     cudaStream_t stream = (cudaStream_t)cuda_stream;
     static size_t configured[64] = {0};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64) dev = 0;
-    if (smem > 48 * 1024 && smem > configured[dev]) {
-        if (cudaFuncSetAttribute(ppo1_advantage_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-            return b200_check_launch();
-        configured[dev] = smem;
-    }
-    const int64_t tiles = (v.count + TM - 1) / TM;
-    const int cap = grid_cap();
-    ppo1_advantage_kernel<<<(unsigned)(tiles < cap ? tiles : cap), LT, smem, stream>>>(v);
+    if ((rc = set_smem(ppo1_advantage_kernel, smem, configured))) return rc;
+    ppo1_advantage_kernel<<<grid_for(v.count), LT, smem, stream>>>(v);
     if ((rc = b200_check_launch())) return rc;
     return launch_grad(pl, stream, value_coef);
 }
@@ -1408,8 +1333,6 @@ extern "C" B200_API int b200_ppo2_permutation(uint64_t perm_key, int64_t B, int6
 
 // ------------------------------------------------------------------------------------------------ DQN host side
 namespace {
-constexpr size_t SMEM_MAX = 227 * 1024 - 12 * 1024;   // as make_plan: room for the kernels' static shared memory
-
 // a Q-net: fill_net with heads up to 64 wide, identity head
 int dqn_fill(const b200_mlp *m, LNet *n) {
     int rc = fill_net(m, WMAX, n);
@@ -1430,19 +1353,6 @@ bool overlaps_net(const void *x, size_t bytes, const b200_mlp *m) {
         if (overlaps(x, bytes, m->w[l], (size_t)m->dims[l] * m->dims[l + 1] * 4) ||
             overlaps(x, bytes, m->b[l], (size_t)m->dims[l + 1] * 4)) return true;
     return false;
-}
-
-template <typename Kernel>
-int set_smem(Kernel k, size_t smem, size_t (&configured)[64]) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64) dev = 0;
-    if (smem > 48 * 1024 && smem > configured[dev]) {
-        if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-            return b200_check_launch();
-        configured[dev] = smem;
-    }
-    return B200ENV_OK;
 }
 } // namespace
 
@@ -1480,9 +1390,7 @@ extern "C" B200_API int b200_dqn_act(int64_t n, const b200_mlp *q, const float *
     a.index = action_index; a.value = action_value; a.q = q_out;
     static size_t configured[64] = {0};
     if ((rc = set_smem(dqn_act_kernel, smem, configured))) return rc;
-    const int64_t tiles = (n + TM - 1) / TM;
-    const int cap = grid_cap();
-    dqn_act_kernel<<<(unsigned)(tiles < cap ? tiles : cap), LT, smem, (cudaStream_t)cuda_stream>>>(a);
+    dqn_act_kernel<<<grid_for(n), LT, smem, (cudaStream_t)cuda_stream>>>(a);
     return b200_check_launch();
 }
 
@@ -1548,9 +1456,7 @@ extern "C" B200_API int b200_dqn_grad(const b200_dqn_batch *bt, const b200_mlp *
     cudaStream_t stream = (cudaStream_t)cuda_stream;
     static size_t conf_t[64] = {0}, conf_g[64] = {0};
     if ((rc = set_smem(dqn_target_kernel, smem_t, conf_t)) || (rc = set_smem(dqn_grad_kernel, smem_g, conf_g))) return rc;
-    const int64_t tiles = (count + TM - 1) / TM;
-    const int cap = grid_cap();
-    const int blocks = (int)(tiles < cap ? tiles : cap);
+    const int blocks = grid_for(count);
     dqn_target_kernel<<<blocks, LT, smem_t, stream>>>(t);
     if ((rc = b200_check_launch())) return rc;
     dqn_grad_kernel<<<blocks, LT, smem_g, stream>>>(g);
@@ -1565,8 +1471,7 @@ extern "C" B200_API int b200_dqn_grad(const b200_dqn_batch *bt, const b200_mlp *
     r.inv_count = g.inv_count;
     r.scale1 = 1.0f;
     r.ent_slot = -1;
-    ppo2_reduce_kernel<<<(g.net.P + 1 + 255) / 256, 256, 0, stream>>>(r);
-    return b200_check_launch();
+    return launch_reduce(r, stream);
 }
 
 extern "C" B200_API int b200_dqn_sample_indices(uint64_t sample_key, int64_t newest_row, int64_t valid_rows, int64_t R,
@@ -1576,7 +1481,7 @@ extern "C" B200_API int b200_dqn_sample_indices(uint64_t sample_key, int64_t new
     if (valid_rows < 1 || valid_rows > R - 1 || newest_row < 0 || newest_row >= R) return B200ENV_EPARAMS;
     if (!out_host && count) return B200ENV_ENULL;
     const DqnSampler sp = {R, N, newest_row, valid_rows, nullptr, sample_key};
-    for (int64_t j = 0; j < count; ++j) out_host[j] = dqn_sample_pos(sp, first + j);
+    for (int64_t j = 0; j < count; ++j) out_host[j] = sp.pos(first + j);
     return B200ENV_OK;
 }
 
