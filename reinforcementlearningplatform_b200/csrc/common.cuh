@@ -303,9 +303,8 @@ static inline int b200_check_launch() {
     return B200ENV_OK;
 }
 
-// grid of a persistent kernel: blocks_per_sm resident blocks on every SM of the current device (148 on B200), never
-// more blocks than tiles
-static inline unsigned b200_persistent_grid(int64_t n, int blocks_per_sm, int block = B200_BLOCK) {
+// number of SMs of the current device (148 on B200), queried once per device
+static inline int b200_sm_count() {
     static int sms[64] = {0};
     int dev = 0;
     cudaGetDevice(&dev);
@@ -315,8 +314,29 @@ static inline unsigned b200_persistent_grid(int64_t n, int blocks_per_sm, int bl
         if (cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || v <= 0) v = 148;
         sms[dev] = v;
     }
-    const int64_t tiles = (n + block - 1) / block, cap = (int64_t)sms[dev] * blocks_per_sm;
+    return sms[dev];
+}
+
+// grid of a persistent kernel: blocks_per_sm resident blocks on every SM of the current device, never more blocks than
+// tiles
+static inline unsigned b200_persistent_grid(int64_t n, int blocks_per_sm, int block = B200_BLOCK) {
+    const int64_t tiles = (n + block - 1) / block, cap = (int64_t)b200_sm_count() * blocks_per_sm;
     return (unsigned)(tiles < cap ? tiles : cap);
+}
+
+// raises `kernel`'s dynamic shared-memory limit to `bytes` where a launch needs more than the default 48 KB, once per
+// device and size (configured: the kernel's limit so far, per device)
+template <typename Kernel>
+static inline int b200_opt_in_smem(Kernel kernel, size_t bytes, size_t (&configured)[64]) {
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (dev < 0 || dev >= 64) dev = 0;
+    if (bytes > 48 * 1024 && bytes > configured[dev]) {
+        if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes) != cudaSuccess)
+            return b200_check_launch();
+        configured[dev] = bytes;
+    }
+    return B200ENV_OK;
 }
 // float32 I/O buffers with fp64 arithmetic (b200env_io::io_dtype); in F32 mode everything is float anyway
 static inline bool b200_io32(const b200env_io *io) { return io->io_dtype == B200ENV_F32; }

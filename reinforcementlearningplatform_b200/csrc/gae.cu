@@ -358,11 +358,9 @@ extern "C" B200_API int b200_adv_normalize(int64_t count, float *adv, const doub
                                            void *cuda_stream) {
     if (count <= 0) return B200ENV_ESIZE;
     if (!adv || !stats) return B200ENV_ENULL;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const int64_t cap = (int64_t)b200_sm_count() * 16;
     int64_t blocks = (count + 255) / 256;
-    if (blocks > (int64_t)sms * 16) blocks = (int64_t)sms * 16;
+    if (blocks > cap) blocks = cap;
     adv_normalize_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)cuda_stream>>>(count, adv, stats, eps);
     return b200_check_launch();
 }

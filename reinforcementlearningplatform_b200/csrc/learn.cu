@@ -1021,17 +1021,8 @@ int fill_net(const b200_mlp *m, int max_out, LNet *net) {
 }
 
 int grid_cap() {
-    static int sms[64] = {0};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64) dev = 0;
-    if (!sms[dev]) {
-        int v = 0;
-        if (cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || v <= 0) v = 148;
-        v *= BLOCKS_PER_SM;
-        sms[dev] = v > GRID_CAP ? GRID_CAP : v;
-    }
-    return sms[dev];
+    const int v = b200_sm_count() * BLOCKS_PER_SM;
+    return v > GRID_CAP ? GRID_CAP : v;
 }
 
 // blocks of a launch over `count` samples: one per tile, at most grid_cap()
@@ -1039,20 +1030,6 @@ int grid_for(int64_t count) {
     const int64_t tiles = (count + TM - 1) / TM;
     const int cap = grid_cap();
     return (int)(tiles < cap ? tiles : cap);
-}
-
-// raises `k`'s dynamic shared-memory limit to `smem` once per device (configured: the kernel's limit per device)
-template <typename Kernel>
-int set_smem(Kernel k, size_t smem, size_t (&configured)[64]) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64) dev = 0;
-    if (smem > 48 * 1024 && smem > configured[dev]) {
-        if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-            return b200_check_launch();
-        configured[dev] = smem;
-    }
-    return B200ENV_OK;
 }
 
 constexpr size_t SMEM_MAX = 227 * 1024 - 12 * 1024;   // room for the kernels' static shared memory (~10 KB) next to it
@@ -1131,7 +1108,7 @@ int launch_reduce(ReduceArgs r, cudaStream_t stream) {
 
 int launch_grad(Plan &pl, cudaStream_t stream, float critic_scale = 1.0f) {
     static size_t configured[64] = {0};
-    int rc = set_smem(ppo2_grad_kernel, pl.smem, configured);
+    int rc = b200_opt_in_smem(ppo2_grad_kernel, pl.smem, configured);
     if (rc) return rc;
     pl.a.nblk[1] = 0;
     if (pl.nets == 2) {
@@ -1274,7 +1251,7 @@ extern "C" B200_API int b200_ppo1_grad(const b200_ppo2_batch *batch, const b200_
     const size_t smem = (size_t)v.net.smem_floats * sizeof(float);
     cudaStream_t stream = (cudaStream_t)cuda_stream;
     static size_t configured[64] = {0};
-    if ((rc = set_smem(ppo1_advantage_kernel, smem, configured))) return rc;
+    if ((rc = b200_opt_in_smem(ppo1_advantage_kernel, smem, configured))) return rc;
     ppo1_advantage_kernel<<<grid_for(v.count), LT, smem, stream>>>(v);
     if ((rc = b200_check_launch())) return rc;
     return launch_grad(pl, stream, value_coef);
@@ -1389,7 +1366,7 @@ extern "C" B200_API int b200_dqn_act(int64_t n, const b200_mlp *q, const float *
     a.seed = seed; a.step = step;
     a.index = action_index; a.value = action_value; a.q = q_out;
     static size_t configured[64] = {0};
-    if ((rc = set_smem(dqn_act_kernel, smem, configured))) return rc;
+    if ((rc = b200_opt_in_smem(dqn_act_kernel, smem, configured))) return rc;
     dqn_act_kernel<<<grid_for(n), LT, smem, (cudaStream_t)cuda_stream>>>(a);
     return b200_check_launch();
 }
@@ -1455,7 +1432,7 @@ extern "C" B200_API int b200_dqn_grad(const b200_dqn_batch *bt, const b200_mlp *
     if (smem_t > SMEM_MAX || smem_g > SMEM_MAX) return B200ENV_ESIZE;
     cudaStream_t stream = (cudaStream_t)cuda_stream;
     static size_t conf_t[64] = {0}, conf_g[64] = {0};
-    if ((rc = set_smem(dqn_target_kernel, smem_t, conf_t)) || (rc = set_smem(dqn_grad_kernel, smem_g, conf_g))) return rc;
+    if ((rc = b200_opt_in_smem(dqn_target_kernel, smem_t, conf_t)) || (rc = b200_opt_in_smem(dqn_grad_kernel, smem_g, conf_g))) return rc;
     const int blocks = grid_for(count);
     dqn_target_kernel<<<blocks, LT, smem_t, stream>>>(t);
     if ((rc = b200_check_launch())) return rc;

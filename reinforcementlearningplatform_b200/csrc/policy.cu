@@ -178,15 +178,8 @@ int policy_launch_fp32(int64_t n, const b200_mlp *actor, const b200_mlp *critic,
     a.io = io;
     const size_t smem = ((size_t)a.arena_floats + (size_t)rows * PB) * sizeof(float);
     if (smem > 227 * 1024) return B200ENV_ESIZE; // nets wider than shared memory holds: not supported by this kernel
-    static size_t configured[64] = {0}; // per device: the opt-in dynamic shared-memory limit set so far
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64) dev = 0;
-    if (smem > 48 * 1024 && smem > configured[dev]) {
-        if (cudaFuncSetAttribute(policy_forward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-            return b200_check_launch();
-        configured[dev] = smem;
-    }
+    static size_t configured[64] = {0};
+    if ((rc = b200_opt_in_smem(policy_forward_kernel, smem, configured))) return rc;
     int per_sm = (int)((227 * 1024) / (smem + 1024));
     if (per_sm < 1) per_sm = 1;
     if (per_sm > 8) per_sm = 8;
@@ -227,14 +220,17 @@ extern "C" B200_API int b200_policy_forward(int64_t n, const b200_mlp *actor, co
 }
 
 extern "C" B200_API size_t b200_policy_workspace_bytes(const b200_mlp *actor, const b200_mlp *critic) {
-    if (!actor && !critic) return 0;
-    return policy_umma_workspace_bytes(actor, critic);
+    PolicyRoute r;
+    if ((!actor && !critic) || policy_route(actor, critic, &r)) return 0;
+    return policy_workspace_bytes(r.p);
 }
 
 extern "C" B200_API int b200_policy_pack(const b200_mlp *actor, const b200_mlp *critic, void *workspace,
                                          size_t workspace_bytes, void *cuda_stream) {
     if (!actor && !critic) return B200ENV_ENULL;
-    return policy_umma_pack(actor, critic, workspace, workspace_bytes, (cudaStream_t)cuda_stream);
+    PolicyRoute r;
+    const int rc = policy_route(actor, critic, &r);
+    return rc ? rc : policy_pack(r, workspace, workspace_bytes, (cudaStream_t)cuda_stream);
 }
 
 extern "C" B200_API int b200_policy_forward_packed(int64_t n, const b200_mlp *actor, const b200_mlp *critic,
@@ -243,15 +239,20 @@ extern "C" B200_API int b200_policy_forward_packed(int64_t n, const b200_mlp *ac
                                                    const float *std_vec, const float *noise, uint64_t seed, uint64_t step,
                                                    int64_t env_index_offset, float *action, float *log_prob, float *mean,
                                                    float *value, void *cuda_stream) {
-    const int rc = policy_check(n, actor, critic, obs, a_min, a_max, std_, std_vec, action, value);
+    int rc = policy_check(n, actor, critic, obs, a_min, a_max, std_, std_vec, action, value);
     if (rc) return rc;
+    PolicyRoute r;
+    if ((rc = policy_route(actor, critic, &r))) return rc;
+    unsigned char *image;
+    float *bias;
+    if ((rc = policy_workspace_split(r.p, const_cast<void *>(workspace), workspace_bytes, &image, &bias))) return rc;
     PolicyIO io = {};
     io.obs = obs; io.a_min = a_min; io.a_max = a_max; io.noise = noise; io.std_ = std_vec ? 1.0f : std_;
     io.std_vec = std_vec;
     io.out_affine = actor && actor->out_act == 2;
     io.seed = seed; io.step = step; io.off = env_index_offset;
     io.action = action; io.log_prob = log_prob; io.mean = mean; io.value = value;
-    return policy_launch_umma(n, actor, critic, workspace, workspace_bytes, io, (cudaStream_t)cuda_stream);
+    return r.launch(n, r.p, io, image, bias, (cudaStream_t)cuda_stream);
 }
 
 extern "C" B200_API int b200_umma_probe(const float *A, const float *W, float *D, int N, int K, int three_pass,

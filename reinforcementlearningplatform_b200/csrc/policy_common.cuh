@@ -1,6 +1,7 @@
 // policy_common.cuh -- pieces shared by the K-POLICY kernels (policy.cu: FP32 FMA pipe; policy_umma.cu and
 // policy_umma16.cu: tcgen05 tensor cores).
 #pragma once
+#include <cuda_fp16.h>
 #include "common.cuh"
 
 struct PolicyIO {
@@ -17,19 +18,86 @@ struct PolicyIO {
 };
 
 int policy_launch_fp32(int64_t n, const b200_mlp *actor, const b200_mlp *critic, const PolicyIO &io, cudaStream_t s);
-// policy_umma.cu (tcgen05 / TMEM): weights pre-packed into a caller-owned workspace
-size_t policy_umma_workspace_bytes(const b200_mlp *actor, const b200_mlp *critic);
-int policy_umma_pack(const b200_mlp *actor, const b200_mlp *critic, void *workspace, size_t bytes, cudaStream_t s);
-int policy_launch_umma(int64_t n, const b200_mlp *actor, const b200_mlp *critic, const void *workspace, size_t bytes,
-                       const PolicyIO &io, cudaStream_t s);
 int policy_umma_probe(const float *A, const float *W, float *D, int N, int K, int three_pass, cudaStream_t s);
-// policy_umma16.cu (tcgen05 / TMEM, fp16-split operands, four tiles in flight): the nets it holds (layers <= 64 wide,
-// <= 32 observation fields) are routed to it by the three policy_umma_* entry points above
-bool policy_umma16_fits(const b200_mlp *actor, const b200_mlp *critic);
-size_t policy_umma16_workspace_bytes(const b200_mlp *actor, const b200_mlp *critic);
-int policy_umma16_pack(const b200_mlp *actor, const b200_mlp *critic, void *workspace, size_t bytes, cudaStream_t s);
-int policy_launch_umma16(int64_t n, const b200_mlp *actor, const b200_mlp *critic, const void *workspace, size_t bytes,
-                         const PolicyIO &io, cudaStream_t s);
+
+// ------------------------------------------------------------------------------------------------ tcgen05 routes
+// The two tcgen05 kernels (policy_umma16.cu for nets <= 64 wide with <= 32 observation fields, policy_umma.cu for the
+// rest) read the same layer records, and their weights are packed by one kernel into a caller-owned workspace.
+constexpr int POLICY_MAX_LAYERS = 8;
+
+struct PolicyLayer {
+    int K, N;        // padded: first layer K to a multiple of 8, others K = previous N; N to a multiple of 16
+    int n_real;      // nn.Linear out features
+    int role;        // 0 hidden (tanh), 1 actor output, 2 critic output
+    int first;       // input = observations: 3xTF32 operand pairs, k-steps of 8
+    int f16;         // operands as fp16 hi / lo pairs, weights pre-scaled by a power of two: k-steps of 16, half the
+                     // image bytes and half the MMAs of the 3xTF32 form
+    int out_act;     // output layers: 0 identity, 1 relu (2, the range map, is applied in policy_sample_store)
+    uint32_t w_off;  // byte offset of the layer's image: k-step kk at w_off + kk * N * 64 (hi plane N * 32 B, then lo)
+    int b_off;       // float offset of the layer's bias (tanh layers: pre-multiplied by 2 log2 e)
+};
+
+struct PolicyPlan {
+    int n_layers, S, A;
+    // policy_umma.cu's operating mode (build_plan); policy_umma16.cu has a single one and leaves these 0
+    int slots, nbuf_log2, streamed;
+    int a_tmem;      // 1: activations (A operand) live in TMEM and the MMAs are issued in the TS form; 0: shared memory (SS)
+    int tmem_cols, slot_cols, pong_off, a_col;   // per slot: D ping at +0, D pong at +pong_off, A hi plane at +a_col,
+                                                 // A lo plane at +a_col + 32 * nbuf (a_tmem only)
+    uint32_t img_bytes;
+    int bias_floats, zs_off;   // zs_off: per-layer accumulator scale (x 2 log2 e for tanh layers) inside the bias array
+    uint32_t stage_bytes;
+    uint32_t off_a, off_b, off_bias, off_scr, smem_bytes;  // dynamic shared memory map (after the barrier block)
+    PolicyLayer L[POLICY_MAX_LAYERS];
+};
+
+// The kernel a net pair runs on, with its plan, and the nn.Linear weight / bias / in-features of every layer (for the
+// packer; the actor's and the critic's input widths may differ, and only b200_policy_forward_packed rejects that)
+struct PolicyRoute {
+    PolicyPlan p;
+    const float *w[POLICY_MAX_LAYERS], *b[POLICY_MAX_LAYERS];
+    int k_real[POLICY_MAX_LAYERS];
+    int (*launch)(int64_t n, const PolicyPlan &p, const PolicyIO &io, const unsigned char *image, const float *bias,
+                  cudaStream_t s);
+};
+
+// Appends the layers of both nets to P->L and r->w / r->b / r->k_real, with their image and bias offsets: K padded to 8 on a net's
+// first layer, N to 16.  The limits are the route's: layer width, first-layer input, and whether the layers after a
+// net's first multiply fp16 pairs.  B200ENV_ESIZE for a net it does not hold.
+int policy_add_nets(const b200_mlp *actor, const b200_mlp *critic, int max_width, int max_first_in, bool f16_hidden,
+                    PolicyRoute *r);
+// policy_umma16.cu's plan and launch when the pair fits it, else B200ENV_ESIZE
+int policy_umma16_route(const b200_mlp *actor, const b200_mlp *critic, PolicyRoute *r);
+// policy_umma16.cu when the pair fits it, else policy_umma.cu
+int policy_route(const b200_mlp *actor, const b200_mlp *critic, PolicyRoute *r);
+// weights and biases -> the workspace of the route, on the stream
+int policy_pack(const PolicyRoute &r, void *workspace, size_t bytes, cudaStream_t s);
+
+// The workspace of a plan: the weight image (rounded up to 128 bytes), then the bias floats
+inline size_t policy_workspace_bytes(const PolicyPlan &p) {
+    return ((size_t)p.img_bytes + 127) / 128 * 128 + (size_t)p.bias_floats * 4;
+}
+// a caller's workspace -> (image, bias); it must be 128-byte aligned and policy_workspace_bytes long
+inline int policy_workspace_split(const PolicyPlan &p, void *workspace, size_t bytes, unsigned char **image, float **bias) {
+    if (!workspace) return B200ENV_ENULL;
+    if (bytes < policy_workspace_bytes(p) || ((uintptr_t)workspace & 127)) return B200ENV_EPARAMS;
+    *image = static_cast<unsigned char *>(workspace);
+    *bias = reinterpret_cast<float *>(*image + ((size_t)p.img_bytes + 127) / 128 * 128);
+    return B200ENV_OK;
+}
+
+// eight values -> fp16 hi / lo pairs, hi = fp16(y), lo = fp16(y - hi) (22 significand bits, as a TF32 pair), two per
+// word: the low half (.x) holds the even index
+__device__ __forceinline__ void policy_split_f16x8(const float *y, uint32_t *hi, uint32_t *lo) {
+#pragma unroll
+    for (int p = 0; p < 4; ++p) {
+        const __half2 h = __floats2half2_rn(y[2 * p], y[2 * p + 1]);
+        const float2 f = __half22float2(h);
+        const __half2 l = __floats2half2_rn(y[2 * p] - f.x, y[2 * p + 1] - f.y);
+        hi[p] = *reinterpret_cast<const uint32_t *>(&h);
+        lo[p] = *reinterpret_cast<const uint32_t *>(&l);
+    }
+}
 
 // Philox key domain of the exploration noise.  The env resets draw from Philox(seed, instance, episode) (common.cuh); with
 // equal seeds the reset of (instance i, episode e) and the noise of (instance i, step e) would consume the same 128-bit

@@ -40,7 +40,6 @@
 // of a core matrix 16 B apart, core matrices 128 B apart along M/N (SBO) and one "slab" (rows x 16 B) apart along K
 // (LBO): element (row, k) of an operand with R rows lives at (k / 4) * R * 16 + row * 16 + (k % 4) * 4.  With thread =
 // row the epilogue's 16-byte stores of a warp are 512 contiguous bytes: conflict-free without swizzling.
-#include <cuda_fp16.h>
 #include "policy_common.cuh"
 #include "umma_ptx.cuh"
 
@@ -54,38 +53,12 @@ constexpr int CHUNK_K = 32;                            // activation chunk: 32 c
 constexpr uint32_t SLAB = TILE_M * 16;                 // bytes of one 4-column K slab of the A operand
 constexpr uint32_t PLANE = (CHUNK_K / 4) * SLAB;       // 16 KB: hi (or lo) plane of a chunk
 constexpr uint32_t CHUNK = 2 * PLANE;                  // 32 KB: hi + lo
-constexpr int UM_MAX_LAYERS = 8;
 constexpr int NSTAGE = 4;                              // weight ring (streamed mode)
 constexpr uint32_t SMEM_LIMIT = 227 * 1024;
 constexpr float TWO_LOG2E = 2.885390081777927f;        // tanh(x) = 1 - 2 / (2^(x * 2 log2 e) + 1)
 
-struct ULayer {
-    int K, N;        // padded: K to a multiple of 8, N to a multiple of 16
-    int n_real;
-    int role;        // 0 hidden (tanh), 1 actor output, 2 critic output
-    int first;       // input = observations
-    int out_act;     // output layers: 0 identity, 1 relu
-    uint32_t w_off;  // byte offset of the layer's image: k-step kk at w_off + kk * N * 64 (hi plane N * 32 B, then lo)
-    int b_off;       // float offset of the layer's bias (tanh layers: pre-multiplied by 2 log2 e)
-    int f16;         // operands as fp16 hi / lo pairs, weights pre-scaled by a power of two (streamed mode, layers after the
-                     // first): k-steps of 16, half the image bytes and half the MMAs of the 3xTF32 form (policy_umma16.cu)
-};
-
-struct UPlan {
-    int n_layers, S, A;
-    int slots, nbuf_log2, streamed;
-    int a_tmem;      // 1: activations (A operand) live in TMEM and the MMAs are issued in the TS form; 0: shared memory (SS)
-    int tmem_cols, slot_cols, pong_off, a_col;   // per slot: D ping at +0, D pong at +pong_off, A hi plane at +a_col,
-                                                 // A lo plane at +a_col + 32 * nbuf (a_tmem only)
-    uint32_t img_bytes;
-    int bias_floats, zs_off;   // zs_off: per-layer accumulator scale (x 2 log2 e for tanh layers) inside the bias array
-    uint32_t stage_bytes;
-    uint32_t off_a, off_b, off_bias, off_scr, smem_bytes;  // dynamic shared memory map (after the barrier block)
-    ULayer L[UM_MAX_LAYERS];
-};
-
 struct UArgs {
-    UPlan p;
+    PolicyPlan p;
     PolicyIO io;
     const unsigned char *image;  // packed weights (global)
     const float *bias;           // packed biases (global)
@@ -139,14 +112,7 @@ __device__ __forceinline__ void store_split4(unsigned char *chunk, int q, int r,
 // eight activations of row r -> fp16 hi / lo pairs -> one 16-byte store into each plane of fp16 slab q8 (8 K columns)
 __device__ __forceinline__ void store_split8(unsigned char *chunk, int q8, int r, const float *y) {
     uint32_t hi[4], lo[4];
-#pragma unroll
-    for (int p = 0; p < 4; ++p) {
-        const __half2 h = __floats2half2_rn(y[2 * p], y[2 * p + 1]);
-        const float2 f = __half22float2(h);
-        const __half2 l = __floats2half2_rn(y[2 * p] - f.x, y[2 * p + 1] - f.y);
-        hi[p] = *reinterpret_cast<const uint32_t *>(&h);
-        lo[p] = *reinterpret_cast<const uint32_t *>(&l);
-    }
+    policy_split_f16x8(y, hi, lo);
     unsigned char *p = chunk + (uint32_t)q8 * SLAB + (uint32_t)r * 16;
     *reinterpret_cast<uint4 *>(p) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
     *reinterpret_cast<uint4 *>(p + PLANE) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
@@ -243,7 +209,7 @@ struct BarMap {                       // byte offsets inside the barrier block a
 // 128 x N x 8 MMA per ~41 cycles whatever N <= 64 -- a limit of that thread's instruction stream, not of the tensor pipe:
 // two issuing warps reach one per ~28 cycles.
 template <bool STREAMED, bool A_TMEM>
-__device__ __forceinline__ void mma_issue_loop(const UPlan &P, uint32_t s, uint32_t sbase, uint32_t tmem_base,
+__device__ __forceinline__ void mma_issue_loop(const PolicyPlan &P, uint32_t s, uint32_t sbase, uint32_t tmem_base,
                                                int64_t groups, int64_t tiles) {
     const uint32_t nbuf_log2 = (uint32_t)P.nbuf_log2, nbuf_mask = (1u << nbuf_log2) - 1u;
     const int n_layers = P.n_layers, slots = P.slots;
@@ -327,7 +293,7 @@ __device__ __forceinline__ void mma_issue_loop(const UPlan &P, uint32_t s, uint3
 template <bool A_TMEM>
 __device__ __forceinline__ void epilogue_loop(const UArgs &a, int64_t n, unsigned char *smem, uint32_t sbase,
                                               uint32_t tmem_base, int warp, int64_t tiles, int64_t groups) {
-    const UPlan &P = a.p;
+    const PolicyPlan &P = a.p;
     const int s = warp >> 3, h = (warp >> 2) & 1;
     const int nbuf = 1 << P.nbuf_log2, nbuf_mask = nbuf - 1;
     const float *bias_s = reinterpret_cast<const float *>(smem + P.off_bias);
@@ -351,7 +317,7 @@ __device__ __forceinline__ void epilogue_loop(const UArgs &a, int64_t n, unsigne
         const bool live = i < n;
         int pending_A = 0;     // > 0: this row's means sit in scr and still have to be sampled (half-group 0 only)
         for (int li = 0; li < P.n_layers; ++li) {
-            const ULayer &L = P.L[li];
+            const PolicyLayer &L = P.L[li];
             if (L.first) {                       // the layer's input is the observation: K columns, zero-padded
                 for (int k0 = 0; k0 < L.K; k0 += CHUNK_K) {
                     const int buf = g & nbuf_mask;
@@ -458,7 +424,7 @@ __device__ __forceinline__ void epilogue_loop(const UArgs &a, int64_t n, unsigne
 __global__ void __launch_bounds__(UM_THREADS, 1)
 policy_umma_kernel(const __grid_constant__ UArgs a, int64_t n) {
     extern __shared__ __align__(128) unsigned char smem[];
-    const UPlan &P = a.p;
+    const PolicyPlan &P = a.p;
     const uint32_t sbase = smem_u32(smem);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     float *bias_s = reinterpret_cast<float *>(smem + P.off_bias);
@@ -519,7 +485,7 @@ policy_umma_kernel(const __grid_constant__ UArgs a, int64_t n) {
                 uint32_t h = 0;
                 for (int64_t grp = blockIdx.x; grp < groups; grp += gridDim.x) {
                     for (int li = 0; li < P.n_layers; ++li) {
-                        const ULayer &L = P.L[li];
+                        const PolicyLayer &L = P.L[li];
                         const uint32_t kstep_bytes = (uint32_t)L.N * 64;
                         for (int kk = 0; kk < L.K / (L.f16 ? 16 : 8); ++kk, ++h) {
                             const int stage = h & (NSTAGE - 1);
@@ -542,28 +508,28 @@ policy_umma_kernel(const __grid_constant__ UArgs a, int64_t n) {
 
 // ------------------------------------------------------------------------------------------------ weight packing
 struct PackArgs {
-    int n_layers;
-    ULayer L[UM_MAX_LAYERS];
-    int k_real[UM_MAX_LAYERS];
-    const float *w[UM_MAX_LAYERS];
-    const float *b[UM_MAX_LAYERS];
+    PolicyPlan p;
+    const float *w[POLICY_MAX_LAYERS];
+    const float *b[POLICY_MAX_LAYERS];
+    int k_real[POLICY_MAX_LAYERS];   // nn.Linear in features
     unsigned char *image;
     float *bias;
-    int zs_off;
 };
 
 // nn.Linear weights [n_real][k_real] -> the UMMA image, zero-padded, and the bias vector (tanh layers: times 2 log2 e).
 // TF32 layers: per k-step of 8 a hi and a lo plane, element (n, k) of a plane at (k % 8 / 4) * N * 16 + n * 16 + (k % 4) * 4.
 // fp16 layers (L.f16): weights times 2^s, s chosen per layer so that max |w| 2^s lies in [2^13, 2^14); per k-step of 16 a hi
 // and a lo plane of fp16, element (n, k) at (k % 16 / 8) * N * 16 + n * 16 + (k % 8) * 2.  zs[l] = 2^-s (x 2 log2 e for tanh
-// layers) is what the epilogue multiplies the accumulator by.
+// layers) is what the epilogue multiplies the accumulator by.  Every block computes its layer's max |w| over all elements
+// itself, so the image does not depend on the grid.
 __global__ void __launch_bounds__(256) policy_pack_kernel(const __grid_constant__ PackArgs a) {
     __shared__ float s_max[8];
     __shared__ int s_exp;
     const int li = blockIdx.y;
-    if (li >= a.n_layers) return;
-    const ULayer &L = a.L[li];
-    const int total = L.K * L.N, real = a.k_real[li] * L.n_real;
+    if (li >= a.p.n_layers) return;
+    const PolicyLayer &L = a.p.L[li];
+    const int k_real = a.k_real[li];
+    const int total = L.K * L.N, real = k_real * L.n_real;
     int sexp = 0;
     if (L.f16) {
         float m = 0.0f;
@@ -585,7 +551,7 @@ __global__ void __launch_bounds__(256) policy_pack_kernel(const __grid_constant_
     const float scale = ldexpf(1.0f, sexp);
     for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < total; e += gridDim.x * blockDim.x) {
         const int k = e / L.N, nn = e - k * L.N;
-        const float w = (nn < L.n_real && k < a.k_real[li]) ? __ldg(a.w[li] + (int64_t)nn * a.k_real[li] + k) : 0.0f;
+        const float w = (nn < L.n_real && k < k_real) ? __ldg(a.w[li] + (int64_t)nn * k_real + k) : 0.0f;
         if (L.f16) {
             const float ws = w * scale;
             const __half hi = __float2half_rn(ws);
@@ -608,47 +574,57 @@ __global__ void __launch_bounds__(256) policy_pack_kernel(const __grid_constant_
             const float b = j < L.n_real ? __ldg(a.b[li] + j) : 0.0f;
             a.bias[L.b_off + j] = L.role == 0 ? b * TWO_LOG2E : b;
         }
-        if (threadIdx.x == 0) a.bias[a.zs_off + li] = (L.role == 0 ? TWO_LOG2E : 1.0f) * ldexpf(1.0f, -sexp);
+        if (threadIdx.x == 0) a.bias[a.p.zs_off + li] = (L.role == 0 ? TWO_LOG2E : 1.0f) * ldexpf(1.0f, -sexp);
     }
 }
 
 // ------------------------------------------------------------------------------------------------ host side
-int add_net(const b200_mlp *m, bool is_actor, UPlan *P, int *k_real, const float **w, const float **b) {
+int add_net(const b200_mlp *m, bool is_actor, int max_width, int max_first_in, bool f16_hidden, PolicyRoute *r) {
+    PolicyPlan *P = &r->p;
     if (m->n_layers < 1 || m->n_layers > 4) return B200ENV_ESIZE;
     for (int l = 0; l < m->n_layers; ++l) {
-        if (P->n_layers >= UM_MAX_LAYERS) return B200ENV_ESIZE;
+        if (P->n_layers >= POLICY_MAX_LAYERS) return B200ENV_ESIZE;
         const int in = m->dims[l], out = m->dims[l + 1];
-        if (in < 1 || out < 1 || in > 256 || out > 256) return B200ENV_ESIZE;   // UMMA N <= 256; K chunks <= 8 per layer
-        ULayer &L = P->L[P->n_layers];
         const bool last = l + 1 == m->n_layers;
-        if (last && out > 16) return B200ENV_ESIZE;                              // output heads: <= 16 actions / 1 value
+        // hidden inputs are the previous layer's outputs; output heads: <= 16 actions / 1 value
+        if (in < 1 || out < 1 || out > max_width || (l == 0 && in > max_first_in) || (last && out > 16)) return B200ENV_ESIZE;
+        PolicyLayer &L = P->L[P->n_layers];
         L.first = l == 0;
+        L.f16 = f16_hidden && l > 0;
         L.K = l == 0 ? (in + 7) / 8 * 8 : P->L[P->n_layers - 1].N;               // hidden input = previous padded width
         L.N = (out + 15) / 16 * 16;
         L.n_real = out;
         L.role = last ? (is_actor ? 1 : 2) : 0;
         L.out_act = m->out_act == 2 ? 0 : m->out_act;                            // 2: range map in policy_sample_store
         L.w_off = P->img_bytes;
-        P->img_bytes += (uint32_t)L.K * (uint32_t)L.N * 8;
+        P->img_bytes += (uint32_t)L.K * (uint32_t)L.N * (L.f16 ? 4u : 8u);
         L.b_off = P->bias_floats;
         P->bias_floats += L.N;
-        if (k_real) k_real[P->n_layers] = in;
-        if (w) w[P->n_layers] = m->w[l];
-        if (b) b[P->n_layers] = m->b[l];
+        r->w[P->n_layers] = m->w[l];
+        r->k_real[P->n_layers] = in;
+        r->b[P->n_layers] = m->b[l];
         ++P->n_layers;
     }
     return B200ENV_OK;
 }
 
-int build_plan(const b200_mlp *actor, const b200_mlp *critic, UPlan *P, int *k_real, const float **w, const float **b) {
-    *P = UPlan{};
-    int rc;
-    if (actor && (rc = add_net(actor, true, P, k_real, w, b))) return rc;
-    if (critic && (rc = add_net(critic, false, P, k_real, w, b))) return rc;
-    P->S = actor ? actor->dims[0] : critic->dims[0];
-    P->A = actor ? actor->dims[actor->n_layers] : 0;
-    P->zs_off = P->bias_floats;
-    P->bias_floats += UM_MAX_LAYERS;
+int launch(int64_t n, const PolicyPlan &p, const PolicyIO &io, const unsigned char *image, const float *bias,
+           cudaStream_t stream) {
+    static size_t configured[64] = {0};
+    const int rc = b200_opt_in_smem(policy_umma_kernel, p.smem_bytes, configured);
+    if (rc) return rc;
+    const int64_t tiles = (n + TILE_M - 1) / TILE_M, groups = (tiles + p.slots - 1) / p.slots, cap = b200_sm_count();
+    const UArgs a = {p, io, image, bias};
+    policy_umma_kernel<<<(unsigned)(groups < cap ? groups : cap), UM_THREADS, p.smem_bytes, stream>>>(a, n);
+    return b200_check_launch();
+}
+
+// this file's plan: the first of build_plan's candidates that fits
+int build_plan(const b200_mlp *actor, const b200_mlp *critic, PolicyRoute *r) {
+    int rc = policy_add_nets(actor, critic, 256, 256, false, r);   // UMMA N <= 256; K chunks <= 8 per layer
+    if (rc) return rc;
+    PolicyPlan *P = &r->p;
+    r->launch = launch;
     int nmax = 16, kmax = 8;
     for (int l = 0; l < P->n_layers; ++l) {
         nmax = P->L[l].N > nmax ? P->L[l].N : nmax;
@@ -676,7 +652,7 @@ int build_plan(const b200_mlp *actor, const b200_mlp *critic, UPlan *P, int *k_r
             // ring per tile and half the MMAs (kind::f16 covers K = 16); the image offsets are laid out again
             uint32_t off = 0;
             for (int l = 0; l < P->n_layers; ++l) {
-                ULayer &L = P->L[l];
+                PolicyLayer &L = P->L[l];
                 L.f16 = !L.first;
                 L.w_off = off;
                 off += (uint32_t)L.K * (uint32_t)L.N * (L.f16 ? 4u : 8u);
@@ -696,58 +672,37 @@ int build_plan(const b200_mlp *actor, const b200_mlp *critic, UPlan *P, int *k_r
 
 } // namespace
 
-size_t policy_umma_workspace_bytes(const b200_mlp *actor, const b200_mlp *critic) {
-    if (policy_umma16_fits(actor, critic)) return policy_umma16_workspace_bytes(actor, critic);
-    UPlan P;
-    if (build_plan(actor, critic, &P, nullptr, nullptr, nullptr)) return 0;
-    return (size_t)(P.img_bytes + 127) / 128 * 128 + (size_t)P.bias_floats * 4;
+int policy_add_nets(const b200_mlp *actor, const b200_mlp *critic, int max_width, int max_first_in, bool f16_hidden,
+                    PolicyRoute *r) {
+    *r = PolicyRoute{};
+    PolicyPlan *P = &r->p;
+    int rc;
+    if (actor && (rc = add_net(actor, true, max_width, max_first_in, f16_hidden, r))) return rc;
+    if (critic && (rc = add_net(critic, false, max_width, max_first_in, f16_hidden, r))) return rc;
+    P->S = actor ? actor->dims[0] : critic->dims[0];
+    P->A = actor ? actor->dims[actor->n_layers] : 0;
+    P->zs_off = P->bias_floats;
+    P->bias_floats += POLICY_MAX_LAYERS;
+    return B200ENV_OK;
 }
 
-int policy_umma_pack(const b200_mlp *actor, const b200_mlp *critic, void *workspace, size_t bytes, cudaStream_t stream) {
-    if (policy_umma16_fits(actor, critic)) return policy_umma16_pack(actor, critic, workspace, bytes, stream);
+int policy_route(const b200_mlp *actor, const b200_mlp *critic, PolicyRoute *r) {
+    if (policy_umma16_route(actor, critic, r) == B200ENV_OK) return B200ENV_OK;
+    return build_plan(actor, critic, r);
+}
+
+int policy_pack(const PolicyRoute &r, void *workspace, size_t bytes, cudaStream_t stream) {
     PackArgs pa = {};
-    UPlan P;
-    int rc = build_plan(actor, critic, &P, pa.k_real, pa.w, pa.b);
-    if (rc) return rc;
-    for (int l = 0; l < P.n_layers; ++l)
-        if (!pa.w[l] || !pa.b[l]) return B200ENV_ENULL;
-    const size_t img = (size_t)(P.img_bytes + 127) / 128 * 128;
-    if (!workspace) return B200ENV_ENULL;
-    if (bytes < img + (size_t)P.bias_floats * 4 || ((uintptr_t)workspace & 127)) return B200ENV_EPARAMS;
-    pa.n_layers = P.n_layers;
-    pa.zs_off = P.zs_off;
-    for (int l = 0; l < P.n_layers; ++l) pa.L[l] = P.L[l];
-    pa.image = static_cast<unsigned char *>(workspace);
-    pa.bias = reinterpret_cast<float *>(pa.image + img);
-    policy_pack_kernel<<<dim3(32, P.n_layers), 256, 0, stream>>>(pa);
-    return b200_check_launch();
-}
-
-int policy_launch_umma(int64_t n, const b200_mlp *actor, const b200_mlp *critic, const void *workspace, size_t bytes,
-                       const PolicyIO &io, cudaStream_t stream) {
-    if (policy_umma16_fits(actor, critic)) return policy_launch_umma16(n, actor, critic, workspace, bytes, io, stream);
-    UArgs a = {};
-    int rc = build_plan(actor, critic, &a.p, nullptr, nullptr, nullptr);
-    if (rc) return rc;
-    const size_t img = (size_t)(a.p.img_bytes + 127) / 128 * 128;
-    if (!workspace) return B200ENV_ENULL;
-    if (bytes < img + (size_t)a.p.bias_floats * 4 || ((uintptr_t)workspace & 127)) return B200ENV_EPARAMS;
-    a.image = static_cast<const unsigned char *>(workspace);
-    a.bias = reinterpret_cast<const float *>(a.image + img);
-    a.io = io;
-    static size_t configured[64] = {0};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64) dev = 0;
-    if (a.p.smem_bytes > configured[dev]) {
-        if (cudaFuncSetAttribute(policy_umma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_LIMIT) != cudaSuccess)
-            return b200_check_launch();
-        configured[dev] = SMEM_LIMIT;
+    for (int l = 0; l < r.p.n_layers; ++l) {
+        if (!r.w[l] || !r.b[l]) return B200ENV_ENULL;
+        pa.w[l] = r.w[l];
+        pa.b[l] = r.b[l];
+        pa.k_real[l] = r.k_real[l];
     }
-    const int64_t tiles = (n + TILE_M - 1) / TILE_M, groups = (tiles + a.p.slots - 1) / a.p.slots;
-    const unsigned cap = b200_persistent_grid(n, 1, 1);      // = number of SMs for any n >= that many
-    const unsigned grid = (unsigned)(groups < (int64_t)cap ? groups : (int64_t)cap);
-    policy_umma_kernel<<<grid, UM_THREADS, a.p.smem_bytes, stream>>>(a, n);
+    const int rc = policy_workspace_split(r.p, workspace, bytes, &pa.image, &pa.bias);
+    if (rc) return rc;
+    pa.p = r.p;
+    policy_pack_kernel<<<dim3(32, r.p.n_layers), 256, 0, stream>>>(pa);
     return b200_check_launch();
 }
 

@@ -25,7 +25,6 @@
 // a_full (128 arrivals: the layer's input is in TMEM and the previous accumulator has been read) and d_ready
 // (tcgen05.commit).
 // Nets this kernel does not hold (a layer wider than 64, more than 32 observation fields) take policy_umma.cu.
-#include <cuda_fp16.h>
 #include "policy_common.cuh"
 #include "umma_ptx.cuh"
 
@@ -35,34 +34,16 @@ using namespace umma;
 constexpr int H_THREADS = 640;
 constexpr int H_SLOTS = 4, H_EPI_WARPS = 16;
 constexpr int H_TILE = 128;
-constexpr int H_MAX_LAYERS = 8;
 constexpr uint32_t H_SLOT_COLS = 128, H_A_COL = 64, H_A_LO = 32;
-constexpr float H_TWO_LOG2E = 2.885390081777927f;
 constexpr uint32_t H_SMEM_LIMIT = 227 * 1024;
 
-struct HLayer {
-    int K, N;        // padded: first layer K to a multiple of 8 (TF32), others K = previous N; N to a multiple of 16
-    int n_real, k_real;
-    int role;        // 0 hidden (tanh), 1 actor output, 2 critic output
-    int first;       // input = observations (3xTF32); else fp16-split
-    int out_act;
-    uint32_t w_off;  // byte offset of the layer's image; k-step kk at w_off + kk * N * 64 (hi plane N * 32 B, then lo)
-    int b_off;
-};
-
-struct HPlan {
-    int n_layers, S, A;
-    uint32_t img_bytes;
-    int bias_floats, zs_off;   // zs_off: per-layer accumulator scale (x 2 log2 e for tanh layers) inside the bias array
-    uint32_t off_b, off_bias, off_scr, smem_bytes;
-    HLayer L[H_MAX_LAYERS];
-};
-
+// io sits after image: ptxas pairs the loads of io's pointers by their 16-byte alignment in the parameter block, and
+// this order keeps the alignment (and so the instructions) this kernel was measured with
 struct HArgs {
-    HPlan p;
+    PolicyPlan p;
+    const unsigned char *image;  // packed weights (global)
     PolicyIO io;
-    const unsigned char *image;
-    const float *bias;
+    const float *bias;           // packed biases (global)
 };
 
 struct HBar {
@@ -105,14 +86,8 @@ __device__ __forceinline__ void epi16_compute(const uint32_t (&v)[16], const flo
 #pragma unroll
     for (int j = 0; j < 16; ++j) t[j] = fmaf(-2.0f, t[j], 1.0f);
     uint32_t hi[8], lo[8];
-#pragma unroll
-    for (int p = 0; p < 8; ++p) {
-        const __half2 h = __floats2half2_rn(t[2 * p], t[2 * p + 1]);          // .x (low half) = even k
-        const float2 f = __half22float2(h);
-        const __half2 l = __floats2half2_rn(t[2 * p] - f.x, t[2 * p + 1] - f.y);
-        hi[p] = *reinterpret_cast<const uint32_t *>(&h);
-        lo[p] = *reinterpret_cast<const uint32_t *>(&l);
-    }
+    policy_split_f16x8(t, hi, lo);
+    policy_split_f16x8(t + 8, hi + 4, lo + 4);
     tmem_st8(a_hi_addr, hi);
     tmem_st8(a_lo_addr, lo);
 }
@@ -133,7 +108,7 @@ __device__ __forceinline__ void epi_hidden(uint32_t slot_t, const float *bias_sc
 __global__ void __launch_bounds__(H_THREADS, 1)
 policy_umma16_kernel(const __grid_constant__ HArgs a, int64_t n) {
     extern __shared__ __align__(128) unsigned char smem[];
-    const HPlan &P = a.p;
+    const PolicyPlan &P = a.p;
     const uint32_t sbase = smem_u32(smem);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     float *bias_s = reinterpret_cast<float *>(smem + P.off_bias);
@@ -189,7 +164,7 @@ policy_umma16_kernel(const __grid_constant__ HArgs a, int64_t n) {
 #pragma unroll
             for (int e = 0; e < 8; ++e) x8[e] = (live && e < P.S) ? __ldg(a.io.obs + (int64_t)e * n + i) : 0.0f;
             for (int li = 0; li < P.n_layers; ++li) {
-                const HLayer &L = P.L[li];
+                const PolicyLayer &L = P.L[li];
                 if (L.first) {
                     // observations -> TF32 hi / lo planes of the A region (zero-padded to K)
                     for (int q = 0; q < L.K / 8; ++q) {
@@ -270,7 +245,7 @@ policy_umma16_kernel(const __grid_constant__ HArgs a, int64_t n) {
             for (int64_t grp = blockIdx.x; grp < groups; grp += gridDim.x) {
                 if (grp * H_SLOTS + (int64_t)s >= tiles) break;
                 for (int li = 0; li < P.n_layers; ++li) {
-                    const HLayer &L = P.L[li];
+                    const PolicyLayer &L = P.L[li];
                     const uint32_t N = (uint32_t)L.N;
                     const uint32_t blo16 = N * 2, kstep16 = N * 4;                // N * 32 B and N * 64 B, >> 4
                     uint32_t b_hi = (b_base16 + (L.w_off >> 4)) | (N << 16);      // LBO = N * 16 B
@@ -306,112 +281,25 @@ policy_umma16_kernel(const __grid_constant__ HArgs a, int64_t n) {
     if (warp == H_EPI_WARPS) tmem_dealloc(tmem_base, 512);
 }
 
-// ------------------------------------------------------------------------------------------------ weight packing
-struct HPackArgs {
-    int n_layers, zs_off;
-    HLayer L[H_MAX_LAYERS];
-    const float *w[H_MAX_LAYERS];
-    const float *b[H_MAX_LAYERS];
-    unsigned char *image;
-    float *bias;
-};
-
-// nn.Linear weights [n_real][k_real] -> the operand image.  First layers: TF32 hi / lo planes, per k-step of 8: element
-// (n, k) at (k % 8 / 4) * N * 16 + n * 16 + (k % 4) * 4.  Other layers: weights times 2^s (s chosen per layer so that
-// max |w| 2^s lies in [2^13, 2^14)), fp16 hi / lo planes, per k-step of 16: element (n, k) at (k % 16 / 8) * N * 16 +
-// n * 16 + (k % 8) * 2.  Bias vector: tanh layers times 2 log2 e; zs[l] = 2^-s (times 2 log2 e for tanh layers).
-__global__ void __launch_bounds__(256) policy_pack16_kernel(const __grid_constant__ HPackArgs a) {
-    __shared__ float s_max[8];
-    __shared__ int s_exp;
-    const int li = blockIdx.y;
-    if (li >= a.n_layers) return;
-    const HLayer &L = a.L[li];
-    const int total = L.K * L.N, real = L.k_real * L.n_real;
-    int sexp = 0;
-    if (!L.first) {
-        float m = 0.0f;
-        for (int e = threadIdx.x; e < real; e += blockDim.x) m = fmaxf(m, fabsf(__ldg(a.w[li] + e)));
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
-        if ((threadIdx.x & 31) == 0) s_max[threadIdx.x >> 5] = m;
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            for (int w = 1; w < 8; ++w) m = fmaxf(m, s_max[w]);
-            int e = 0;
-            if (m > 0.0f && m < 3.0e38f) frexpf(m, &e);      // m = f 2^e, f in [0.5, 1)
-            else e = 14;
-            int sx = 14 - e;
-            sx = sx > 100 ? 100 : (sx < -100 ? -100 : sx);
-            s_exp = sx;
-        }
-        __syncthreads();
-        sexp = s_exp;
-    }
-    const float scale = ldexpf(1.0f, sexp);
-    for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < total; e += gridDim.x * blockDim.x) {
-        const int k = e / L.N, nn = e - k * L.N;
-        const float w = (nn < L.n_real && k < L.k_real) ? __ldg(a.w[li] + (int64_t)nn * L.k_real + k) : 0.0f;
-        if (L.first) {
-            const uint32_t hi = tf32_hi(w);
-            unsigned char *ks = a.image + L.w_off + (uint32_t)(k / 8) * (uint32_t)L.N * 64;
-            const uint32_t in_plane = (uint32_t)((k & 7) >> 2) * (uint32_t)L.N * 16 + (uint32_t)nn * 16 + (uint32_t)(k & 3) * 4;
-            *reinterpret_cast<uint32_t *>(ks + in_plane) = hi;
-            *reinterpret_cast<float *>(ks + (uint32_t)L.N * 32 + in_plane) = w - __uint_as_float(hi);
-        } else {
-            const float ws = w * scale;
-            const __half hi = __float2half_rn(ws);
-            const __half lo = __float2half_rn(ws - __half2float(hi));
-            unsigned char *ks = a.image + L.w_off + (uint32_t)(k / 16) * (uint32_t)L.N * 64;
-            const uint32_t in_plane = (uint32_t)((k & 15) >> 3) * (uint32_t)L.N * 16 + (uint32_t)nn * 16 + (uint32_t)(k & 7) * 2;
-            *reinterpret_cast<__half *>(ks + in_plane) = hi;
-            *reinterpret_cast<__half *>(ks + (uint32_t)L.N * 32 + in_plane) = lo;
-        }
-    }
-    if (blockIdx.x == 0) {
-        for (int j = threadIdx.x; j < L.N; j += blockDim.x) {
-            const float b = j < L.n_real ? __ldg(a.b[li] + j) : 0.0f;
-            a.bias[L.b_off + j] = L.role == 0 ? b * H_TWO_LOG2E : b;
-        }
-        if (threadIdx.x == 0) a.bias[a.zs_off + li] = (L.role == 0 ? H_TWO_LOG2E : 1.0f) * ldexpf(1.0f, -sexp);
-    }
-}
-
 // ------------------------------------------------------------------------------------------------ host side
-int h_add_net(const b200_mlp *m, bool is_actor, HPlan *P, const float **w, const float **b) {
-    if (m->n_layers < 1 || m->n_layers > 4) return B200ENV_ESIZE;
-    for (int l = 0; l < m->n_layers; ++l) {
-        if (P->n_layers >= H_MAX_LAYERS) return B200ENV_ESIZE;
-        const int in = m->dims[l], out = m->dims[l + 1];
-        HLayer &L = P->L[P->n_layers];
-        const bool last = l + 1 == m->n_layers;
-        if (in < 1 || out < 1 || out > 64 || (l == 0 && in > 32) || (last && out > 16)) return B200ENV_ESIZE;
-        L.first = l == 0;
-        L.K = l == 0 ? (in + 7) / 8 * 8 : P->L[P->n_layers - 1].N;
-        L.N = (out + 15) / 16 * 16;
-        L.n_real = out;
-        L.k_real = in;
-        L.role = last ? (is_actor ? 1 : 2) : 0;
-        L.out_act = m->out_act == 2 ? 0 : m->out_act;
-        L.w_off = P->img_bytes;
-        P->img_bytes += (uint32_t)L.K * (uint32_t)L.N * (l == 0 ? 8u : 4u);
-        L.b_off = P->bias_floats;
-        P->bias_floats += L.N;
-        if (w) w[P->n_layers] = m->w[l];
-        if (b) b[P->n_layers] = m->b[l];
-        ++P->n_layers;
-    }
-    return B200ENV_OK;
+int launch(int64_t n, const PolicyPlan &p, const PolicyIO &io, const unsigned char *image, const float *bias,
+           cudaStream_t stream) {
+    static size_t configured[64] = {0};
+    const int rc = b200_opt_in_smem(policy_umma16_kernel, p.smem_bytes, configured);
+    if (rc) return rc;
+    const int64_t tiles = (n + H_TILE - 1) / H_TILE, groups = (tiles + H_SLOTS - 1) / H_SLOTS, cap = b200_sm_count();
+    const HArgs a = {p, image, io, bias};
+    policy_umma16_kernel<<<(unsigned)(groups < cap ? groups : cap), H_THREADS, p.smem_bytes, stream>>>(a, n);
+    return b200_check_launch();
 }
 
-int h_build_plan(const b200_mlp *actor, const b200_mlp *critic, HPlan *P, const float **w, const float **b) {
-    *P = HPlan{};
-    int rc;
-    if (actor && (rc = h_add_net(actor, true, P, w, b))) return rc;
-    if (critic && (rc = h_add_net(critic, false, P, w, b))) return rc;
-    P->S = actor ? actor->dims[0] : critic->dims[0];
-    P->A = actor ? actor->dims[actor->n_layers] : 0;
-    P->zs_off = P->bias_floats;
-    P->bias_floats += H_MAX_LAYERS;
+} // namespace
+
+int policy_umma16_route(const b200_mlp *actor, const b200_mlp *critic, PolicyRoute *r) {
+    int rc = policy_add_nets(actor, critic, 64, 32, true, r);
+    if (rc) return rc;
+    PolicyPlan *P = &r->p;
+    r->launch = launch;
     const uint32_t bias_bytes = ((uint32_t)P->bias_floats * 4 + 127) / 128 * 128;
     const uint32_t b_bytes = (P->img_bytes + 127) / 128 * 128;
     const uint32_t scr_bytes = H_SLOTS * 16 * H_TILE * 4 + 512;
@@ -420,63 +308,4 @@ int h_build_plan(const b200_mlp *actor, const b200_mlp *critic, HPlan *P, const 
     P->off_scr = P->off_bias + bias_bytes;
     P->smem_bytes = P->off_scr + scr_bytes;
     return P->smem_bytes > H_SMEM_LIMIT ? B200ENV_ESIZE : B200ENV_OK;
-}
-
-} // namespace
-
-bool policy_umma16_fits(const b200_mlp *actor, const b200_mlp *critic) {
-    HPlan P;
-    return h_build_plan(actor, critic, &P, nullptr, nullptr) == B200ENV_OK;
-}
-
-size_t policy_umma16_workspace_bytes(const b200_mlp *actor, const b200_mlp *critic) {
-    HPlan P;
-    if (h_build_plan(actor, critic, &P, nullptr, nullptr)) return 0;
-    return (size_t)(P.img_bytes + 127) / 128 * 128 + (size_t)P.bias_floats * 4;
-}
-
-int policy_umma16_pack(const b200_mlp *actor, const b200_mlp *critic, void *workspace, size_t bytes, cudaStream_t stream) {
-    HPackArgs pa = {};
-    HPlan P;
-    int rc = h_build_plan(actor, critic, &P, pa.w, pa.b);
-    if (rc) return rc;
-    for (int l = 0; l < P.n_layers; ++l)
-        if (!pa.w[l] || !pa.b[l]) return B200ENV_ENULL;
-    const size_t img = (size_t)(P.img_bytes + 127) / 128 * 128;
-    if (!workspace) return B200ENV_ENULL;
-    if (bytes < img + (size_t)P.bias_floats * 4 || ((uintptr_t)workspace & 127)) return B200ENV_EPARAMS;
-    pa.n_layers = P.n_layers;
-    pa.zs_off = P.zs_off;
-    for (int l = 0; l < P.n_layers; ++l) pa.L[l] = P.L[l];
-    pa.image = static_cast<unsigned char *>(workspace);
-    pa.bias = reinterpret_cast<float *>(pa.image + img);
-    policy_pack16_kernel<<<dim3(8, P.n_layers), 256, 0, stream>>>(pa);
-    return b200_check_launch();
-}
-
-int policy_launch_umma16(int64_t n, const b200_mlp *actor, const b200_mlp *critic, const void *workspace, size_t bytes,
-                         const PolicyIO &io, cudaStream_t stream) {
-    HArgs a = {};
-    int rc = h_build_plan(actor, critic, &a.p, nullptr, nullptr);
-    if (rc) return rc;
-    const size_t img = (size_t)(a.p.img_bytes + 127) / 128 * 128;
-    if (!workspace) return B200ENV_ENULL;
-    if (bytes < img + (size_t)a.p.bias_floats * 4 || ((uintptr_t)workspace & 127)) return B200ENV_EPARAMS;
-    a.image = static_cast<const unsigned char *>(workspace);
-    a.bias = reinterpret_cast<const float *>(a.image + img);
-    a.io = io;
-    static size_t configured[64] = {0};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64) dev = 0;
-    if (a.p.smem_bytes > configured[dev]) {
-        if (cudaFuncSetAttribute(policy_umma16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)H_SMEM_LIMIT) != cudaSuccess)
-            return b200_check_launch();
-        configured[dev] = H_SMEM_LIMIT;
-    }
-    const int64_t tiles = (n + H_TILE - 1) / H_TILE, groups = (tiles + H_SLOTS - 1) / H_SLOTS;
-    const unsigned cap = b200_persistent_grid(n, 1, 1);
-    const unsigned grid = (unsigned)(groups < (int64_t)cap ? groups : (int64_t)cap);
-    policy_umma16_kernel<<<grid, H_THREADS, a.p.smem_bytes, stream>>>(a, n);
-    return b200_check_launch();
 }

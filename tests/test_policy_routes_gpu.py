@@ -1,8 +1,8 @@
 """K-POLICY (csrc/policy.cu, policy_umma.cu, policy_umma16.cu) against a float64 restatement of choose_action, on every
 kernel route.
 
-Routes.  ``b200_policy_forward_packed`` ("umma") sends a net pair to ``policy_umma16.cu`` when ``policy_umma16_fits``
-holds, else to one of the modes ``build_plan`` of ``policy_umma.cu`` picks: weights resident with the activations in
+Routes.  ``b200_policy_forward_packed`` ("umma") sends a net pair to ``policy_umma16.cu`` when ``policy_umma16_route``
+accepts it, else to one of the modes ``build_plan`` of ``policy_umma.cu`` picks (``policy_route``): weights resident with the activations in
 TMEM ("tmem"), resident with the activations in shared memory and one tile in flight ("smem1"; two tiles, ``cand == 1``,
 is unreachable), or weights streamed through a TMA ring ("streamed").  ``_h_plan`` / ``_u_plan`` restate both host
 plans line for line; ``test_route_restatement_matches_the_library`` holds them to ``b200_policy_workspace_bytes`` and
@@ -15,7 +15,7 @@ the scale of a net's output in units of 2^-24 by a float64 forward pass alongsid
   * each hidden activation adds ``TANH_UNITS``: the SFU tanh (<= 4e-7, about 7 units) and the rounding of the fp16 or
     TF32 operand pair the next layer multiplies (|x| <= 1, <= 6e-8); tanh itself is 1-Lipschitz;
   * every layer multiplied as fp16 hi / lo pairs (each layer after a net's first, on policy_umma16.cu and in the
-    streamed mode) adds ``2^-14 max|W_l| sum_k |h_{l-1,k}|``.  ``policy_pack16_kernel`` / ``policy_pack_kernel`` scale
+    streamed mode) adds ``2^-14 max|W_l| sum_k |h_{l-1,k}|``.  ``policy_pack_kernel`` (both routes) scales
     the whole layer by one power of two that puts max|W_l| just below 2^14, so the lo half of a small weight stops at
     fp16's subnormal spacing 2^-24 of that scale: its error is relative to the layer's largest weight, not to its own
     row (2^-24 * 2^-14 max|W_l| per weight);
@@ -74,83 +74,84 @@ def _fp32_holds(row):
 
 # ------------------------------------------------------------------------------------------------ host plans (CPU)
 def _h_plan(actor, critic):
-    """policy_umma16.cu:380-423 (h_add_net, h_build_plan): the per-layer (K, N, first, role) list, image bytes and bias
-    floats, or None where it returns B200ENV_ESIZE (policy_umma16_fits false)"""
+    """policy_umma16_route (policy_umma16.cu:298-311) over the layer walk policy_add_nets / add_net (policy_umma.cu:582-608,
+    675-687) with the limits 64, 32 and fp16 after a net's first layer: the per-layer (K, N, first, role) list, image
+    bytes and bias floats, or None where it returns B200ENV_ESIZE"""
     layers, img, bias = [], 0, 0
     for dims, is_actor in ((actor, True), (critic, False)):
         if dims is None:
             continue
-        if not 1 <= len(dims) - 1 <= 4:                                    # :381
+        if not 1 <= len(dims) - 1 <= 4:                                    # policy_umma.cu:584
             return None
         for l in range(len(dims) - 1):
-            if len(layers) >= 8:                                           # :383 H_MAX_LAYERS
+            if len(layers) >= 8:                                           # :586 POLICY_MAX_LAYERS
                 return None
             i, o, last = dims[l], dims[l + 1], l + 2 == len(dims)
-            if i < 1 or o < 1 or o > 64 or (l == 0 and i > 32) or (last and o > 16):   # :387
+            if i < 1 or o < 1 or o > 64 or (l == 0 and i > 32) or (last and o > 16):   # :590
                 return None
-            K = (i + 7) // 8 * 8 if l == 0 else layers[-1]["N"]           # :389
-            N = (o + 15) // 16 * 16                                        # :390
+            K = (i + 7) // 8 * 8 if l == 0 else layers[-1]["N"]           # :594
+            N = (o + 15) // 16 * 16                                        # :595
             layers.append(dict(K=K, N=N, first=l == 0, role=(1 if is_actor else 2) if last else 0, f16=l > 0))
-            img += K * N * (8 if l == 0 else 4)                            # :396
-            bias += N                                                      # :398
-    bias += 8                                                              # :414 zs
-    smem = 128 + (img + 127) // 128 * 128 + (bias * 4 + 127) // 128 * 128 + 4 * 16 * 128 * 4 + 512   # :415-421
-    if smem > 227 * 1024:                                                  # :422
+            img += K * N * (8 if l == 0 else 4)                            # :600
+            bias += N                                                      # :602
+    bias += 8                                                              # :685 zs
+    smem = 128 + (img + 127) // 128 * 128 + (bias * 4 + 127) // 128 * 128 + 4 * 16 * 128 * 4 + 512   # policy_umma16.cu:303-309
+    if smem > 227 * 1024:                                                  # policy_umma16.cu:310
         return None
-    return dict(mode="umma16", layers=layers, ws=(img + 127) // 128 * 128 + bias * 4)          # :435
+    return dict(mode="umma16", layers=layers, ws=(img + 127) // 128 * 128 + bias * 4)          # policy_common.cuh:77-79
 
 
 def _u_plan(actor, critic):
-    """policy_umma.cu:616-695 (add_net, build_plan): cand 0 -> "tmem", 1 -> "smem2", 2 -> "smem1", 3 -> "streamed";
-    None where it returns B200ENV_ESIZE"""
+    """policy_umma.cu:582-608, 623-687 (add_net with the limits 256, 256 and no fp16, build_plan): cand 0 -> "tmem",
+    1 -> "smem2", 2 -> "smem1", 3 -> "streamed"; None where it returns B200ENV_ESIZE"""
     layers, img, bias = [], 0, 0
     for dims, is_actor in ((actor, True), (critic, False)):
         if dims is None:
             continue
-        if not 1 <= len(dims) - 1 <= 4:                                    # :617
+        if not 1 <= len(dims) - 1 <= 4:                                    # :584
             return None
         for l in range(len(dims) - 1):
-            if len(layers) >= 8:                                           # :619
+            if len(layers) >= 8:                                           # :586
                 return None
             i, o, last = dims[l], dims[l + 1], l + 2 == len(dims)
-            if i < 1 or o < 1 or i > 256 or o > 256 or (last and o > 16):  # :621, :624
+            if i < 1 or o < 1 or i > 256 or o > 256 or (last and o > 16):  # :590 (hidden inputs: earlier outputs)
                 return None
-            K = (i + 7) // 8 * 8 if l == 0 else layers[-1]["N"]           # :626
-            N = (o + 15) // 16 * 16                                        # :627
+            K = (i + 7) // 8 * 8 if l == 0 else layers[-1]["N"]           # :594
+            N = (o + 15) // 16 * 16                                        # :595
             layers.append(dict(K=K, N=N, first=l == 0, role=(1 if is_actor else 2) if last else 0, f16=False))
-            img += K * N * 8                                               # :632
-            bias += N                                                      # :634
-    bias += 8                                                              # :651
-    nmax = max([16] + [L["N"] for L in layers])                            # :652-656
+            img += K * N * 8                                               # :600
+            bias += N                                                      # :602
+    bias += 8                                                              # :685
+    nmax = max([16] + [L["N"] for L in layers])                            # :628-632
     kmax = max([8] + [L["K"] for L in layers])
-    bias_bytes = (bias * 4 + 127) // 128 * 128                             # :657
-    chunks = (kmax + 31) // 32                                             # :658
-    scr = 2 * 16 * 128 * 4 + 512                                           # :661
-    for cand in range(4):                                                  # :662
+    bias_bytes = (bias * 4 + 127) // 128 * 128                             # :633
+    chunks = (kmax + 31) // 32                                             # :634
+    scr = 2 * 16 * 128 * 4 + 512                                           # :637
+    for cand in range(4):                                                  # :638
         slots, streamed, a_tmem = (2 if cand <= 1 else 1), cand == 3, cand == 0
-        nbuf_log2 = 2 if streamed else (2 if chunks > 2 else 1)            # :664
-        if a_tmem and chunks > (1 << nbuf_log2):                           # :665
+        nbuf_log2 = 2 if streamed else (2 if chunks > 2 else 1)            # :640
+        if a_tmem and chunks > (1 << nbuf_log2):                           # :641
             continue
-        a_bytes = 0 if a_tmem else slots * (1 << nbuf_log2) * 32768        # :666
-        b_bytes = 4 * nmax * 64 if streamed else (img + 127) // 128 * 128  # :667-668
-        total = 256 + a_bytes + b_bytes + bias_bytes + scr                 # :669
-        cols = slots * (2 * nmax + (2 * 32 * (1 << nbuf_log2) if a_tmem else 0))   # :670-671
+        a_bytes = 0 if a_tmem else slots * (1 << nbuf_log2) * 32768        # :642
+        b_bytes = 4 * nmax * 64 if streamed else (img + 127) // 128 * 128  # :643-644
+        total = 256 + a_bytes + b_bytes + bias_bytes + scr                 # :645
+        cols = slots * (2 * nmax + (2 * 32 * (1 << nbuf_log2) if a_tmem else 0))   # :646-647
         pow2 = 32
-        while pow2 < cols:                                                 # :672
+        while pow2 < cols:                                                 # :648
             pow2 *= 2
-        if total > 227 * 1024 or pow2 > 512:                               # :673
+        if total > 227 * 1024 or pow2 > 512:                               # :649
             continue
-        if streamed:                                                       # :674-685
+        if streamed:                                                       # :650-661
             for L in layers:
                 L["f16"] = not L["first"]
             img = sum(L["K"] * L["N"] * (4 if L["f16"] else 8) for L in layers)
         mode = ("tmem", "smem2", "smem1", "streamed")[cand]
-        return dict(mode=mode, layers=layers, ws=(img + 127) // 128 * 128 + bias * 4)   # policy_umma.cu:703
+        return dict(mode=mode, layers=layers, ws=(img + 127) // 128 * 128 + bias * 4)   # policy_common.cuh:77-79
     return None
 
 
 def route(actor, critic):
-    """the plan of b200_policy_forward_packed for this pair (policy_umma.cu:728: policy_umma16_fits first)"""
+    """the plan of b200_policy_forward_packed for this pair (policy_route, policy_umma.cu:689-692: umma16 first)"""
     return _h_plan(actor, critic) or _u_plan(actor, critic)
 
 
