@@ -613,8 +613,8 @@ B200_API int b200_ppo1_grad(const b200_ppo2_batch *batch, const b200_mlp *actor,
  * gradient push, Distributed_PPO2.py:86-104).  Segment j covers elements seg_off[j] .. seg_off[j] + seg_len[j] - 1 of
  * all four buffers and uses learning rate lr[j] (host arrays).  grad_norm_out: device float32 [n_seg] or NULL. */
 B200_API int b200_adam_step(int n_seg, const int64_t *seg_off, const int64_t *seg_len, const float *lr, float *param,
-                            const float *grad, float *exp_avg, float *exp_avg_sq, int64_t step, float beta1,
-                            float beta2, float eps, float max_norm, float grad_scale, float *grad_norm_out,
+                            const float *grad, float *exp_avg, float *exp_avg_sq, int64_t step, double beta1,
+                            double beta2, float eps, float max_norm, float grad_scale, float *grad_norm_out,
                             void *cuda_stream);
 
 /* The keyed permutation of [0, B) the kernels above draw mini-batches from, evaluated on the HOST (no GPU involved):
@@ -631,7 +631,7 @@ B200_API int b200_ppo2_permutation(uint64_t perm_key, int64_t B, int64_t first, 
 B200_API int b200_ppo2_learn(const b200_ppo2_batch *batch, const b200_mlp *actor, const b200_mlp *critic, float std,
                              const float *std_vec, const float *a_min, const float *a_max, float eps_clip,
                              float entropy_coef, int k_epochs, int64_t mini_batch, float lr_actor, float lr_critic,
-                             float beta1, float beta2, float adam_eps, float max_norm, int64_t step, float *param,
+                             double beta1, double beta2, float adam_eps, float max_norm, int64_t step, float *param,
                              float *grad, float *exp_avg, float *exp_avg_sq, float *loss_out, void *workspace,
                              size_t workspace_bytes, void *cuda_stream);
 

@@ -217,12 +217,12 @@ def load() -> C.CDLL:
     lib.b200_ppo1_grad.restype = i32
     lib.b200_ppo1_grad.argtypes = [vp, vp, vp, f32, vp, vp, vp, f32, f32, f32, vp, vp, vp, vp, vp, sz, vp]
     lib.b200_adam_step.restype = i32
-    lib.b200_adam_step.argtypes = [i32, C.POINTER(i64), C.POINTER(i64), C.POINTER(f32), vp, vp, vp, vp, i64, f32, f32, f32,
+    lib.b200_adam_step.argtypes = [i32, C.POINTER(i64), C.POINTER(i64), C.POINTER(f32), vp, vp, vp, vp, i64, f64, f64, f32,
                                    f32, f32, vp, vp]
     lib.b200_ppo2_permutation.restype = i32
     lib.b200_ppo2_permutation.argtypes = [u64, i64, i64, i64, C.POINTER(i64)]
     lib.b200_ppo2_learn.restype = i32
-    lib.b200_ppo2_learn.argtypes = [vp, vp, vp, f32, vp, vp, vp, f32, f32, i32, i64, f32, f32, f32, f32, f32, f32, i64, vp,
+    lib.b200_ppo2_learn.argtypes = [vp, vp, vp, f32, vp, vp, vp, f32, f32, i32, i64, f32, f32, f64, f64, f32, f32, i64, vp,
                                     vp, vp, vp, vp, vp, sz, vp]
     lib.b200_dqn_act.restype = i32
     lib.b200_dqn_act.argtypes = [i64, vp, vp, vp, f32, u64, u64, i64, vp, vp, vp, vp]

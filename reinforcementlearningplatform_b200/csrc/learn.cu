@@ -1152,7 +1152,7 @@ int launch_grad(Plan &pl, cudaStream_t stream, float critic_scale = 1.0f) {
 }
 
 int launch_adam(int n_seg, const int64_t *seg_off, const int64_t *seg_len, const float *lr, float *param, const float *grad,
-                float *m, float *v, int64_t step, float beta1, float beta2, float eps, float max_norm, float grad_scale,
+                float *m, float *v, int64_t step, double beta1, double beta2, float eps, float max_norm, float grad_scale,
                 float *norm_out, cudaStream_t stream) {
     if (n_seg < 1 || n_seg > 2 || !seg_off || !seg_len || !lr) return B200ENV_EPARAMS;
     if (!param || !grad || !m || !v) return B200ENV_ENULL;
@@ -1165,12 +1165,14 @@ int launch_adam(int n_seg, const int64_t *seg_off, const int64_t *seg_len, const
         if (seg_len[j] > longest) longest = seg_len[j];
     }
     a.param = param; a.m = m; a.v = v; a.grad = grad;
-    a.one_minus_b1 = (float)(1.0 - (double)beta1);
-    a.b2 = beta2;
-    a.one_minus_b2 = (float)(1.0 - (double)beta2);
+    // torch.optim.Adam's constants: 1 - beta and the bias corrections in double from the double betas, then rounded
+    // (from float betas, 1 - 0.999f = 0.00099998713 instead of 0.001)
+    a.one_minus_b1 = (float)(1.0 - beta1);
+    a.b2 = (float)beta2;
+    a.one_minus_b2 = (float)(1.0 - beta2);
     a.eps = eps;
-    a.bc1 = (float)(1.0 - pow((double)beta1, (double)step));
-    a.bc2_sqrt = (float)sqrt(1.0 - pow((double)beta2, (double)step));
+    a.bc1 = (float)(1.0 - pow(beta1, (double)step));
+    a.bc2_sqrt = (float)sqrt(1.0 - pow(beta2, (double)step));
     a.max_norm = max_norm;
     a.grad_scale = grad_scale;
     a.norm_out = norm_out;
@@ -1259,7 +1261,7 @@ extern "C" B200_API int b200_ppo1_grad(const b200_ppo2_batch *batch, const b200_
 
 extern "C" B200_API int b200_adam_step(int n_seg, const int64_t *seg_off, const int64_t *seg_len, const float *lr,
                                        float *param, const float *grad, float *exp_avg, float *exp_avg_sq, int64_t step,
-                                       float beta1, float beta2, float eps, float max_norm, float grad_scale,
+                                       double beta1, double beta2, float eps, float max_norm, float grad_scale,
                                        float *grad_norm_out, void *cuda_stream) {
     return launch_adam(n_seg, seg_off, seg_len, lr, param, grad, exp_avg, exp_avg_sq, step, beta1, beta2, eps, max_norm,
                        grad_scale, grad_norm_out, (cudaStream_t)cuda_stream);
@@ -1268,7 +1270,7 @@ extern "C" B200_API int b200_adam_step(int n_seg, const int64_t *seg_off, const 
 extern "C" B200_API int b200_ppo2_learn(const b200_ppo2_batch *batch, const b200_mlp *actor, const b200_mlp *critic,
                                         float std_, const float *std_vec, const float *a_min, const float *a_max,
                                         float eps_clip, float entropy_coef, int k_epochs, int64_t mini_batch,
-                                        float lr_actor, float lr_critic, float beta1, float beta2, float adam_eps,
+                                        float lr_actor, float lr_critic, double beta1, double beta2, float adam_eps,
                                         float max_norm, int64_t step, float *param, float *grad, float *exp_avg,
                                         float *exp_avg_sq, float *loss_out, void *workspace, size_t workspace_bytes,
                                         void *cuda_stream) {

@@ -99,13 +99,23 @@ def allreduce_stats(stats: torch.Tensor, group=None) -> torch.Tensor:
     return stats
 
 
+def agree_sum(value: int, group=None) -> int:
+    """The sum of an integer over the ranks of ``group`` (the value itself without torch.distributed): e.g. the group's
+    instance count, so that counters derived from it are the same on every rank."""
+    return _agree(value, group, dist.ReduceOp.SUM) if dist.is_available() else int(value)
+
+
 def agree_min(value: int, group=None) -> int:
     """The minimum of an integer over the ranks of ``group`` (the value itself without torch.distributed).  Used to agree
     on loop trip counts that contain collectives: ranks whose shard sizes differ by one must not issue different numbers
     of all-reduces (NCCL would deadlock)."""
-    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
+    return _agree(value, group, dist.ReduceOp.MIN) if dist.is_available() else int(value)
+
+
+def _agree(value: int, group, op) -> int:
+    if not dist.is_initialized() or dist.get_world_size(group) == 1:
         return int(value)
     dev = torch.device("cuda", torch.cuda.current_device()) if dist.get_backend(group) == "nccl" else torch.device("cpu")
     t = torch.tensor([int(value)], dtype=torch.int64, device=dev)
-    dist.all_reduce(t, op=dist.ReduceOp.MIN, group=group)
+    dist.all_reduce(t, op=op, group=group)
     return int(t.item())

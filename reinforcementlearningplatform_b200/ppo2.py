@@ -85,7 +85,10 @@ class VecPPO2:
         self._epoch_key = (int(seed) * 0x9E3779B97F4A7C15 + 0x5851F42D4C957F2D) & (2 ** 64 - 1)
         self.reward_norm = Normalization(1, device=env.device, group=group) if reward_norm else None
         self.episodes = EpisodeTracker(env.n_envs, env.device, group=group) if track_episodes else None
+        # total_steps counts the env steps of the whole group: every rank decays its learning rates on the same schedule,
+        # the one a single process holding all the group's instances would follow
         self.total_steps = 0
+        self._group_envs = _dist.agree_sum(env.n_envs, group)
         self._gen = torch.Generator(device=env.device)
         self._gen.manual_seed(seed + 1)
 
@@ -112,7 +115,7 @@ class VecPPO2:
             # r = reward_norm(env.reward) (:210) for the whole column at once: row t enters the statistics after rows < t
             # and is normalised with the statistics after row t, as the per-step calls did (three launches per rollout)
             self.reward_norm.normalize_rows(buf.r, out=buf.r)
-        self.total_steps += buf.batch_size * buf.n_envs
+        self.total_steps += buf.batch_size * self._group_envs
         if self.reward_norm is None:
             return float(buf.r.mean())
         # mean raw reward of this rollout from the normaliser's own float64 statistics (n, mean) before and after it (with
@@ -173,10 +176,11 @@ class VecPPO2:
         # BatchSampler(SubsetRandomSampler(range(B)), mb, drop_last=False) (PPO2.py:104): ceil(B / mb) mini-batches, the last
         # one partial.  Every mini-batch issues gradient all-reduces, so all ranks must run the SAME number of them even
         # when dist.shard() gave them n_local values that differ by one: the count comes from the smallest B of the group
-        # and each rank spreads its own B samples over that many batches.
+        # and each rank spreads its own B samples evenly over that many batches, as the fused path does
+        # (FusedPPO2Update.learn).
         n_mb = _dist.agree_min(-(-B // mb), self.group)
-        bounds = [(B * j) // n_mb for j in range(n_mb + 1)] if n_mb != -(-B // mb) else \
-                 [min(j * mb, B) for j in range(n_mb + 1)]
+        grouped = _dist.dist.is_initialized() and _dist.dist.get_world_size(self.group) > 1
+        bounds = [(B * j) // n_mb for j in range(n_mb + 1)] if grouped else [min(j * mb, B) for j in range(n_mb + 1)]
         last = {}
         for _ in range(self.K_epochs):
             perm = torch.randperm(B, device=s.device, generator=self._gen)
