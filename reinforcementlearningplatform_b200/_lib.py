@@ -8,6 +8,8 @@ from __future__ import annotations
 import ctypes as C
 import os
 
+import torch
+
 _HERE = os.path.dirname(os.path.abspath(__file__))
 # B200ENV_LIB selects an alternative build of the same library (A/B experiments with compile-time options)
 LIB_PATH = os.environ.get("B200ENV_LIB") or os.path.join(_HERE, "libb200env.so")
@@ -16,6 +18,7 @@ LIB_PATH = os.environ.get("B200ENV_LIB") or os.path.join(_HERE, "libb200env.so")
 CARTPOLE, FAS, SOI, BALLBALANCER, TWOLINK, UGV, UGVO, UAV_ATT, UAV_POS, UAVROBUST, FAS_DISCRETE = range(11)
 F64, F32 = 0, 1
 AUTO_RESET = 1
+OUT_ACT = {"identity": 0, "relu": 1, "tanh_range": 2}   # b200_mlp.out_act: the head of the net's last layer
 
 ERRORS = {
     0: "ok",
@@ -255,6 +258,44 @@ def check(rc: int, what: str) -> None:
         if rc == -5:
             extra = f" (cudaError {load().b200env_last_cuda_error()})"
         raise B200EnvError(f"{what}: {ERRORS.get(rc, rc)}{extra}")
+
+
+def ptr(t):
+    """A tensor's device address as a ctypes argument; ``None`` (NULL) for ``None``."""
+    return None if t is None else C.c_void_p(t.data_ptr())
+
+
+def stream(device):
+    """The current CUDA stream of ``device`` as a ctypes argument."""
+    return C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
+
+
+def mlp(layers, out_act: int, base=None) -> MLP:
+    """``struct b200_mlp`` of ``layers``: 1..4 ``nn.Linear`` in forward order, contiguous float32 CUDA with bias.
+    ``base``: a flat float32 buffer laid out like the layers' own storage, which starts at the first layer's weight (a
+    ``learn.FlatParams`` net); the weight and bias pointers are re-based into it, so the descriptor reads a second copy
+    of the parameters (the DQN target net)."""
+    if not 1 <= len(layers) <= 4:
+        raise ValueError("1..4 linear layers")
+    m = MLP()
+    m.n_layers = len(layers)
+    m.dims[0] = layers[0].in_features
+    for l, lin in enumerate(layers):
+        w, b = lin.weight, lin.bias
+        if not (w.is_cuda and w.dtype == torch.float32 and w.is_contiguous() and b is not None and b.is_contiguous()):
+            raise B200EnvError("policy layers must be contiguous float32 CUDA nn.Linear with bias")
+        m.dims[l + 1] = lin.out_features
+        m.w[l], m.b[l] = w.data_ptr(), b.data_ptr()
+    m.out_act = out_act
+    if base is not None:
+        if not (base.is_cuda and base.dtype == torch.float32 and base.is_contiguous()
+                and base.numel() == sum(lin.weight.numel() + lin.bias.numel() for lin in layers)):
+            raise ValueError("mlp: base must be a contiguous float32 CUDA buffer of the layers' parameter count")
+        shift = base.data_ptr() - m.w[0]
+        for l in range(m.n_layers):
+            m.w[l] += shift
+            m.b[l] += shift
+    return m
 
 
 def state_layout(env_id: int, variant: int = 0):

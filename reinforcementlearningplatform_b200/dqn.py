@@ -22,8 +22,8 @@ import torch
 
 from . import _lib
 from . import dist as _dist
-from .episodes import EpisodeTracker
-from .learn import FlatParams
+from .episodes import EpisodeTracker, evaluate_first_episodes
+from .learn import FlatAdam, learn_fits
 from .policy import linear_layers
 
 DEFAULT_DQN_MSG = {
@@ -62,7 +62,7 @@ def q_net(state_dim: int, action_num: int, device, hidden=(64, 64)) -> torch.nn.
     return torch.nn.Sequential(*layers).to(device)
 
 
-class VecDQN:
+class VecDQN(FlatAdam):
     def __init__(self, env, q_net: torch.nn.Module, dqn_msg: Optional[dict] = None, epsilon: float = 0.1, seed: int = 0,
                  group=None, track_episodes: bool = False):
         """The replay ring (``memory_capacity`` = R rows, all on the device):
@@ -101,8 +101,7 @@ class VecDQN:
         self._check_epsilon(epsilon)
         layers = linear_layers(q_net)
         A = int(env.action_num[0])
-        if not (1 <= len(layers) <= 4 and all(l.in_features <= 64 and l.out_features <= 64 and l.bias is not None
-                                                for l in layers)):
+        if not learn_fits(layers, 64):
             raise _lib.B200EnvError("K-DQN: the Q-net must have 1..4 linear layers with bias, widths and state_dim <= 64, "
                                     "<= 64 actions")
         if layers[0].in_features != env.state_dim or layers[-1].out_features != A:
@@ -112,11 +111,10 @@ class VecDQN:
             raise _lib.B200EnvError("the engine has no CPU path: env and Q-net must live on a CUDA device")
         if not env.auto_reset:
             raise ValueError("VecDQN: env must be built with auto_reset=True")
-        self._lib = _lib.load()
+        super().__init__([q_net], [m['lr']], m['betas'], m['adam_eps'], m['max_grad_norm'])
         self.env, self.q_net, self.msg, self.group = env, q_net, m, group
         self.R, self.batch_size, self.A = R, M, A
-        self.gamma, self.lr, self.betas = float(m['gamma']), float(m['lr']), (float(m['betas'][0]), float(m['betas'][1]))
-        self.adam_eps, self.max_grad_norm = float(m['adam_eps']), float(m['max_grad_norm'])
+        self.gamma = float(m['gamma'])
         self.target_replace_iter, self.learn_start = int(m['target_replace_iter']), int(m['learn_start'])
         self.double_dqn = bool(m['double_dqn'])
         self.epsilon, self.seed = float(epsilon), int(seed)
@@ -133,31 +131,19 @@ class VecDQN:
         self.table = torch.tensor(env.action_space[0], **f32)    # the float32 image of action_space[0]
         self._value = torch.zeros((1, N), **f32)                  # the env's action buffer of a collection step
 
-        self.params = FlatParams([q_net])
         self.target = self.params.flat.clone()
-        self._q = self.params.mlp(0, 0)
-        self._q_target = self.params.mlp(0, 0)
-        base, tbase = self.params.flat.data_ptr(), self.target.data_ptr()
-        for l in range(self._q.n_layers):
-            self._q_target.w[l] = tbase + (self._q.w[l] - base)
-            self._q_target.b[l] = tbase + (self._q.b[l] - base)
-        P = self.params.flat.numel()
-        self.grad = torch.zeros(P, **f32)
-        self.exp_avg = torch.zeros(P, **f32)
-        self.exp_avg_sq = torch.zeros(P, **f32)
+        self.q_mlp = self.params.mlp(0, 0)
+        self.target_mlp = _lib.mlp(self.params.layers[0], 0, base=self.target)
         self.loss = torch.zeros(1, **f32)
-        need = int(self._lib.b200_dqn_workspace_bytes(C.byref(self._q), M))
+        need = int(self._lib.b200_dqn_workspace_bytes(C.byref(self.q_mlp), M))
         if need == 0:
             raise _lib.B200EnvError("b200_dqn_workspace_bytes: net not supported by K-DQN")
         self.workspace = torch.zeros(need, dtype=torch.uint8, device=dev)
-        self._seg_off = (C.c_int64 * 1)(0)
-        self._seg_len = (C.c_int64 * 1)(P)
         self._key0 = (self.seed * 0x9E3779B97F4A7C15 + 0x44514E5253) & _M64
 
         self.episodes = EpisodeTracker(N, dev) if track_episodes else None
         self.k = 0                 # collection steps so far (the Philox step of the next one)
         self.updates = 0           # learn() updates so far
-        self.step_count = 0        # Adam steps
         self._started = False
 
     # ------------------------------------------------------------------ small pieces
@@ -169,9 +155,6 @@ class VecDQN:
     def set_epsilon(self, epsilon: float) -> None:
         self._check_epsilon(epsilon)
         self.epsilon = float(epsilon)
-
-    def _stream(self):
-        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
 
     @property
     def valid_rows(self) -> int:
@@ -189,10 +172,10 @@ class VecDQN:
             q: Optional[torch.Tensor] = None) -> None:
         """``b200_dqn_act`` on ``obs_soa [S, N]`` -> ``index [N]`` int32, ``value [1, N]`` (and ``q [A, N]``)."""
         N = obs_soa.shape[1]
-        p = lambda t: None if t is None else C.c_void_p(t.data_ptr())
+        p = _lib.ptr
         with torch.cuda.device(self.device):
             _lib.check(self._lib.b200_dqn_act(
-                N, C.byref(self._q), p(obs_soa), p(self.table), float(epsilon), self.seed & _M64, int(step) & _M64,
+                N, C.byref(self.q_mlp), p(obs_soa), p(self.table), float(epsilon), self.seed & _M64, int(step) & _M64,
                 self.env.env_index_offset, p(index), p(value), p(q), self._stream()), "b200_dqn_act")
 
     # ------------------------------------------------------------------ collection
@@ -236,21 +219,11 @@ class VecDQN:
         if index is not None and not (index.is_cuda and index.dtype == torch.int64 and index.is_contiguous()):
             raise ValueError("grad_step: index must be a contiguous CUDA int64 tensor")
         b = self._batch(sample_key, index)
-        p = lambda t: C.c_void_p(t.data_ptr())
+        p = _lib.ptr
         with torch.cuda.device(self.device):
             _lib.check(self._lib.b200_dqn_grad(
-                C.byref(b), C.byref(self._q), C.byref(self._q_target), self.gamma, int(self.double_dqn), p(self.grad),
+                C.byref(b), C.byref(self.q_mlp), C.byref(self.target_mlp), self.gamma, int(self.double_dqn), p(self.grad),
                 p(self.loss), p(self.workspace), self.workspace.numel(), self._stream()), "b200_dqn_grad")
-
-    def adam_step(self) -> None:
-        self.step_count += 1
-        lr = (C.c_float * 1)(self.lr)
-        p = lambda t: C.c_void_p(t.data_ptr())
-        with torch.cuda.device(self.device):
-            _lib.check(self._lib.b200_adam_step(
-                1, self._seg_off, self._seg_len, lr, p(self.params.flat), p(self.grad), p(self.exp_avg),
-                p(self.exp_avg_sq), self.step_count, self.betas[0], self.betas[1], self.adam_eps, self.max_grad_norm, 1.0,
-                None, self._stream()), "b200_adam_step")
 
     def learn(self, updates: int = 1) -> Optional[dict]:
         """``updates`` x (target copy when due, gradient, Adam).  Returns None (and does nothing) while fewer than
@@ -280,22 +253,9 @@ class VecDQN:
         float32 io), reset here and stepped until every instance has finished an episode (checked every 64 steps) or
         ``max_steps`` steps have run.  Nothing of the agent changes.  Returns ``ep_return``, ``ep_length``, ``ep_flag``
         ([N] device tensors; NaN / -1 = unfinished) and the keys of :meth:`EpisodeTracker.summary`."""
-        if env is self.env or type(env) is not type(self.env):
-            raise ValueError("evaluate_episodes: env must be a separate instance of the training env's class")
-        if not env.auto_reset or env.io_dtype != torch.float32:
-            raise ValueError("evaluate_episodes: env must be built with auto_reset=True and io_dtype=torch.float32")
         if env.state_dim != self.env.state_dim:
             raise ValueError("evaluate_episodes: env dimensions differ from the Q-net's")
-        tracker = EpisodeTracker(env.n_envs, env.device, first_only=True)
         index = torch.empty(env.n_envs, dtype=torch.int32, device=env.device)
         value = torch.empty(1, env.n_envs, dtype=torch.float32, device=env.device)
-        env.reset(True)
-        for t in range(int(max_steps)):
-            # env._reset_obs is the policy-facing observation; step_soa may swap it with _obs, so it is read every step
-            self.act(env._reset_obs, index, value, 0.0, 0)
-            env.step_soa(value)
-            tracker.update(env._reward, env._done, env._flag)
-            if (t + 1) % 64 == 0 and bool(tracker.finished().all()):
-                break
-        return {"ep_return": tracker.ep_return, "ep_length": tracker.ep_length, "ep_flag": tracker.ep_flag,
-                **tracker.summary()}
+        act = lambda obs: self.act(obs, index, value, 0.0, 0)
+        return evaluate_first_episodes(self.env, env, act, value, max_steps, self.group)

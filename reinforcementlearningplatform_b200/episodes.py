@@ -10,7 +10,6 @@ copy; with ``torch.distributed`` initialised they are summed over ranks first.
 """
 from __future__ import annotations
 
-import ctypes as C
 import math
 
 import torch
@@ -19,10 +18,6 @@ from . import _lib
 
 STATS = 22                # B200_EPISODE_STATS (include/b200env.h)
 FLAG_BINS = 16            # flags 0 .. 15 have a bin each; index 16 of flag_counts counts every other flag
-
-
-def _p(t):
-    return None if t is None else C.c_void_p(t.data_ptr())
 
 
 class EpisodeTracker:
@@ -78,13 +73,13 @@ class EpisodeTracker:
             if tuple(t.shape) != shape or not t.is_contiguous() or t.device != self.device:
                 raise ValueError(f"update: r, done and flag must be contiguous tensors of one shape on {self.device}")
         T = shape[0] if len(shape) == 2 else 1
+        p = _lib.ptr
         with torch.cuda.device(self.device):
-            stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
             _lib.check(self._lib.b200_episode_scan(
-                _lib.F64 if r.dtype == torch.float64 else _lib.F32, T, self.n_envs, _p(r), _p(done), _p(flag),
-                _p(self.acc_return), _p(self.acc_length), _p(self.ep_return), _p(self.ep_length), _p(self.ep_flag),
-                int(self.first_only), _p(self.stats), _p(self._scratch), self._scratch.numel() * 8, stream),
-                "b200_episode_scan")
+                _lib.F64 if r.dtype == torch.float64 else _lib.F32, T, self.n_envs, p(r), p(done), p(flag),
+                p(self.acc_return), p(self.acc_length), p(self.ep_return), p(self.ep_length), p(self.ep_flag),
+                int(self.first_only), p(self.stats), p(self._scratch), self._scratch.numel() * 8,
+                _lib.stream(self.device)), "b200_episode_scan")
 
     def finished(self) -> torch.Tensor:
         """bool ``[N]``: the instances that have finished at least one episode since ``reset()``."""
@@ -106,3 +101,27 @@ class EpisodeTracker:
         std = lambda k: math.sqrt(max(v[k + 1] / n - mean(k) ** 2, 0.0)) if n > 0 else math.nan
         return {"episodes": int(n), "mean_return": mean(1), "std_return": std(1), "mean_length": mean(3),
                 "std_length": std(3), "flag_counts": [int(c) for c in v[5:5 + FLAG_BINS + 1]]}
+
+
+def evaluate_first_episodes(train_env, env, act, action: torch.Tensor, max_steps: int, group=None) -> dict:
+    """The first episode of every instance of ``env`` under a fixed policy: ``env`` (a separate instance of
+    ``train_env``'s class, built with ``auto_reset=True, io_dtype=torch.float32``) is reset, then each step
+    ``act(obs)`` writes the action for the policy-facing observation into ``action``, which the env steps with, until
+    every instance has finished an episode (checked every 64 steps, one host read each) or ``max_steps`` steps have run.
+    Returns ``ep_return`` (float64, NaN = unfinished), ``ep_length`` and ``ep_flag`` (int32, -1 = unfinished), all
+    ``[N]`` device tensors, and the keys of :meth:`EpisodeTracker.summary` (summed over ``group``)."""
+    if env is train_env or type(env) is not type(train_env):
+        raise ValueError("evaluate_episodes: env must be a separate instance of the training env's class")
+    if not env.auto_reset or env.io_dtype != torch.float32:
+        raise ValueError("evaluate_episodes: env must be built with auto_reset=True and io_dtype=torch.float32")
+    tracker = EpisodeTracker(env.n_envs, env.device, first_only=True, group=group)
+    env.reset(True)
+    for t in range(int(max_steps)):
+        # env._reset_obs is the policy-facing observation; step_soa may swap it with _obs, so it is read every step
+        act(env._reset_obs)
+        env.step_soa(action)
+        tracker.update(env._reward, env._done, env._flag)
+        if (t + 1) % 64 == 0 and bool(tracker.finished().all()):
+            break
+    return {"ep_return": tracker.ep_return, "ep_length": tracker.ep_length, "ep_flag": tracker.ep_flag,
+            **tracker.summary()}

@@ -7,15 +7,10 @@ normalises with the GLOBAL mean / unbiased std, the multi-GPU analogue of ``adv.
 """
 from __future__ import annotations
 
-import ctypes as C
-
 import torch
 
 from . import _lib
-
-
-def _p(t):
-    return C.c_void_p(t.data_ptr())
+from ._lib import ptr as _p
 
 
 def _scratch(N: int, device) -> torch.Tensor:
@@ -37,10 +32,9 @@ def gae(r, vs, vs_next, done, success, gamma: float, lmd: float, acc_mode: int =
     if stats is None:
         stats = torch.zeros(3, dtype=torch.float64, device=r.device)
     with torch.cuda.device(r.device):
-        stream = C.c_void_p(torch.cuda.current_stream(r.device).cuda_stream)
         scr = _scratch(N, r.device)
         _lib.check(lib.b200_gae(T, N, *[_p(t) for t in ts], float(gamma), float(lmd), int(acc_mode), _p(adv), _p(vt),
-                                _p(stats), _p(scr), scr.numel() * 8, stream), "b200_gae")
+                                _p(stats), _p(scr), scr.numel() * 8, _lib.stream(r.device)), "b200_gae")
     return adv, vt, stats
 
 
@@ -61,11 +55,10 @@ def gae_flags(r, vs, vs_next, done_u8, flag_i32, timeout_flag: int, gamma: float
     if stats is None:
         stats = torch.zeros(3, dtype=torch.float64, device=r.device)
     with torch.cuda.device(r.device):
-        stream = C.c_void_p(torch.cuda.current_stream(r.device).cuda_stream)
         scr = _scratch(N, r.device)
         _lib.check(lib.b200_gae_flags(T, N, _p(r), _p(vs), _p(vs_next), _p(done_u8), _p(flag_i32), int(timeout_flag),
                                       float(gamma), float(lmd), int(acc_mode), _p(adv), _p(vt), _p(stats), _p(scr),
-                                      scr.numel() * 8, stream), "b200_gae_flags")
+                                      scr.numel() * 8, _lib.stream(r.device)), "b200_gae_flags")
     return adv, vt, stats
 
 
@@ -77,8 +70,8 @@ def normalize_advantage(adv: torch.Tensor, stats: torch.Tensor, eps: float = 1e-
         dist.all_reduce(stats, op=dist.ReduceOp.SUM, group=group)
     lib = _lib.load()
     with torch.cuda.device(adv.device):
-        stream = C.c_void_p(torch.cuda.current_stream(adv.device).cuda_stream)
-        _lib.check(lib.b200_adv_normalize(adv.numel(), _p(adv), _p(stats), float(eps), stream), "b200_adv_normalize")
+        _lib.check(lib.b200_adv_normalize(adv.numel(), _p(adv), _p(stats), float(eps), _lib.stream(adv.device)),
+                   "b200_adv_normalize")
     return adv
 
 
@@ -98,7 +91,7 @@ def mc_returns(r: torch.Tensor, done_u8: torch.Tensor, gamma: float, stats: torc
     out = torch.empty(T, N, dtype=torch.float32, device=r.device)
     dt = _lib.F64 if r.dtype == torch.float64 else _lib.F32
     with torch.cuda.device(r.device):
-        stream = C.c_void_p(torch.cuda.current_stream(r.device).cuda_stream)
+        stream = _lib.stream(r.device)
         if stats is None:
             _lib.check(_lib.load().b200_mc_returns(dt, T, N, _p(r), _p(done_u8), float(gamma), _p(out), stream),
                        "b200_mc_returns")

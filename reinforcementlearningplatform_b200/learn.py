@@ -21,7 +21,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .policy import linear_layers
+from .policy import gaussian_head, linear_layers
 
 
 class FlatParams:
@@ -43,62 +43,80 @@ class FlatParams:
             o += n
 
     def mlp(self, k: int, out_act: int) -> _lib.MLP:
-        layers = self.layers[k]
-        m = _lib.MLP()
-        m.n_layers = len(layers)
-        m.dims[0] = layers[0].in_features
-        for l, lin in enumerate(layers):
-            m.dims[l + 1] = lin.out_features
-            m.w[l], m.b[l] = lin.weight.data_ptr(), lin.bias.data_ptr()
-        m.out_act = out_act
-        return m
+        """``struct b200_mlp`` of net ``k`` (its parameters live in the flat buffer, so the pointers stay valid)."""
+        return _lib.mlp(self.layers[k], out_act)
+
+
+def learn_fits(layers, max_out: int) -> bool:
+    """The nets K-LEARN and K-DQN hold (every layer in shared memory): 1..4 linear layers with bias, widths and state_dim
+    <= 64, at most ``max_out`` outputs (16 actions for the PPO actor, 64 for a Q-net)."""
+    return (1 <= len(layers) <= 4 and all(l.in_features <= 64 and l.out_features <= 64 and l.bias is not None
+                                          for l in layers) and layers[-1].out_features <= max_out)
 
 
 def fused_supported(actor, critic) -> bool:
     """K-LEARN holds every layer in shared memory: <= 4 layers per net, widths and state_dim <= 64, <= 16 actions."""
-    for net in (actor, critic):
-        layers = linear_layers(net)
-        if not 1 <= len(layers) <= 4:
-            return False
-        if any(l.in_features > 64 or l.out_features > 64 or l.bias is None for l in layers):
-            return False
-    return linear_layers(actor)[-1].out_features <= 16 and linear_layers(critic)[-1].out_features == 1
+    critic = linear_layers(critic)
+    return learn_fits(linear_layers(actor), 16) and learn_fits(critic, 1) and critic[-1].out_features == 1
 
 
-class FusedPPO2Update:
-    def __init__(self, actor, critic, std, a_min, a_max, actor_out_act: str = "relu", a_lr: float = 1e-4,
-                 c_lr: float = 1e-3, adam_eps: float = 1e-5, betas=(0.9, 0.999), max_grad_norm: float = 0.5,
-                 eps_clip: float = 0.2, entropy_coef: float = 0.01, group=None):
+class FlatAdam:
+    """The parameters of ``nets`` in one flat buffer (:class:`FlatParams`, one Adam segment per net), their gradient and
+    Adam moments, and the clip_grad_norm_ + Adam step over all segments in one launch (``b200_adam_step``).  ``lr``: one
+    learning rate per net; ``grad_norm``: the gradient norm of every segment at the last step.  The flat buffers are
+    allocated here once and never re-bound: the launches hold their addresses."""
+
+    def __init__(self, nets, lr, betas, adam_eps: float, max_grad_norm: float):
         self._lib = _lib.load()
-        if not fused_supported(actor, critic):
-            raise _lib.B200EnvError("K-LEARN: nets must have <= 4 layers, widths <= 64, <= 16 actions, 1 value")
-        self.params = FlatParams([actor, critic])
+        self.params = FlatParams(nets)
         self.device = self.params.flat.device
         if self.device.type != "cuda":
             raise _lib.B200EnvError("the engine has no CPU path: nets must live on a CUDA device")
-        self.out_act = {"identity": 0, "relu": 1, "tanh_range": 2}[actor_out_act]
-        self.a_min = torch.as_tensor(np.asarray(a_min, dtype=np.float32), device=self.device).contiguous()
-        self.a_max = torch.as_tensor(np.asarray(a_max, dtype=np.float32), device=self.device).contiguous()
-        std_arr = np.asarray(std.detach().cpu() if torch.is_tensor(std) else std, dtype=np.float32).reshape(-1)
-        self.std_vec = torch.as_tensor(std_arr, device=self.device).contiguous() if std_arr.size > 1 else None
-        self.std = float(std_arr[0])
-        self.lr = [float(a_lr), float(c_lr)]
+        self.lr = [float(x) for x in lr]
         self.adam_eps, self.betas, self.max_grad_norm = float(adam_eps), (float(betas[0]), float(betas[1])), float(max_grad_norm)
-        self.eps_clip, self.entropy_coef, self.group = float(eps_clip), float(entropy_coef), group
-        n = self.params.flat.numel()
-        self.grad = torch.zeros(n, dtype=torch.float32, device=self.device)
+        k = len(nets)
+        self.grad = torch.zeros(self.params.flat.numel(), dtype=torch.float32, device=self.device)
         self.exp_avg = torch.zeros_like(self.grad)
         self.exp_avg_sq = torch.zeros_like(self.grad)
-        self.loss = torch.zeros(2, dtype=torch.float32, device=self.device)
-        self.grad_norm = torch.zeros(2, dtype=torch.float32, device=self.device)
+        self.grad_norm = torch.zeros(k, dtype=torch.float32, device=self.device)
         self.step_count = 0
-        am, cm = self.params.mlp(0, self.out_act), self.params.mlp(1, 0)
-        need = int(self._lib.b200_ppo2_workspace_bytes(C.byref(am), C.byref(cm)))
+        # the arguments of b200_adam_step that never change, built once: a small update is bound by its host work
+        self._segs = (k, (C.c_int64 * k)(*self.params.net_off), (C.c_int64 * k)(*self.params.net_len))
+        self._lr_array = C.c_float * k
+        self._bufs = tuple(map(_lib.ptr, (self.params.flat, self.grad, self.exp_avg, self.exp_avg_sq)))
+        self._norm_out = _lib.ptr(self.grad_norm)
+
+    def _stream(self):
+        return _lib.stream(self.device)
+
+    def adam_step(self, grad_scale: float = 1.0) -> None:
+        """clip_grad_norm_ + Adam over every parameter segment (one launch); ``grad_scale`` multiplies the gradient
+        first (1 / world size after a summing all-reduce)."""
+        self.step_count += 1
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.b200_adam_step(
+                *self._segs, self._lr_array(*self.lr), *self._bufs, self.step_count, self.betas[0], self.betas[1],
+                self.adam_eps, self.max_grad_norm, float(grad_scale), self._norm_out, self._stream()),
+                "b200_adam_step")
+
+
+class FusedPPO2Update(FlatAdam):
+    def __init__(self, actor, critic, std, a_min, a_max, actor_out_act: str = "relu", a_lr: float = 1e-4,
+                 c_lr: float = 1e-3, adam_eps: float = 1e-5, betas=(0.9, 0.999), max_grad_norm: float = 0.5,
+                 eps_clip: float = 0.2, entropy_coef: float = 0.01, group=None):
+        if not fused_supported(actor, critic):
+            raise _lib.B200EnvError("K-LEARN: nets must have <= 4 layers, widths <= 64, <= 16 actions, 1 value")
+        super().__init__([actor, critic], (a_lr, c_lr), betas, adam_eps, max_grad_norm)
+        self.out_act, self.a_min, self.a_max, self.std, self.std_vec = gaussian_head(std, a_min, a_max, actor_out_act,
+                                                                                     self.device)
+        self.eps_clip, self.entropy_coef, self.group = float(eps_clip), float(entropy_coef), group
+        self.loss = torch.zeros(2, dtype=torch.float32, device=self.device)
+        # the parameters live in the flat buffer from here on, so the descriptors' pointers stay valid
+        self.mlps = (self.params.mlp(0, self.out_act), self.params.mlp(1, 0))
+        need = int(self._lib.b200_ppo2_workspace_bytes(*map(C.byref, self.mlps)))
         if need == 0:
             raise _lib.B200EnvError("b200_ppo2_workspace_bytes: net not supported by K-LEARN")
         self.workspace = torch.zeros(need, dtype=torch.uint8, device=self.device)
-        self._seg_off = (C.c_int64 * 2)(*self.params.net_off)
-        self._seg_len = (C.c_int64 * 2)(*self.params.net_len)
 
     # ------------------------------------------------------------------ pieces
     def _batch(self, s, a, a_lp, adv, v_target, first, count, perm_key=0, index=None) -> _lib.PPO2Batch:
@@ -115,21 +133,27 @@ class FusedPPO2Update:
         b.first, b.count, b.perm_key = int(first), int(count), int(perm_key) & (2 ** 64 - 1)
         return b
 
-    def _stream(self):
-        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+    def _args(self, b: _lib.PPO2Batch) -> tuple:
+        """The arguments b200_ppo2_grad, b200_ppo1_grad and b200_ppo2_learn share, in their order: the batch, both nets,
+        the Gaussian head, the clip range and the entropy coefficient.  Read at every call: ``VecPPO2.set_action_std``
+        may have changed the scalar ``std``."""
+        p = _lib.ptr
+        return (C.byref(b), *map(C.byref, self.mlps), self.std, p(self.std_vec), p(self.a_min), p(self.a_max),
+                self.eps_clip, self.entropy_coef)
+
+    def _grads(self) -> tuple:
+        """``grad_actor, grad_critic``: the two segments of ``self.grad``."""
+        return _lib.ptr(self.grad), C.c_void_p(self.grad.data_ptr() + 4 * self.params.net_off[1])
 
     def grad_step(self, s, a, a_lp, adv, v_target, first: int, count: int, perm_key: int = 0,
                   index: Optional[torch.Tensor] = None) -> None:
         """Gradients of both mean losses for one mini-batch -> ``self.grad`` ([actor | critic]); losses -> ``self.loss``."""
         b = self._batch(s, a, a_lp, adv, v_target, first, count, perm_key, index)
-        am, cm = self.params.mlp(0, self.out_act), self.params.mlp(1, 0)
-        p = lambda t: None if t is None else C.c_void_p(t.data_ptr())
-        o = self.params.net_off[1]
+        p = _lib.ptr
         with torch.cuda.device(self.device):
             _lib.check(self._lib.b200_ppo2_grad(
-                C.byref(b), C.byref(am), C.byref(cm), self.std, p(self.std_vec), p(self.a_min), p(self.a_max),
-                self.eps_clip, self.entropy_coef, p(self.grad), C.c_void_p(self.grad.data_ptr() + 4 * o), p(self.loss),
-                p(self.workspace), self.workspace.numel(), self._stream()), "b200_ppo2_grad")
+                *self._args(b), *self._grads(), p(self.loss), p(self.workspace), self.workspace.numel(),
+                self._stream()), "b200_ppo2_grad")
 
     def ppo1_grad_step(self, s, a, a_lp, ret_hat, adv_out, value_coef: float, first: int, count: int, perm_key: int = 0,
                        index: Optional[torch.Tensor] = None, value: Optional[torch.Tensor] = None) -> None:
@@ -140,26 +164,11 @@ class FusedPPO2Update:
         if value is not None and not (value.is_cuda and value.dtype == torch.float32 and value.is_contiguous()
                                       and tuple(value.shape) == tuple(ret_hat.shape)):
             raise ValueError("K-LEARN: value must be a contiguous CUDA float32 [T, N] tensor")
-        am, cm = self.params.mlp(0, self.out_act), self.params.mlp(1, 0)
-        p = lambda t: None if t is None else C.c_void_p(t.data_ptr())
-        o = self.params.net_off[1]
+        p = _lib.ptr
         with torch.cuda.device(self.device):
             _lib.check(self._lib.b200_ppo1_grad(
-                C.byref(b), C.byref(am), C.byref(cm), self.std, p(self.std_vec), p(self.a_min), p(self.a_max),
-                self.eps_clip, self.entropy_coef, float(value_coef), p(value), p(self.grad),
-                C.c_void_p(self.grad.data_ptr() + 4 * o), p(self.loss), p(self.workspace), self.workspace.numel(),
-                self._stream()), "b200_ppo1_grad")
-
-    def adam_step(self, grad_scale: float = 1.0) -> None:
-        """clip_grad_norm_ + Adam over both parameter segments (one launch)."""
-        self.step_count += 1
-        lr = (C.c_float * 2)(*self.lr)
-        p = lambda t: C.c_void_p(t.data_ptr())
-        with torch.cuda.device(self.device):
-            _lib.check(self._lib.b200_adam_step(
-                2, self._seg_off, self._seg_len, lr, p(self.params.flat), p(self.grad), p(self.exp_avg), p(self.exp_avg_sq),
-                self.step_count, self.betas[0], self.betas[1], self.adam_eps, self.max_grad_norm, float(grad_scale),
-                p(self.grad_norm), self._stream()), "b200_adam_step")
+                *self._args(b), float(value_coef), p(value), *self._grads(), p(self.loss), p(self.workspace),
+                self.workspace.numel(), self._stream()), "b200_ppo1_grad")
 
     # ------------------------------------------------------------------ the loop
     def learn(self, s, a, a_lp, adv, v_target, k_epochs: int, mini_batch: int, perm_key: int, n_mb: Optional[int] = None):
@@ -173,12 +182,10 @@ class FusedPPO2Update:
         world = dist.get_world_size(self.group) if dist.is_available() and dist.is_initialized() else 1
         if world == 1 and n_mb is None:
             b = self._batch(s, a, a_lp, adv, v_target, 0, B, perm_key)
-            am, cm = self.params.mlp(0, self.out_act), self.params.mlp(1, 0)
-            p = lambda t: None if t is None else C.c_void_p(t.data_ptr())
+            p = _lib.ptr
             with torch.cuda.device(self.device):
                 _lib.check(self._lib.b200_ppo2_learn(
-                    C.byref(b), C.byref(am), C.byref(cm), self.std, p(self.std_vec), p(self.a_min), p(self.a_max),
-                    self.eps_clip, self.entropy_coef, int(k_epochs), int(mini_batch), self.lr[0], self.lr[1], self.betas[0],
+                    *self._args(b), int(k_epochs), int(mini_batch), self.lr[0], self.lr[1], self.betas[0],
                     self.betas[1], self.adam_eps, self.max_grad_norm, self.step_count + 1, p(self.params.flat), p(self.grad),
                     p(self.exp_avg), p(self.exp_avg_sq), p(self.loss), p(self.workspace), self.workspace.numel(),
                     self._stream()), "b200_ppo2_learn")

@@ -18,13 +18,13 @@ std`` names (``std = mean`` while ``n == 1``, sic).
 """
 from __future__ import annotations
 
-import ctypes as C
 from typing import Optional
 
 import numpy as np
 import torch
 
 from . import _lib
+from ._lib import ptr as _p
 
 EPS = 1e-8  # utils/classes.py:654
 
@@ -115,9 +115,6 @@ class Normalization:
             return _lib.F32
         raise ValueError("normalisation input must be float32 or float64")
 
-    def _stream(self):
-        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-
     def _world(self) -> int:
         import torch.distributed as dist
         if self.sync and dist.is_available() and dist.is_initialized():
@@ -134,19 +131,19 @@ class Normalization:
             raise ValueError(f"normalize_soa: expected a contiguous CUDA [{self.dim}, N] tensor")
         code, n = self._code(x), x.shape[1]
         y = torch.empty_like(x) if out is None else out.view_as(x)
-        p = lambda t: C.c_void_p(t.data_ptr())
         with torch.cuda.device(self.device):
+            stream = _lib.stream(self.device)
             nb, batch = 0, self._batch
             if update:
-                _lib.check(self._lib.b200_norm_batch_stats(code, n, self.dim, p(x), p(self._run), p(self._batch),
-                                                           p(self._scratch), self._stream()), "b200_norm_batch_stats")
+                _lib.check(self._lib.b200_norm_batch_stats(code, n, self.dim, _p(x), _p(self._run), _p(self._batch),
+                                                           _p(self._scratch), stream), "b200_norm_batch_stats")
                 nb = 1
                 w = self._world()
                 if w > 1:
                     self._gathered = gather_batch_stats(self._batch, self._gathered, self.group)
                     nb, batch = w, self._gathered
-            _lib.check(self._lib.b200_norm_merge_apply(code, n, self.dim, p(x), p(y), p(batch), nb, p(self._run),
-                                                       p(self._run_next), 1 if update else 0, EPS, self._stream()),
+            _lib.check(self._lib.b200_norm_merge_apply(code, n, self.dim, _p(x), _p(y), _p(batch), nb, _p(self._run),
+                                                       _p(self._run_next), 1 if update else 0, EPS, stream),
                        "b200_norm_merge_apply")
             if update:
                 self._run, self._run_next = self._run_next, self._run
@@ -171,19 +168,19 @@ class Normalization:
             self._rows_cum = torch.zeros(3, T, dtype=torch.float64, device=self.device)
             self._rows_scratch = torch.zeros(self._lib.b200_norm_scratch_bytes(T), dtype=torch.uint8, device=self.device)
             self._rows_gathered = None
-        p = lambda t: C.c_void_p(t.data_ptr())
         with torch.cuda.device(self.device):
-            _lib.check(self._lib.b200_norm_batch_stats(code, n, T, p(x), None, p(self._rows_batch), p(self._rows_scratch),
-                                                       self._stream()), "b200_norm_batch_stats")
+            stream = _lib.stream(self.device)
+            _lib.check(self._lib.b200_norm_batch_stats(code, n, T, _p(x), None, _p(self._rows_batch), _p(self._rows_scratch),
+                                                       stream), "b200_norm_batch_stats")
             nb, batch = 1, self._rows_batch
             w = self._world()
             if w > 1:
                 self._rows_gathered = gather_batch_stats(self._rows_batch, self._rows_gathered, self.group)
                 nb, batch = w, self._rows_gathered
-            _lib.check(self._lib.b200_norm_rows_prefix(T, p(batch), nb, p(self._run), p(self._rows_cum), p(self._run_next),
-                                                       self._stream()), "b200_norm_rows_prefix")
-            _lib.check(self._lib.b200_norm_merge_apply(code, n, T, p(x), p(y), None, 0, p(self._rows_cum), None, 0, EPS,
-                                                       self._stream()), "b200_norm_merge_apply")
+            _lib.check(self._lib.b200_norm_rows_prefix(T, _p(batch), nb, _p(self._run), _p(self._rows_cum), _p(self._run_next),
+                                                       stream), "b200_norm_rows_prefix")
+            _lib.check(self._lib.b200_norm_merge_apply(code, n, T, _p(x), _p(y), None, 0, _p(self._rows_cum), None, 0, EPS,
+                                                       stream), "b200_norm_merge_apply")
             self._run, self._run_next = self._run_next, self._run
         return y
 
@@ -212,9 +209,8 @@ class Normalization:
             raise ValueError(f"seq: expected a contiguous CUDA [{self.dim}, rows] tensor")
         y = torch.empty_like(x)
         with torch.cuda.device(self.device):
-            _lib.check(self._lib.b200_norm_seq(self._code(x), x.shape[1], self.dim, C.c_void_p(x.data_ptr()),
-                                               C.c_void_p(y.data_ptr()), C.c_void_p(self._run.data_ptr()),
-                                               1 if update else 0, EPS, self._stream()), "b200_norm_seq")
+            _lib.check(self._lib.b200_norm_seq(self._code(x), x.shape[1], self.dim, _p(x), _p(y), _p(self._run),
+                                               1 if update else 0, EPS, _lib.stream(self.device)), "b200_norm_seq")
         return y
 
     # ------------------------------------------------------------------ state

@@ -30,6 +30,26 @@ def linear_layers(module) -> list:
     return [m for m in module.modules() if isinstance(m, torch.nn.Linear)]
 
 
+def gaussian_std(std, device=None, out: Optional[torch.Tensor] = None):
+    """``(std, std_vec)`` as K-POLICY and K-LEARN take them: a scalar std is ``(float, None)``; one value per action
+    dimension is ``(1.0, float32 tensor on device)`` -- no kernel reads the scalar then.  ``out``: the ``std_vec`` of an
+    existing head, overwritten in place instead of allocating a new one."""
+    arr = np.asarray(std.detach().cpu() if torch.is_tensor(std) else std, dtype=np.float32).reshape(-1)
+    if arr.size == 1:
+        return float(arr[0]), None
+    if out is None:
+        return 1.0, torch.as_tensor(arr, device=device).contiguous()
+    out.copy_(torch.as_tensor(arr, device=out.device))
+    return 1.0, out
+
+
+def gaussian_head(std, a_min, a_max, out_act: str, device):
+    """The Gaussian action head of an actor, as K-POLICY and K-LEARN read it: ``(out_act code, a_min, a_max, std,
+    std_vec)`` with the action clamp as float32 device tensors and ``std, std_vec`` from :func:`gaussian_std`."""
+    bound = lambda x: torch.as_tensor(np.asarray(x, dtype=np.float32), device=device).contiguous()
+    return (_lib.OUT_ACT[out_act], bound(a_min), bound(a_max), *gaussian_std(std, device))
+
+
 class GaussianPolicy:
     def __init__(self, actor_layers: Optional[Sequence], critic_layers: Optional[Sequence], a_min, a_max, std: float,
                  device="cuda", seed: int = 0, env_index_offset: int = 0, actor_out_act: str = "relu",
@@ -50,18 +70,10 @@ class GaussianPolicy:
             raise _lib.B200EnvError("the engine has no CPU path: device must be a CUDA device")
         as_list = lambda x: None if x is None else (list(x) if isinstance(x, (list, tuple)) else linear_layers(x))
         self.actor, self.critic = as_list(actor_layers), as_list(critic_layers)
-        self.out_act = {"identity": 0, "relu": 1, "tanh_range": 2}[actor_out_act]
-        self.a_min = torch.as_tensor(np.asarray(a_min, dtype=np.float32), device=self.device).contiguous()
-        self.a_max = torch.as_tensor(np.asarray(a_max, dtype=np.float32), device=self.device).contiguous()
-        std_arr = np.asarray(std, dtype=np.float32).reshape(-1)
-        self.std_vec = None
-        if std_arr.size > 1:
-            if self.precision != "umma":
-                raise ValueError("a per-dimension std needs precision='umma'")
-            self.std_vec = torch.as_tensor(std_arr, device=self.device).contiguous()
-            self.std = 1.0
-        else:
-            self.std = float(std_arr[0])
+        self.out_act, self.a_min, self.a_max, self.std, self.std_vec = gaussian_head(std, a_min, a_max, actor_out_act,
+                                                                                     self.device)
+        if self.std_vec is not None and self.precision != "umma":
+            raise ValueError("a per-dimension std needs precision='umma'")
         self._ws = None          # packed weights (precision "umma")
         self._ws_versions = None
         self.seed, self.env_index_offset, self.step = int(seed), int(env_index_offset), 0
@@ -69,21 +81,6 @@ class GaussianPolicy:
             self.state_dim, self.action_dim = self.actor[0].in_features, self.actor[-1].out_features
         else:
             self.state_dim, self.action_dim = self.critic[0].in_features, 0
-
-    def _mlp(self, layers, out_act) -> _lib.MLP:
-        m = _lib.MLP()
-        m.n_layers = len(layers)
-        if not 1 <= len(layers) <= 4:
-            raise ValueError("1..4 linear layers")
-        m.dims[0] = layers[0].in_features
-        for l, lin in enumerate(layers):
-            w, b = lin.weight, lin.bias
-            if not (w.is_cuda and w.dtype == torch.float32 and w.is_contiguous() and b is not None and b.is_contiguous()):
-                raise _lib.B200EnvError("policy layers must be contiguous float32 CUDA nn.Linear with bias")
-            m.dims[l + 1] = lin.out_features
-            m.w[l], m.b[l] = w.data_ptr(), b.data_ptr()
-        m.out_act = out_act
-        return m
 
     def forward(self, obs_soa: torch.Tensor, noise: Optional[torch.Tensor] = None, *, action: torch.Tensor = None,
                 log_prob: torch.Tensor = None, mean: torch.Tensor = None, value: torch.Tensor = None,
@@ -98,7 +95,7 @@ class GaussianPolicy:
         out = {}
         am = cm = None
         if self.actor:
-            am = self._mlp(self.actor, self.out_act)
+            am = _lib.mlp(self.actor, self.out_act)
             out["action"] = action if action is not None else torch.empty(A, n, dtype=torch.float32, device=dev)
             out["log_prob"] = log_prob if log_prob is not None else torch.empty(A, n, dtype=torch.float32, device=dev)
             if want_mean or mean is not None:
@@ -106,21 +103,20 @@ class GaussianPolicy:
             if noise is not None and not (noise.shape == (A, n) and noise.dtype == torch.float32 and noise.is_contiguous()):
                 raise ValueError("noise must be a contiguous float32 [A, N] tensor")
         if self.critic:
-            cm = self._mlp(self.critic, 0)
+            cm = _lib.mlp(self.critic, 0)
             out["value"] = value if value is not None else torch.empty(n, dtype=torch.float32, device=dev)
-        p = lambda t: None if t is None else C.c_void_p(t.data_ptr())
         if self.precision == "umma":
             self._forward_umma(n, am, cm, obs_soa, noise, out)
             if noise is None:
                 self.step += 1
             return out
+        p = _lib.ptr
         with torch.cuda.device(dev):
-            stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
             _lib.check(self._lib.b200_policy_forward(
                 n, None if am is None else C.byref(am), None if cm is None else C.byref(cm), p(obs_soa), p(self.a_min),
                 p(self.a_max), self.std, p(noise), self.seed, self.step, self.env_index_offset, 0,  # B200_POLICY_FP32
                 p(out.get("action")),
-                p(out.get("log_prob")), p(out.get("mean")), p(out.get("value")), stream), "b200_policy_forward")
+                p(out.get("log_prob")), p(out.get("mean")), p(out.get("value")), _lib.stream(dev)), "b200_policy_forward")
         if noise is None:
             self.step += 1
         return out
@@ -132,8 +128,8 @@ class GaussianPolicy:
     def refresh(self, am=None, cm=None):
         """(Re)pack the weights into the tensor core's operand layout (b200_policy_pack).  Called automatically by
         ``forward`` when a parameter changed in place; call it yourself after replacing ``.data`` of a parameter."""
-        am = am if am is not None or not self.actor else self._mlp(self.actor, self.out_act)
-        cm = cm if cm is not None or not self.critic else self._mlp(self.critic, 0)
+        am = am if am is not None or not self.actor else _lib.mlp(self.actor, self.out_act)
+        cm = cm if cm is not None or not self.critic else _lib.mlp(self.critic, 0)
         ra, rc = (None if am is None else C.byref(am)), (None if cm is None else C.byref(cm))
         need = int(self._lib.b200_policy_workspace_bytes(ra, rc))
         if need == 0:
@@ -141,22 +137,21 @@ class GaussianPolicy:
         if self._ws is None or self._ws.numel() < need:
             self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)   # torch allocations are 512 B aligned
         with torch.cuda.device(self.device):
-            stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-            _lib.check(self._lib.b200_policy_pack(ra, rc, C.c_void_p(self._ws.data_ptr()), self._ws.numel(), stream),
+            _lib.check(self._lib.b200_policy_pack(ra, rc, _lib.ptr(self._ws), self._ws.numel(), _lib.stream(self.device)),
                        "b200_policy_pack")
         self._ws_versions = self._param_versions()
 
     def _forward_umma(self, n, am, cm, obs_soa, noise, out):
         if self._ws is None or self._ws_versions != self._param_versions():
             self.refresh(am, cm)
-        p = lambda t: None if t is None else C.c_void_p(t.data_ptr())
+        p = _lib.ptr
         dev = obs_soa.device
         with torch.cuda.device(dev):
-            stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
             _lib.check(self._lib.b200_policy_forward_packed(
                 n, None if am is None else C.byref(am), None if cm is None else C.byref(cm),
-                C.c_void_p(self._ws.data_ptr()), self._ws.numel(), p(obs_soa), p(self.a_min), p(self.a_max), self.std,
+                p(self._ws), self._ws.numel(), p(obs_soa), p(self.a_min), p(self.a_max), self.std,
                 p(self.std_vec), p(noise), self.seed, self.step, self.env_index_offset, p(out.get("action")),
-                p(out.get("log_prob")), p(out.get("mean")), p(out.get("value")), stream), "b200_policy_forward_packed")
+                p(out.get("log_prob")), p(out.get("mean")), p(out.get("value")), _lib.stream(dev)),
+                "b200_policy_forward_packed")
 
     __call__ = forward

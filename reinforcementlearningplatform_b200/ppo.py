@@ -65,9 +65,6 @@ class VecPPO(VecPPO2):
                 if world > 1:
                     _dist.dist.all_reduce(self.fused.grad, op=_dist.dist.ReduceOp.SUM, group=self.group)
                 self.fused.adam_step(1.0 / world)
-        self.policy.refresh()            # K-POLICY multiplies from a packed copy of the weights
-        self.value_net.refresh()
-        if self.msg['use_lr_decay']:
-            self.lr_decay(self.total_steps)
+        self._after_fused_update()
         la, lc = self.fused.loss.tolist()
         return {"actor_loss": la, "critic_loss": lc, "loss": la + lc}

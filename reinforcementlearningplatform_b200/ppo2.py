@@ -27,10 +27,10 @@ import torch
 import torch.nn.functional as F
 
 from . import dist as _dist
-from .episodes import EpisodeTracker
+from .episodes import EpisodeTracker, evaluate_first_episodes
 from .learn import FusedPPO2Update, fused_supported
 from .normalization import Normalization
-from .policy import GaussianPolicy, linear_layers
+from .policy import GaussianPolicy, gaussian_std, linear_layers
 from .rollout import RolloutBuffer
 
 DEFAULT_PPO_MSG = {  # demonstration/PPO2/PPO2-4-CartPoleAngleOnly/train.py:141-158
@@ -133,15 +133,10 @@ class VecPPO2:
                              f"got shape {new.shape}")
         if not (np.isfinite(new).all() and (new > 0).all()):
             raise ValueError("set_action_std: std must be finite and positive")
-        new = new.reshape(-1)
-        self.std.copy_(torch.as_tensor(new, device=self.std.device))
+        self.std.copy_(torch.as_tensor(new.reshape(-1), device=self.std.device))
         for holder in (self.policy, self.fused):
-            if holder is None:
-                continue
-            if holder.std_vec is not None:
-                holder.std_vec.copy_(self.std)
-            else:
-                holder.std = float(new[0])
+            if holder is not None:
+                holder.std, holder.std_vec = gaussian_std(new, out=holder.std_vec)
 
     # ------------------------------------------------------------------ update (PPO2.py:78-170)
     def _log_prob_entropy(self, s, a):
@@ -221,23 +216,29 @@ class VecPPO2:
             n_mb = _dist.agree_min(-(-B // mb), self.group)
         loss = self.fused.learn(buf.s, buf.a, buf.a_lp, adv, v_target, self.K_epochs, mb, self._epoch_key, n_mb)
         self._epoch_key = (self._epoch_key + self.K_epochs) & (2 ** 64 - 1)
-        self.policy.refresh()            # K-POLICY multiplies from a packed copy of the weights
-        self.value_net.refresh()
-        if m['use_lr_decay']:
-            self.lr_decay(self.total_steps)
+        self._after_fused_update()
         la, lc = loss.tolist()
         return {"actor_loss": la, "critic_loss": lc}
 
+    def _after_fused_update(self) -> None:
+        """What follows every K-LEARN update: the packed weights K-POLICY multiplies from are refreshed, then the
+        learning rates decay."""
+        self.policy.refresh()
+        self.value_net.refresh()
+        if self.msg['use_lr_decay']:
+            self.lr_decay(self.total_steps)
+
     def lr_decay(self, total_steps):                                                 # PPO2.py:162-171
-        if total_steps < self.msg['max_train_steps'] and self.fused is not None:
-            f = 1 - total_steps / self.msg['max_train_steps']
-            self.fused.lr = [max(self.msg['a_lr'] * f, 1e-6), max(self.msg['c_lr'] * f, 1e-6)]
+        if total_steps >= self.msg['max_train_steps']:
             return
-        if total_steps < self.msg['max_train_steps']:
-            f = 1 - total_steps / self.msg['max_train_steps']
-            for opt, lr in ((self.optimizer_actor, self.msg['a_lr']), (self.optimizer_critic, self.msg['c_lr'])):
-                for p in opt.param_groups:
-                    p['lr'] = max(lr * f, 1e-6)
+        f = 1 - total_steps / self.msg['max_train_steps']
+        lr = [max(self.msg['a_lr'] * f, 1e-6), max(self.msg['c_lr'] * f, 1e-6)]
+        if self.fused is not None:
+            self.fused.lr = lr
+            return
+        for opt, x in zip((self.optimizer_actor, self.optimizer_critic), lr):
+            for g in opt.param_groups:
+                g['lr'] = x
 
     def evaluate(self, obs_soa: torch.Tensor) -> torch.Tensor:
         """actor mean for ``[state_dim, N]`` observations (``agent.evaluate``, PPO2.py:62-66)."""
@@ -253,26 +254,13 @@ class VecPPO2:
         agent changes: not the training env, the policy's noise counter, the reward normaliser or the parameters.
         Returns ``ep_return`` (float64, NaN = unfinished), ``ep_length`` and ``ep_flag`` (int32, -1 = unfinished), all
         ``[N]`` device tensors, and the keys of :meth:`EpisodeTracker.summary`."""
-        if env is self.env or type(env) is not type(self.env):
-            raise ValueError("evaluate_episodes: env must be a separate instance of the training env's class")
-        if not env.auto_reset or env.io_dtype != torch.float32:
-            raise ValueError("evaluate_episodes: env must be built with auto_reset=True and io_dtype=torch.float32")
         if (env.state_dim, env.action_dim) != (self.policy.state_dim, self.policy.action_dim):
             raise ValueError("evaluate_episodes: env dimensions differ from the policy's")
-        tracker = EpisodeTracker(env.n_envs, env.device, first_only=True, group=self.group)
         zero = torch.zeros(env.action_dim, env.n_envs, dtype=torch.float32, device=env.device)
         action = torch.empty_like(zero)
         log_prob = torch.empty_like(zero)
-        env.reset(True)
-        for t in range(int(max_steps)):
-            # env._reset_obs is the policy-facing observation; step_soa may swap it with _obs, so it is read every step
-            self.policy(env._reset_obs, noise=zero, action=action, log_prob=log_prob)
-            env.step_soa(action)
-            tracker.update(env._reward, env._done, env._flag)
-            if (t + 1) % 64 == 0 and bool(tracker.finished().all()):
-                break
-        return {"ep_return": tracker.ep_return, "ep_length": tracker.ep_length, "ep_flag": tracker.ep_flag,
-                **tracker.summary()}
+        act = lambda obs: self.policy(obs, noise=zero, action=action, log_prob=log_prob)
+        return evaluate_first_episodes(self.env, env, act, action, max_steps, self.group)
 
 
 def reference_nets(state_dim: int, action_dim: int, device, init_std: float = 0.5, mean_act: str = "relu"):

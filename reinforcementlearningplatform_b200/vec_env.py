@@ -112,14 +112,6 @@ class VecEnvBase:
     def make_params(self) -> C.Structure:
         raise NotImplementedError
 
-    # ----------------------------------------------------------------- helpers
-    @staticmethod
-    def _ptr(t: Optional[torch.Tensor]):
-        return None if t is None else C.c_void_p(t.data_ptr())
-
-    def _stream(self):
-        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-
     # ------------------------------------------------------------------ rl_base metadata (algorithm/rl_base.py:5-124)
     # Descriptive lists the reference keeps next to state_dim / action_dim; the info printers and the PPO / DQN scripts read
     # them.  Every env of the engine is continuous in state and action unless a subclass says otherwise
@@ -238,8 +230,8 @@ class VecEnvBase:
                 if mask is not None:
                     m = mask.to(device=self.device, dtype=torch.uint8).contiguous()
                 _lib.check(self._lib.b200env_reset(self.ENV_ID, self._dt_code, self.n_envs, C.byref(self._params),
-                                                   C.sizeof(self._params), C.byref(io), self._ptr(m), self.seed,
-                                                   self.env_index_offset, self._stream()), "b200env_reset")
+                                                   C.sizeof(self._params), C.byref(io), _lib.ptr(m), self.seed,
+                                                   self.env_index_offset, _lib.stream(self.device)), "b200env_reset")
         else:
             self._reset_default(mask)
             if mask is None:
@@ -266,7 +258,7 @@ class VecEnvBase:
         with torch.cuda.device(self.device):
             io = self._io(obs=False, reset_obs=False)
             _lib.check(self._lib.b200env_observe(self.ENV_ID, self._dt_code, self.n_envs, C.byref(self._params),
-                                                 C.sizeof(self._params), C.byref(io), self._stream()),
+                                                 C.sizeof(self._params), C.byref(io), _lib.stream(self.device)),
                        "b200env_observe")
         return self.next_state
 
@@ -349,7 +341,7 @@ class VecEnvBase:
             flags = _lib.AUTO_RESET if self.auto_reset else 0
             _lib.check(self._lib.b200env_step(self.ENV_ID, self._dt_code, self.n_envs, C.byref(self._params),
                                               C.sizeof(self._params), C.byref(io), flags, self.seed,
-                                              self.env_index_offset, self._stream()), "b200env_step")
+                                              self.env_index_offset, _lib.stream(self.device)), "b200env_step")
 
     def rollout_into(self, steps: int, action: torch.Tensor, *, obs: torch.Tensor, next_obs: torch.Tensor,
                      reward: torch.Tensor, done: torch.Tensor, flag: torch.Tensor,
@@ -375,7 +367,7 @@ class VecEnvBase:
             _lib.check(self._lib.b200env_rollout(self.ENV_ID, self._dt_code, N, C.byref(self._params),
                                                  C.sizeof(self._params), C.byref(io), C.byref(spec),
                                                  _lib.AUTO_RESET if self.auto_reset else 0, self.seed,
-                                                 self.env_index_offset, self._stream()), "b200env_rollout")
+                                                 self.env_index_offset, _lib.stream(self.device)), "b200env_rollout")
         self._policy_obs_valid = True
 
     def get_reward(self) -> torch.Tensor:

@@ -58,15 +58,7 @@ def _lin(net):
 
 
 def _mlp(net):
-    m = _lib().MLP()
-    lins = _lin(net)
-    m.n_layers = len(lins)
-    m.dims[0] = lins[0].in_features
-    for l, lin in enumerate(lins):
-        m.dims[l + 1] = lin.out_features
-        m.w[l], m.b[l] = lin.weight.data_ptr(), lin.bias.data_ptr()
-    m.out_act = 0
-    return m
+    return _lib().mlp(_lin(net), 0)
 
 
 def _fwd64(net, x):

@@ -97,7 +97,7 @@ def main(argv=None):
     # 3. one update
     for M in (4096, 16384):
         agent.batch_size = M
-        agent.workspace = torch.zeros(int(agent._lib.b200_dqn_workspace_bytes(C.byref(agent._q), M)),
+        agent.workspace = torch.zeros(int(agent._lib.b200_dqn_workspace_bytes(C.byref(agent.q_mlp), M)),
                                       dtype=torch.uint8, device=dev)
         u = [0]
 

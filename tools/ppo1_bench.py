@@ -151,10 +151,10 @@ def ab_bench(other_path, runs=5, launches=200):
     a_lp = (-1.5 - 0.5 * torch.rand(T, A, N, device="cuda", generator=g)).contiguous()
     adv = torch.randn(T, N, device="cuda", generator=g).contiguous()
     vt = torch.randn(T, N, device="cuda", generator=g).contiguous()
-    am, cm = upd.params.mlp(0, upd.out_act), upd.params.mlp(1, 0)
-    p = lambda t: None if t is None else C.c_void_p(t.data_ptr())
+    am, cm = upd.mlps
+    p = _lib.ptr
     o = upd.params.net_off[1]
-    stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
+    stream = _lib.stream(upd.device)
     out = {}
     for count in (4096, 16384):
         b = upd._batch(s, a, a_lp, adv, vt, 0, count, perm_key=5)
