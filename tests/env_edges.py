@@ -26,12 +26,16 @@ import numpy as np
 from helpers import env_specs
 
 NAMES = ["cartpole", "cartpole_angleonly_env", "cartpole_angleonly_ppo2", "fas", "fas_ppo2", "fas_discrete", "soi",
-         "soi_dppo2", "ballbalancer", "twolink", "ugv_forward", "ugv_bidirectional"]
+         "soi_dppo2", "ballbalancer", "twolink", "ugv_forward", "ugv_bidirectional", "ugvo", "ugvo_dppo2"]
+UGV_NAMES = ("ugv_forward", "ugv_bidirectional")
+# UGVForwardObstacleAvoidance: variant 0 (the env, dt 0.1) and variant 1 (the PPO2 / DPPO2 demo copy, dt 0.05); flags
+# 1 bounds, 2 time-out, 3 success, 4 collision
+UGVO_NAMES = ("ugvo", "ugvo_dppo2")
 # the reference loops `while time < tt` in sub-steps of dt / 10: 10 or 11 of them, decided by the rounding of time
 SUBSTEP_NAMES = {"cartpole", "cartpole_angleonly_env", "fas", "fas_ppo2", "ballbalancer"}
 # success tests on a Euclidean norm: CartPole's Python `sqrt(a*a + b*b + ...)`, the others np.linalg.norm
 NORM_EDGES = [("cartpole", "success"), ("cartpole_angleonly_ppo2", "success"), ("soi", "success"), ("twolink", "success"),
-              ("ugv_forward", "success"), ("ugv_bidirectional", "success")]
+              ("ugv_forward", "success"), ("ugv_bidirectional", "success"), ("ugvo", "success"), ("ugvo_dppo2", "success")]
 TIME = -1          # Edge.coord of the pre-step time
 SEED = 20261021    # Philox seed of the auto-resets (both sides)
 
@@ -138,7 +142,13 @@ def rule_flag(name, p, pre, post, time, dt=np.float64):
     elif name == "twolink":
         en, wn = np_norm2(s[:, 4], s[:, 5], dt), np_norm2(s[:, 2], s[:, 3], dt)
         flag[:] = np.where(tout, 2, np.where((en <= T(p.miss)) & (wn <= T(p.omega_ok)), 3, 0))
-    elif name.startswith("ugv"):
+    elif name in UGVO_NAMES:  # is_Terminal: every test runs, the last true one wins
+        x, y = s[:, 0], s[:, 1]
+        flag[(x > T(p.map_x)) | (x < T(0)) | (y > T(p.map_y)) | (y < T(0))] = 1
+        flag[tout] = 2
+        flag[_ugvo_success(p, s, dt)] = 3
+        flag[_ugvo_collided(p, s, dt)] = 4
+    elif name in UGV_NAMES:
         x, y, vel = s[:, 0], s[:, 1], s[:, 2]
         flag[(x > T(p.map_x)) | (x < T(0)) | (y > T(p.map_y)) | (y < T(0))] = 1
         flag[tout] = 2
@@ -151,6 +161,25 @@ def rule_flag(name, p, pre, post, time, dt=np.float64):
     else:
         raise KeyError(name)
     return flag
+
+
+def _ugvo_success(p, s, dt=np.float64, norm=None):
+    """is_success :423-429 (variant 0) / demo copy :421-427 (variant 1, no omega test) on states [lanes, 56] in `dt`."""
+    T = dt
+    s = np.asarray(s, dt)
+    norm = norm or (lambda a, b: np_norm2(a, b, dt))
+    ok = (norm(s[:, 5] - s[:, 0], s[:, 6] - s[:, 1]) <= T(0.05)) & (np.abs(s[:, 2]) < T(0.01))
+    return ok & (np.abs(s[:, 4]) < T(0.01)) if p.variant == 0 else ok
+
+
+def _ugvo_collided(p, s, dt=np.float64):
+    """collision_check :261-272: some circle k < n_obs with |pos - centre| <= r_k + r_vehicle."""
+    s = np.asarray(s, dt)
+    hit = np.zeros(len(s), bool)
+    for k in range(16):
+        cx, cy, r = s[:, 8 + 3 * k], s[:, 9 + 3 * k], s[:, 10 + 3 * k]
+        hit |= (k < s[:, 7]) & (np_norm2(s[:, 0] - cx, s[:, 1] - cy, dt) <= r + dt(p.r_vehicle))
+    return hit
 
 
 def contracted_success(name, p, post):
@@ -172,7 +201,9 @@ def contracted_success(name, p, post):
         return (np.sqrt(sq(p.target_x - s[:, 0], p.target_y - s[:, 1])) <= 0.05) & (np.sqrt(sq(s[:, 2], s[:, 3])) < 0.05)
     if name == "twolink":
         return (np.sqrt(sq(s[:, 4], s[:, 5])) <= p.miss) & (np.sqrt(sq(s[:, 2], s[:, 3])) <= p.omega_ok)
-    if name.startswith("ugv"):
+    if name in UGVO_NAMES:
+        return _ugvo_success(p, s, norm=lambda a, b: np.sqrt(sq(a, b)))
+    if name in UGV_NAMES:
         return (np.sqrt(sq(p.target_x - s[:, 0], p.target_y - s[:, 1])) <= 0.05) & (np.abs(s[:, 2]) < 0.01)
     raise KeyError(name)
 
@@ -190,7 +221,9 @@ def reference_success(name, p, post):
         return (np_norm2(p.target_x - s[:, 0], p.target_y - s[:, 1]) <= 0.05) & (np_norm2(s[:, 2], s[:, 3]) < 0.05)
     if name == "twolink":
         return (np_norm2(s[:, 4], s[:, 5]) <= p.miss) & (np_norm2(s[:, 2], s[:, 3]) <= p.omega_ok)
-    if name.startswith("ugv"):
+    if name in UGVO_NAMES:
+        return _ugvo_success(p, s)
+    if name in UGV_NAMES:
         return (np_norm2(p.target_x - s[:, 0], p.target_y - s[:, 1]) <= 0.05) & (np.abs(s[:, 2]) < 0.01)
     raise KeyError(name)
 
@@ -227,6 +260,33 @@ def _ugv_reward(p, post, flag):
     return tot, ok
 
 
+def _ugvo_reward(p, out):
+    """get_reward :451-467 (variant 0) / demo copy :449-473 (variant 1) from a lane's own outputs (fp64).  Variant 0: the
+    heading term from numpy's atan2 and `ok` = lanes where that is well defined against the kernel's; variant 1 has no
+    transcendental: r2 / r3 compare the pre- and post-step observations, r4 reads the success rule and the flag.
+    Returns (reward, ok, branch code)."""
+    s = np.asarray(out["state"], np.float64)
+    x, y, vel, phi, om = s[:, :5].T
+    dx, dy = s[:, 5] - x, s[:, 6] - y
+    err = np_norm2(dx, dy)
+    if p.variant == 0:
+        c, sn = np.cos(phi), np.sin(phi)
+        guard = (err < 1e-4) | (np_norm2(c, sn) < 1e-4)
+        ephi = np.where(guard, 0.0, np.arctan2(c * dy - sn * dx, c * dx + sn * dy))
+        u_pos, u_vel, u_om = -np.abs(err) * p.Q_pos, -np.abs(vel) * p.Q_vel, -np.abs(om) * p.Q_omega
+        u_phi = np.where(err > 0.1, -np.abs(ephi) * p.Q_phi, 0.0)
+        u_psi = np.where(out["flag"] == 1, (p.time_max - np.asarray(out["time"], np.float64)) / p.dt * (u_pos + u_vel + u_phi + u_om), 0.0)
+        return u_pos + u_vel + u_phi + u_om + u_psi, np.ones(len(s), bool), (err > 0.1).astype(np.int32)
+    cur, nxt = np.asarray(out["obs"], np.float64), np.asarray(out["next_obs"], np.float64)
+    r1 = -1 - np.abs(om) * 0.1
+    r2 = np.where(cur[:, 0] > nxt[:, 0] + 1e-3, 5.0, np.where(1e-3 + cur[:, 0] < nxt[:, 0], -5.0, 0.0))
+    a, b = np.abs(cur[:, 1]), np.abs(nxt[:, 1])
+    r3 = np.where(a > b + 1e-2, 2.0, np.where(1e-2 + a < b, -2.0, 0.0))
+    r4 = np.where(_ugvo_success(p, s), 500.0, np.where(out["flag"] == 4, -300.0, 0.0))
+    code = (3 * (np.sign(r2) + 1) + np.sign(r3) + 1).astype(np.int32) + 9 * np.sign(r4).astype(np.int32)
+    return r1 + r2 + r3 + r4, np.ones(len(s), bool), code
+
+
 def reward_branch(name, p, out):
     """the reward branch a lane took, from its own outputs (None: the reward has no branch besides the flag's)."""
     s = np.asarray(out["state"], np.float64)
@@ -234,7 +294,9 @@ def reward_branch(name, p, out):
         return _angleonly_reward(p, out["obs"][:, 0], out["next_obs"][:, 0], out["flag"])
     if name == "ballbalancer":
         return (np.abs(s[:, 3]) <= 0.001) & (np.abs(s[:, 1]) <= 0.005) & (np.abs(s[:, 2]) <= p.deg1)
-    if name.startswith("ugv"):
+    if name in UGVO_NAMES:
+        return _ugvo_reward(p, out)[2]
+    if name in UGV_NAMES:
         return np_norm2(p.target_x - s[:, 0], p.target_y - s[:, 1]) > 0.1
     return None
 
@@ -256,7 +318,16 @@ def rule_extras(name, p, out):
         bad["theta clamp"] = (s[:, 2] < p.theta_min) | (s[:, 2] > p.theta_max)
     elif name == "twolink":
         bad["wrap into [-theta_max, theta_max]"] = (np.abs(s[:, 0]) > p.theta_max) | (np.abs(s[:, 1]) > p.theta_max)
-    elif name.startswith("ugv"):
+    elif name in UGVO_NAMES:
+        bad["phi wrap into [-pi, pi]"] = np.abs(s[:, 3]) > np.pi
+        if p.variant == 0:
+            bad["vel >= 0 clamp"] = s[:, 2] < 0
+        want, ok, _ = _ugvo_reward(p, out)
+        if p.variant == 0:   # atan2 in the heading term: within 1e-9 relative
+            bad["reward (u_phi above err 0.1, u_psi on flag 1)"] = ok & (np.abs(out["reward"] - want) > 1e-9 * np.maximum(1.0, np.abs(want)))
+        else:                # every term a branch constant: bit for bit
+            bad["reward r1 + r2 + r3 + r4"] = out["reward"] != want
+    elif name in UGV_NAMES:
         bad["phi wrap into [-pi, pi]"] = np.abs(s[:, 3]) > np.pi
         if not p.bidirectional:
             bad["vel >= 0 clamp"] = s[:, 2] < 0
@@ -403,6 +474,147 @@ def _time_edges(name, p, st0, act0, loops):
         edges.append(Edge("substeps", "time", TIME, np.repeat(st0[None, :], B, 0), grid[at], np.repeat(act0[None, :], B, 0),
                           pred=lambda o: o["substeps"] == 11, lo=grid[at], hi=grid[at + 1], K=24))
     return edges
+
+
+UGVO_TARGET = (2.5, 2.5)
+# Circles for the pose-level UGV-FOA lanes.  A lane carries those that lie out of laser range of its pose by 0.5 m (more
+# than any step moves), so the in-range list is built and comes out empty: the laser only meets walls, whose ranges do
+# not jump with an ulp of the slope.  The collision blocks add one circle of their own.
+_UGVO_FAR = ((0.4, 0.4, 0.3), (4.6, 0.4, 0.25), (0.4, 4.6, 0.35), (4.6, 4.6, 0.2), (2.5, 0.3, 0.2), (2.5, 4.7, 0.25),
+             (0.3, 2.5, 0.2), (4.7, 2.5, 0.3))
+
+
+def ugvo_row(p, x, y, vel=0.0, phi=0.3, omega=0.0, near=(), target=UGVO_TARGET):
+    """one UGV-FOA state [56]: pose, target, the circles `near` first, then the far ones (headings near 0.3 keep every
+    ray at least 2 degrees off the vertical)."""
+    s = np.zeros(56)
+    s[:7] = x, y, vel, phi, omega, target[0], target[1]
+    circ = list(near) + [c for c in _UGVO_FAR if np.hypot(c[0] - x, c[1] - y) > p.laser_dis + c[2] + 0.5]
+    assert len(circ) >= 1
+    s[7] = len(circ)
+    for k, c in enumerate(circ):
+        s[8 + 3 * k:11 + 3 * k] = c
+    return s
+
+
+def _ugvo_rows(p, x, y, vel, phi, omega, target=UGVO_TARGET):
+    return np.stack([ugvo_row(p, *v, target=target) for v in zip(*np.broadcast_arrays(x, y, vel, phi, omega))])
+
+
+def _ugvo_edges(name, p, rng):
+    """the pose-level edges of UGVForwardObstacleAvoidance (variant 0 and the demo copy, variant 1)."""
+    E = []
+    flag_is = lambda f: (lambda o: o["flag"] == f)
+    tx, ty = UGVO_TARGET
+    v = p.variant
+    B, A = 32, 2
+    z1, a0 = np.zeros(1), np.zeros((1, A))
+    late = np.array([p.time_max - p.dt / 2])   # the post-step time is past time_max
+    box = [("x_hi", 0, p.map_x), ("x_lo", 0, 0.0), ("y_hi", 1, p.map_y), ("y_lo", 1, 0.0)]
+    for lab, c, thr in box:
+        xy = [tx, ty]
+        xy[c] = thr
+        s = ugvo_row(p, *xy)
+        E.append(Edge(lab, "parked", c, s[None], z1, a0, flag_is(1), center=np.array([thr])))
+        E.append(Edge(lab + "+time", "priority", c, s[None], late, a0, flag_is(2), center=np.array([thr]), cover=False))
+    for lab, thr in (("phi_hi", np.pi), ("phi_lo", -np.pi)):
+        s = ugvo_row(p, 1.0, 1.0, phi=thr)
+        E.append(Edge(lab, "parked", 3, s[None], z1, a0, lambda o, t=thr: o["state"][:, 3] * t < 0, center=np.array([thr])))
+    s = ugvo_row(p, tx - 0.05, ty)
+    E.append(Edge("success_parked", "parked", 0, s[None], z1, a0, flag_is(3), center=np.array([tx - 0.05])))
+    sd = np.stack([ugvo_row(p, tx - 0.03, ty - 0.04, phi=1.0), ugvo_row(p, tx + 0.04, ty + 0.03, phi=-2.0)])
+    E.append(Edge("success_parked_diag", "parked", 1, sd, np.zeros(2), np.zeros((2, A)), flag_is(3),
+                  lo=sd[:, 1] - np.sign(sd[:, 1] - ty) * 0.005, hi=sd[:, 1] + np.sign(sd[:, 1] - ty) * 0.005))
+    E.append(Edge("success+time", "priority", 0, s[None], late, a0, flag_is(3), center=np.array([tx - 0.05])))
+    # err exactly fl(0.05): x = 2^-10 and target x = 2^-10 + fl(0.05) (the sum and the difference are exact; the target's
+    # ulps are err's, so the scan of the target moves err one ulp at a time)
+    g = 2.0 ** -10
+    s = ugvo_row(p, g, ty, target=(g + 0.05, ty))
+    E.append(Edge("success_parked_exact", "parked", 5, s[None], z1, a0, flag_is(3), center=np.array([g + 0.05])))
+    s = ugvo_row(p, tx - 1e-4, ty)   # vector_rad_oriented's `norm < 1e-4` guard: ephi (obs 2) == 0
+    E.append(Edge("ephi_guard", "parked", 0, s[None], z1, a0, lambda o: o["next_obs"][:, 2] != 0,
+                  lo=np.array([tx - 2e-4]), hi=np.array([tx])))
+    if v == 0:   # reward branch err > 0.1 (heading error 0.5 rad: u_phi = -1)
+        s = ugvo_row(p, tx - 0.1, ty, phi=0.5)
+        E.append(Edge("reward_e_0.1", "parked", 0, s[None], z1, a0, lambda o: o["reward"] < -0.5, center=np.array([tx - 0.1])))
+    # collision at |pos - centre| == r + r_vehicle: the centre's x bisected to the flip; with several flags at once the
+    # collision must win over success + time-out and over bounds
+    R = 0.3 + p.r_vehicle
+    for lab, kind, (x, y), ang, tm, cov in (("collision", "parked", (1.5, 2.5), 0.0, 0.0, True),
+                                            ("collision_diag", "parked", (1.5, 2.5), 0.7, 0.0, True),
+                                            ("collision+success+time", "priority", (tx - 0.03, ty), 0.0, late[0], True),
+                                            ("collision+x_hi", "priority", (p.map_x, ty), np.pi, 0.0, False)):
+        cx, cy = x + R * np.cos(ang), y + R * np.sin(ang)
+        s = ugvo_row(p, x, y, near=[(cx, cy, 0.3)])
+        sg = 1.0 if np.cos(ang) >= 0 else -1.0
+        E.append(Edge(lab, kind, 8, s[None], np.array([tm]), a0, flag_is(4), lo=np.array([cx + sg * 0.01]),
+                      hi=np.array([cx - sg * 0.01]), cover=cov))
+    if v == 1:   # the pose frozen on the PRE-update velocity (vel < 0): -0.0 and +0.0 move, -5e-324 freezes
+        frozen = lambda o: o["state"][:, 0] == 2.0
+        s, act = ugvo_row(p, 2.0, 2.0, phi=0.3, omega=0.2), np.array([[2.0, 0.5]])
+
+        def neg0(st, dt):
+            st[:, 2] = -0.0
+        E.append(Edge("frozen_vel", "cross", 2, s[None], z1, act, frozen, center=np.array([0.0]), K=3))
+        E.append(Edge("frozen_vel_neg0", "cross", 2, s[None], z1, act, frozen, center=np.array([0.0]), K=0, derive=neg0, cover=False))
+        E.append(Edge("frozen_vel_neg", "cross", 2, s[None], z1, act, frozen, center=np.array([-1e-3]), K=2, cover=False))
+        s = ugvo_row(p, p.map_x, ty, vel=-0.5, phi=0.3)   # frozen on the border: the flag from the unmoved x
+        E.append(Edge("x_hi_frozen", "cross", 0, s[None], z1, np.array([[1.0, 0.5]]), flag_is(1), center=np.array([p.map_x])))
+    E += _time_edges(name, p, ugvo_row(p, 1.5, 1.5), np.zeros(A), False)
+    # ---- crossing lanes
+    for lab, c, thr in box:
+        sgn = 1 if lab.endswith("hi") else -1
+        head = (0.0 if sgn > 0 else np.pi) if c == 0 else sgn * np.pi / 2
+        xy = [np.full(B, tx), np.full(B, ty)]
+        xy[c][:] = thr
+        st = _ugvo_rows(p, xy[0], xy[1], rng.uniform(0.5, 2.5, B), head + rng.uniform(-0.4, 0.4, B), rng.uniform(-1, 1, B))
+        act = _f32(rng.uniform(-3, 3, (B, A)))
+        E.append(Edge(lab + "_cross", "cross", c, st, np.zeros(B), act, flag_is(1), lo=np.full(B, thr - sgn * 0.2),
+                      hi=np.full(B, thr + sgn * 0.01), K=64))
+    for lab, sgn in (("phi_hi", 1), ("phi_lo", -1)):   # heading wrap at +-pi after RK4
+        st = _ugvo_rows(p, rng.uniform(1.5, 3.5, B), rng.uniform(1.5, 3.5, B), rng.uniform(0, 1, B), 0.0,
+                        sgn * rng.uniform(0.5, 3, B))
+        act = _f32(rng.uniform(-3, 3, (B, A)))
+        E.append(Edge(lab + "_cross", "cross", 3, st, np.zeros(B), act, lambda o, s=sgn: s * o["state"][:, 3] < 0,
+                      lo=np.full(B, sgn * (np.pi - 0.2)), hi=np.full(B, sgn * np.pi), K=64))
+    # success on err <= 0.05 (np.linalg.norm's FMA form), crossed by x; small velocity and rate.  A target near the
+    # corner (0, 0): an ulp of x there moves err by a few of its own ulps, so scans land on the threshold
+    BS, g = 256, 0.25
+    ang = rng.uniform(0, 2 * np.pi, BS)
+    om = rng.uniform(-0.005, 0.005, BS) if v == 0 else rng.uniform(-0.5, 0.5, BS)
+    st = _ugvo_rows(p, g, g + 0.04 * np.sin(ang), rng.uniform(0, 0.005, BS), rng.uniform(-np.pi, np.pi, BS), om, (g, g))
+    act = _f32(np.stack([rng.uniform(-0.03, 0.03, BS), rng.uniform(-0.02, 0.02, BS)], 1))
+    E.append(Edge("success", "cross", 0, st, np.zeros(BS), act, flag_is(3), lo=np.full(BS, g), hi=np.full(BS, g + 0.1), K=16))
+    # success on |vel| < 0.01, crossed by the pre-step velocity (at the target: err stays ~vel dt)
+    st = _ugvo_rows(p, tx, ty, 0.0, rng.uniform(-np.pi, np.pi, B), 0.0)
+    act = _f32(np.stack([rng.uniform(-0.05, 0.05, B), np.zeros(B)], 1))
+    E.append(Edge("success_vel", "cross", 2, st, np.zeros(B), act, flag_is(3), lo=np.zeros(B), hi=np.full(B, 0.03), K=64))
+    if v == 0:   # success on |omega| < 0.01 (variant 0 only), crossed by the pre-step rate, both signs
+        for lab, sgn in (("success_omega_pos", 1), ("success_omega_neg", -1)):
+            st = _ugvo_rows(p, tx - 0.02, ty, 0.0, rng.uniform(-np.pi, np.pi, B), 0.0)
+            act = _f32(np.stack([np.zeros(B), rng.uniform(-0.05, 0.05, B)], 1))
+            E.append(Edge(lab, "cross", 4, st, np.zeros(B), act, flag_is(3), lo=np.zeros(B), hi=np.full(B, sgn * 0.03), K=64))
+        st = _ugvo_rows(p, tx - 0.1, ty, rng.uniform(0.05, 0.3, B), rng.uniform(0.4, 0.8, B), 0.0)
+        act = _f32(rng.uniform(-0.5, 0.5, (B, A)))
+        E.append(Edge("reward_e_0.1_cross", "cross", 0, st, np.zeros(B), act, lambda o: o["reward"] < -0.5,
+                      lo=np.full(B, tx - 0.2), hi=np.full(B, tx - 0.02), K=64))
+        st = _ugvo_rows(p, rng.uniform(1.5, 3.5, B), rng.uniform(1.5, 3.5, B), 0.0, rng.uniform(-3, 3, B), 0.0)
+        act = _f32(np.stack([rng.uniform(-3, -0.5, B), rng.uniform(-3, 3, B)], 1))
+        E.append(Edge("vel_clamp", "cross", 2, st, np.zeros(B), act, lambda o: o["state"][:, 2] == 0,
+                      lo=np.full(B, 0.1), hi=np.zeros(B), K=64))
+    else:
+        # r2 = +-5 where cur_e - nk0 crosses +-1e-3: heading to / away from the target, crossed by the velocity
+        for lab, head, pred in (("reward_r2_pos", 0.0, lambda o: o["reward"] > 0), ("reward_r2_neg", np.pi, lambda o: o["reward"] < -3)):
+            st = _ugvo_rows(p, tx - 1.0, ty, 0.0, head + rng.uniform(-0.2, 0.2, B), 0.0)
+            E.append(Edge(lab, "cross", 2, st, np.zeros(B), np.zeros((B, A)), pred, lo=np.full(B, 0.01), hi=np.full(B, 0.08), K=64))
+        # r3 = +-2 where |cur1| - |nk1| crosses +-1e-2: moving across the target's bearing, the step's velocity change
+        # 0.05 (a - 0.1 vel) crossing 0.015 at vel = 0.1
+        for lab, a, lo, hi, pred in (("reward_r3_pos", 0.31, 0.0, 0.2, lambda o: o["reward"] > 0.5),
+                                     ("reward_r3_neg", -0.29, 0.0, 0.2, lambda o: o["reward"] < -2)):
+            st = _ugvo_rows(p, tx - 1.0, ty, 0.0, np.pi / 2 + rng.uniform(-0.05, 0.05, B), 0.0)
+            act = _f32(np.stack([np.full(B, a), np.zeros(B)], 1))
+            E.append(Edge(lab, "cross", 2, st, np.zeros(B), act, pred, lo=np.full(B, lo), hi=np.full(B, hi), K=64))
+    return E
 
 
 def _family_edges(name, p, rng):
@@ -635,7 +847,9 @@ def _family_edges(name, p, rng):
         ang = rng.uniform(0, 2 * np.pi, BS)
         st[:, 7] = endy + 0.008 * np.sin(ang)
         E.append(Edge("success", "cross", 6, st, tm, act, flag_is(3), lo=np.full(BS, endx), hi=np.full(BS, endx + 0.05), K=KS))
-    elif name.startswith("ugv"):
+    elif name in UGVO_NAMES:
+        E += _ugvo_edges(name, p, rng)
+    elif name in UGV_NAMES:
         F, A = 5, 2
         tx, ty = p.target_x, p.target_y
         bid = bool(p.bidirectional)
@@ -743,6 +957,6 @@ def state_compare(name, p, a, b):
     """per-lane mixed error |a - b| / max(1, |b|) of post-step states, the wrapped angles compared modulo their period."""
     a, b = np.asarray(a, np.float64), np.asarray(b, np.float64)
     d = a - b
-    cols, per = ([0, 1], 2 * p.theta_max) if name == "twolink" else ([3], 2 * np.pi) if name.startswith("ugv") else ([], 1.0)
+    cols, per = ([0, 1], 2 * p.theta_max) if name == "twolink" else ([3], 2 * np.pi) if name in UGV_NAMES + UGVO_NAMES else ([], 1.0)
     d[:, cols] = (d[:, cols] + per / 2) % per - per / 2
     return np.max(np.abs(d) / np.maximum(1.0, np.abs(b)), axis=1)

@@ -76,9 +76,9 @@ def test_parked_and_time_lanes_equal_the_oracle(name, oracle_lib):
     # reward holds no transcendental: UGV's heading term -|ephi| Q_phi (atan2, taken when e > 0.1) is within ENGINE_TOL
     still = E.oracle_step(name, L.state, L.time, L.action)["state"]   # before any auto-reset
     exact = np.all(still == L.state, axis=1)
-    if name.startswith("ugv"):
-        p = E.host(name)._params
-        exact &= E.np_norm2(p.target_x - L.state[:, 0], p.target_y - L.state[:, 1]) <= 0.1
+    if name in E.UGV_NAMES or name == "ugvo":   # (UGV-FOA's demo-copy reward has no heading term)
+        tx, ty = (L.state[:, 5], L.state[:, 6]) if name == "ugvo" else (E.host(name)._params.target_x, E.host(name)._params.target_y)
+        exact &= E.np_norm2(tx - L.state[:, 0], ty - L.state[:, 1]) <= 0.1
     bad = np.where(exact, g["reward"] != o["reward"], _mixed(g["reward"], o["reward"]) > tol)
     assert not bad.any(), (name, "reward", int(bad.sum()), _where(L, bad))
     assert exact.sum() > 0 or name in ("cartpole_angleonly_ppo2", "fas", "fas_ppo2", "fas_discrete"), name
